@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the batched delivery_drone simulator (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]           # ours (CUDA, sm_100a)
+    python bench.py [--gpus N] [--steps K] [--warmup W]           # ours (CUDA, sm_100a): K timed steps
+    python bench.py ... --dump-outputs DIR                         # + the last timed step's outputs as DIR/*.npy
     python bench.py --impl reference [--gpus N] --steps K ...      # the reference's CPU path (port)
     torchrun ... bench.py --gpus N ...                             # one rank per GPU, weak scaling
 
@@ -38,6 +39,7 @@ METRIC = "env-steps/sec"
 UNIT = "env-steps/s"
 ENVS_PER_GPU = 1 << 20
 MAX_STEPS = 250
+LEAD_IN = 32              # launches queued, untimed, ahead of the timed steps (~0.8 ms of GPU work at 1M envs per launch)
 BYTES_STEP_ONLY = 86      # SURVEY.md 8d: read 44 + action 1, write 36 + reward 4 + flags 1
 BYTES_GYM = 146           # + 60 B observation row
 WORKLOAD = ("1M drone envs per GPU, auto-reset + spawn randomisation (drone+platform), max_steps 250, "
@@ -248,6 +250,30 @@ def socket_shim_rate(dev, games: int = 6, seconds: float = 2.0):
             "what": "compat.DroneSocketServer + DroneGameClient over 127.0.0.1 (the reference's wire protocol), one request per step"}
 
 
+DUMP_ROWS = 1 << 19      # env rows written by --dump-outputs: 17 float32 + 1 float64 per row, 40 MB at most
+
+
+def dump_outputs(out_dir: str, env) -> dict:
+    """What the last timed step handed its caller, as DIR/<name>.npy: the observations, rewards and flags (DD_* bits,
+    as numbers) of the shard that step advanced, in float32.  A shard of more than DUMP_ROWS envs is sampled at fixed,
+    seeded rows; env_index.npy (float64) lists the rows written."""
+    import numpy as np
+    import torch
+    env.join()
+    s = (env.t - 1) % env.S
+    sh = env.shards[s]
+    n = sh.num_envs
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(sh.obs.device)
+    arrays = {"obs": sh.obs[idx], "reward": sh.reward[idx], "flags": sh.step_flags[idx]}
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+    return {"dir": out_dir, "shard": s, "launch": env.t - 1, "rows": len(rows), "of": n,
+            "files": ["env_index.npy"] + [name + ".npy" for name in arrays]}
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -319,31 +345,55 @@ def run_ours(args):
         env.random_trace()
         return env
 
-    def time_steps(env, want_obs, sampler=None, est_us=25.0):
-        """R repeats of the K-step block, R sized so that the timed region is >= --min-time-ms; every block runs
-        through env.run(K): graph replays whatever K is.  Returns (ms_total, R)."""
+    def time_steps(env, want_obs, sampler=None):
+        """The K timed steps: one block env.run(K) (graph replays whatever K is), after the warm-up steps, a rehearsal that
+        captures every graph a block can replay and an untimed lead-in: one run() of at least LEAD_IN launches, whole
+        K-step blocks, so that the host has queued the timed block long before the GPU reaches it.  The events are
+        recorded on the env's chain streams, after the lead-in and after the K steps: each chain's share of the K launches
+        is timed from the end of its own lead-in to its own end, and the region is the longest of these spans.  So the
+        launches are timed as they flow behind work in flight, and neither the host's launch latency, the fork and join
+        of the chains, the refill of an idle GPU nor the phase offset between the chains enters it.  On a B200 at 1,000 W,
+        one CUDA-event pair on the caller's stream around the block measured ~22 us per region above the steady per-step
+        time, these spans ~10 us (the drain of the last launch).  Returns the milliseconds of the K steps (max over ranks)."""
         period = env.S * env.L
-        R = max(1, int(math.ceil(args.min_time_ms * 1e3 / (K * est_us))))
-        rehearse = max(R, period // math.gcd(K, period))        # visits every (offset, length) piece of the schedule
 
         def blocks(r):
             for _ in range(r):
                 env.run(K, want_obs=want_obs)
-            env.join()                                          # the current stream (where the events are) waits for the chains
+            env.join()
         blocks(-(-W // K))                                      # the W warm-up steps
-        blocks(rehearse)                                        # all graphs captured before the clock starts
-        g0 = env.graphs_cached
-        ms = timed(lambda: None, lambda: blocks(R), sampler)
-        if max_over_ranks(float(env.graphs_cached != g0)) > 0:  # a capture happened inside the timed region (any rank): redo
-            ms = timed(lambda: None, lambda: blocks(R), sampler)
-        return ms, R
+        blocks(period // math.gcd(K, period))                   # visits every (offset, length) piece of the schedule
+
+        def measure():
+            barrier()
+            env.run(K * -(-max(LEAD_IN, env.C) // K), want_obs=want_obs)   # the lead-in (may capture: not timed)
+            g0 = env.graphs_cached
+            t0, t1 = ([torch.cuda.Event(enable_timing=True) for _ in env._chains] for _ in range(2))
+            for ev, ch in zip(t0, env._chains):
+                ev.record(ch)
+            if sampler is not None:
+                sampler.start()
+            env.run(K, want_obs=want_obs)
+            for ev, ch in zip(t1, env._chains):
+                ev.record(ch)
+            env.join()
+            torch.cuda.synchronize(dev)
+            if sampler is not None:
+                sampler.stop()
+            barrier()
+            return max_over_ranks(max(a.elapsed_time(b) for a, b in zip(t0, t1))), env.graphs_cached != g0
+        ms, captured = measure()
+        if max_over_ranks(float(captured)) > 0:                 # a capture happened inside the timed region (any rank): redo
+            ms, _ = measure()
+        return ms
 
     sampler = ClockSampler(local, period_s=0.004)
     env = make_sharded(torch.float32, S)
-    ms_gym, R_gym = time_steps(env, True, sampler)
-    launches += K * R_gym
-    ms_so, R_so = time_steps(env, False, None, est_us=15.0)
-    launches += K * R_so
+    ms_gym = time_steps(env, True, sampler)
+    launches += K
+    dumped = dump_outputs(args.dump_outputs, env) if args.dump_outputs and rank == 0 else None
+    ms_so = time_steps(env, False, None)
+    launches += K
     launch_mode = (f"eager: one dd_step_planned call per step on {env.C} chain stream(s)" if args.eager else
                    f"CUDA graphs (product path ShardedDroneEnv.run): each K-step block is one piece of the {env.S * env.L}-launch "
                    f"schedule and replays one cached graph per chain; {env.C} parallel chain(s) over independent shards, joined to "
@@ -382,12 +432,12 @@ def run_ours(args):
     if not args.no_f64:
         S64 = max(2, min(S, 4))
         env64 = make_sharded(torch.float64, S64)
-        ms64, R64 = time_steps(env64, True, None, est_us=60.0)
-        launches += K * R64
-        a64 = n * BYTES_GYM_F64 / (ms64 * 1e-3 / (K * R64)) / 1e9
-        f64 = {"value": n * K * R64 * ws / (ms64 * 1e-3), "ms_per_step": ms64 / (K * R64), "dtype": "f64",
+        ms64 = time_steps(env64, True, None)
+        launches += K
+        a64 = n * BYTES_GYM_F64 / (ms64 * 1e-3 / K) / 1e9
+        f64 = {"value": n * K * ws / (ms64 * 1e-3), "ms_per_step": ms64 / K, "dtype": "f64",
                "algorithmic_bytes_per_env_step": BYTES_GYM_F64, "achieved_gbs": a64, "frac": a64 / peak_gbs,
-               "shards_per_gpu": S64, "repeats": R64, "timed_region_ms": ms64,
+               "shards_per_gpu": S64, "timed_region_ms": ms64,
                "what": "step_kernel<double,AUTO,OBS>: state, observations and rewards in float64, flags / counters bit-exact "
                        "against the oracle (tests/test_gpu_parity.py); FP64 pipe bound on B200, not HBM bound"}
         del env64
@@ -653,12 +703,11 @@ def run_ours(args):
     stats = env.stats(reduce=ws > 1)
 
     if rank == 0:
-        steps_timed = K * R_gym
-        value = n * steps_timed * ws / (ms_gym * 1e-3)
-        per_launch_s = ms_gym * 1e-3 / steps_timed
+        value = n * K * ws / (ms_gym * 1e-3)
+        per_launch_s = ms_gym * 1e-3 / K
         achieved = n * BYTES_GYM / per_launch_s / 1e9
         traffic, traffic_src = _ncu_traffic(n)
-        so_per = ms_so * 1e-3 / (K * R_so)
+        so_per = ms_so * 1e-3 / K
         so_achieved = n * BYTES_STEP_ONLY / so_per / 1e9
         eg_ach = n * BYTES_GYM / (ms_eager * 1e-3 / Ke) / 1e9
         others["step_kernel_step_only"] = {"bound": "hbm", "achieved": so_achieved, "peak": peak_gbs, "unit": "GB/s",
@@ -669,16 +718,16 @@ def run_ours(args):
                                          "note": "limited by the FP64 pipe of B200, reported against HBM for comparison"}
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": ws, "steps": K, "warmup": W,
-            "ms_per_step": ms_gym / steps_timed, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "ms_per_step": ms_gym / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
-            "repeats": R_gym, "timed_region_ms": ms_gym, "steps_timed": steps_timed,
+            "timed_region_ms": ms_gym, "steps_timed": K,
             "config": {"workload": WORKLOAD, "envs_per_gpu_per_step": n, "shards_per_gpu": S,
                        "l2": f"inputs larger than L2: steps rotate over {S} independent {n}-env shards "
                              f"({S} x ~{n * 116 >> 20} MiB state+outputs > 126 MB L2)",
                        "launch": launch_mode, "parallelism": f"env-sharded x{ws}, no per-step comms",
-                       "timing": f"the K = {K}-step block repeated {R_gym}x back to back inside one CUDA-event pair "
-                                 f"(>= {args.min_time_ms:.0f} ms); ms_per_step = timed_region_ms / (K x repeats); clocks sampled by NVML "
-                                 f"every 4 ms inside that region"},
+                       "timing": f"the K = {K} steps as one block behind an untimed lead-in, timed by CUDA events on "
+                                 f"the chain streams: the longest span of a chain from the end of its lead-in to the end of its "
+                                 f"share; ms_per_step = timed_region_ms / K; clocks sampled by NVML every 4 ms inside that region"},
             "roofline": {"bound": "hbm", "kernel": "step_kernel<float,AUTO,OBS>", "achieved": achieved, "peak": peak_gbs,
                          "unit": "GB/s", "frac": achieved / peak_gbs, "frac_of_nominal_8000_gbs": achieved / 8000.0,
                          "traffic": traffic, "traffic_unit": "bytes per launch",
@@ -686,9 +735,9 @@ def run_ours(args):
                          "algorithmic_bytes_per_env_step": BYTES_GYM, "env_steps_per_launch": n,
                          "others": others, "others_tensor_peak_source": PK["bf16_src"]},
             "variants": {
-                "step_only": {"value": n * K * R_so * ws / (ms_so * 1e-3), "ms_per_step": so_per * 1e3,
+                "step_only": {"value": n * K * ws / (ms_so * 1e-3), "ms_per_step": so_per * 1e3,
                               "algorithmic_bytes_per_env_step": BYTES_STEP_ONLY, "achieved_gbs": so_achieved,
-                              "frac": so_achieved / peak_gbs, "repeats": R_so, "timed_region_ms": ms_so},
+                              "frac": so_achieved / peak_gbs, "timed_region_ms": ms_so},
                 "gym_step_f64": f64,
                 "gym_step_eager_api": {"value": n * Ke * ws / (ms_eager * 1e-3), "ms_per_step": ms_eager / Ke, "achieved_gbs": eg_ach,
                                        "frac": eg_ach / peak_gbs, "steps": Ke, "host_us_per_step_raw_call": host_us,
@@ -720,6 +769,8 @@ def run_ours(args):
         }
         if mgc is not None:
             line["multi_gpu_check"] = mgc
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         if ws == 1 and not args.no_socket:
             try:
                 line["socket_shim"] = socket_shim_rate(dev)
@@ -792,7 +843,7 @@ def multi_gpu_check(dd, dist, cenv, cap, rank, ws, NC, dev):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=int(os.environ.get("WORLD_SIZE", "1")))
-    ap.add_argument("--steps", type=int, default=12000)
+    ap.add_argument("--steps", type=int, default=12000, help="timed steps (of the gym step, the step-only and the float64 variants)")
     ap.add_argument("--warmup", type=int, default=600)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--envs", type=int, default=ENVS_PER_GPU, help="envs per shard (= per step launch)")
@@ -800,7 +851,7 @@ def main():
     ap.add_argument("--chains", type=int, default=2, help="parallel launch chains in the CUDA graph (shard s -> chain s %% chains)")
     ap.add_argument("--e2e-steps", type=int, default=100)
     ap.add_argument("--trace-len", type=int, default=16, help="rows of the device action trace per shard (schedule period = shards x this)")
-    ap.add_argument("--min-time-ms", type=float, default=150.0, help="repeat the K-step block until the timed region is at least this long")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy")
     ap.add_argument("--eager", action="store_true", help="no CUDA graphs: one Python -> C-ABI launch per step (A/B)")
     ap.add_argument("--no-f64", action="store_true", help="skip the float64 (exact-parity) instantiation variant")
     ap.add_argument("--cpu-ticks", type=int, default=250000)
@@ -814,6 +865,8 @@ def main():
     ap.add_argument("--launch-flags", type=lambda v: int(v, 0), default=0x01,
                     help="DD_LAUNCH_* bits (include/drone_b200.h): 0x01 PDL, 0x10 CTA 128, 0x20 CTA 512")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -13,7 +13,7 @@ import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
-# DRONE_B200_LIB selects another in-tree build of the same sources (A/B runs of kernel variants on one box)
+# DRONE_B200_LIB selects another build of the sources (A/B timing of two versions in one process run)
 LIB_PATH = os.environ.get("DRONE_B200_LIB") or os.path.join(_HERE, "libdrone_b200.so")
 SOURCES = ("drone_kernels.cu", "ppo_kernels.cu", "policy_rollout.cu")
 NVCC_FLAGS = (
@@ -106,7 +106,7 @@ def build_native(force: bool = False, verbose: bool = False) -> str:
     if not force and os.path.exists(LIB_PATH) and all(
             os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
-    cmd = [nvcc_path(), *NVCC_FLAGS, *os.environ.get("DD_NVCC_EXTRA", "").split(), "-o", LIB_PATH + ".tmp", *srcs]
+    cmd = [nvcc_path(), *NVCC_FLAGS, "-o", LIB_PATH + ".tmp", *srcs]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
         print(" ".join(cmd))

@@ -1,6 +1,6 @@
-// drone_device.cuh -- device-side helpers shared by the kernels of drone_kernels.cu and
-// policy_rollout.cu: kernel argument block, 16-byte vector access, load pinning, programmatic
-// dependent launch, warp-aggregated episode statistics.
+// drone_device.cuh -- device-side helpers shared by the kernels of drone_kernels.cu, policy_rollout.cu
+// and ppo_kernels.cu: kernel argument block, 16-byte vector access, load pinning, programmatic
+// dependent launch, warp sums, warp-aggregated episode statistics.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -103,7 +103,8 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 // (word 6, env_steps, is derived at collapse time: sum_length + steps of the live episodes.)
 // Integer accumulation makes the totals independent of summation order, hence of grid shape and
 // GPU count.
-__device__ __forceinline__ long long warp_sum_ll(long long v) {
+template <typename T>                                   // sum over the 32 lanes of a converged warp
+__device__ __forceinline__ T warp_sum(T v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
@@ -126,7 +127,7 @@ __device__ __forceinline__ void stats_warp_commit(unsigned long long* stats, uin
     const unsigned landed = __ballot_sync(0xffffffffu, (f & DD_LANDED) != 0u);
     const unsigned crashed = __ballot_sync(0xffffffffu, (f & DD_CRASHED) != 0u);
     const unsigned trunc = __ballot_sync(0xffffffffu, (f & DD_TRUNCATED) != 0u);
-    const long long rsum = warp_sum_ll(f ? return_fx(ret) : 0ll);
+    const long long rsum = warp_sum(f ? return_fx(ret) : 0ll);
     const unsigned len = __reduce_add_sync(0xffffffffu, f ? (unsigned)steps : 0u);
     if ((threadIdx.x & 31) == 0) {
         const unsigned gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -159,7 +160,7 @@ struct StatsAcc {
         if (nd == 0u) return;                              // warp-uniform
         const unsigned nl = __reduce_add_sync(0xffffffffu, landed), nc = __reduce_add_sync(0xffffffffu, crashed),
                        nt = __reduce_add_sync(0xffffffffu, trunc);
-        const long long lsum = warp_sum_ll((long long)len), rsum = warp_sum_ll(ret);
+        const long long lsum = warp_sum((long long)len), rsum = warp_sum(ret);
         if ((threadIdx.x & 31) == 0) {
             const unsigned gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
             unsigned long long* s = stats + (gw % DD_STATS_SLOTS) * DD_STATS_WORDS;

@@ -17,7 +17,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string.h>
-#include <utility>
 #include "drone_device.cuh"
 #include "host_guard.h"
 
@@ -361,7 +360,7 @@ __global__ void __launch_bounds__(kBlock) live_steps_kernel(const int32_t* steps
     unsigned long long t = 0;
     for (int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (int64_t)gridDim.x * kBlock)
         if (!(flags[i] & DD_DONE)) t += (unsigned long long)steps[i];
-    t = (unsigned long long)warp_sum_ll((long long)t);
+    t = (unsigned long long)warp_sum((long long)t);
     if ((threadIdx.x & 31) == 0 && t) atomicAdd(out + 6, t);
 }
 
@@ -400,19 +399,6 @@ static int fill_args(KArgs<R>& a, const DDState* s, const DDParams* p, const DDE
 
 static inline int check_stride(int32_t stride) {
     return (stride == DD_OBS_DIM || stride == kMaxObsStride) ? 0 : DD_E_RANGE;
-}
-
-// One launch, optionally as a programmatic dependent of the previous kernel in the stream.
-template <typename... KP, typename... AP>
-static int launch(void (*kern)(KP...), int grid, int block, cudaStream_t st, bool pdl, AP&&... args)
-{
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-    return (int)cudaLaunchKernelEx(&cfg, kern, std::forward<AP>(args)...);
 }
 
 template <typename R>

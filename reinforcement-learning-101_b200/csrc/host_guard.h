@@ -1,4 +1,5 @@
-// host_guard.h -- host-side helper of the C ABI: run a call on the device that owns its stream / buffers.
+// host_guard.h -- host-side helpers of the C ABI: run a call on the device that owns its stream / buffers, and
+// launch a kernel, optionally as a programmatic dependent of the previous kernel in the stream.
 //
 // The ABI promises "safe to call on any device": a launch on a stream of device B while device A is current
 // fails with an invalid resource handle, so every entry point that enqueues work switches to the owning
@@ -8,6 +9,7 @@
 //     (cudaPointerGetAttributes), or the current one when `ptr` is not device memory.
 #pragma once
 #include <cuda_runtime.h>
+#include <utility>
 
 namespace dd {
 
@@ -46,5 +48,19 @@ private:
         if (err == cudaSuccess && prev != device) { err = cudaSetDevice(device); switched = err == cudaSuccess; }
     }
 };
+
+// One launch, optionally as a programmatic dependent of the previous kernel in the stream (the kernel then calls
+// pdl_wait() before it reads what that kernel wrote, drone_device.cuh).
+template <typename... KP, typename... AP>
+inline int launch(void (*kern)(KP...), int grid, int block, cudaStream_t st, bool pdl, AP&&... args)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = 0; cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
+    return (int)cudaLaunchKernelEx(&cfg, kern, std::forward<AP>(args)...);
+}
 
 }  // namespace dd

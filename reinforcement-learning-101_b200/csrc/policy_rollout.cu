@@ -88,10 +88,7 @@
 namespace dd {
 
 constexpr int kTile = 128;                     // envs per tile == UMMA M == TMEM lanes
-#ifndef DD_K5_GROUPS
-#define DD_K5_GROUPS 4
-#endif
-constexpr int kGroups = DD_K5_GROUPS;          // tiles per CTA (4 = all 512 TMEM columns; fewer only for experiments)
+constexpr int kGroups = 4;                     // tiles per CTA: 4 x 128 columns = all 512 TMEM columns
 constexpr int kPolThreads = kTile * kGroups;   // 512
 constexpr int kH1 = 128, kH2 = 128, kH3 = 64, kIn = 15, kInPad = 16, kOut = 3;
 
@@ -117,25 +114,7 @@ static_assert(offsetof(DDPolicyConsts, beta1) == pBe1 * 4 && offsetof(DDPolicyCo
               offsetof(DDPolicyConsts, w3) == pW3 * 4 && offsetof(DDPolicyConsts, b3) == pB3 * 4 &&
               offsetof(DDPolicyConsts, operands) == pFmt * 4, "DDPolicyConsts layout");
 constexpr float kGammaFloor = 1e-12f;                      // |gamma| below this is treated as +-1e-12
-#ifndef DD_K5_CHUNK
-#define DD_K5_CHUNK 16
-#endif
-#ifndef DD_K5_TS_LAYER3
-#define DD_K5_TS_LAYER3 1                      // layer 3 reads its A operand from TMEM (tcgen05.mma "TS" form), see the header comment
-#endif
-#ifndef DD_K5_TRACE
-#define DD_K5_TRACE 0                          // profiling only: CTA 0 records globaltimer-free clock64 stamps per tile / step / phase
-#endif
-#ifndef DD_K5_ABLATE
-#define DD_K5_ABLATE 0                         // profiling only (wrong results): 1 no MMA issue, 2 no env step, 4 no Philox,
-#endif                                         //   8 no output stores / obs staging, 16 no LayerNorm pass 1, 32 no pass 2, 64 / 128 one beta / w3 constant for all columns
-#ifndef DD_K5_MMA_HEAD
-#define DD_K5_MMA_HEAD 1                       // policy head (64 -> 3) as a fourth tcgen05.mma (TS form) instead of 96 FFMA2 + 64 FMNMX + 48 LDCU per env-step
-#endif
-#ifndef DD_K5_FLUSH_AT
-#define DD_K5_FLUSH_AT 1                       // which MMA shadow hosts the previous step's deferred outputs (1 or 3)
-#endif
-constexpr int kChunk = DD_K5_CHUNK;                        // accumulator columns per tcgen05.ld (8, 16 or 32; 16 measured best)
+constexpr int kChunk = 16;                                 // accumulator columns per tcgen05.ld (8, 16 and 32 measured: 16 best)
 
 constexpr int kABytes = kTile * kH1 * 2;                   // 32 KB: A tile of one group (A0 aliases its head)
 constexpr int kSmemBlob = 0;
@@ -148,14 +127,6 @@ constexpr int kSmemObs = kSmemBar + 80;                             //   contigu
                                                                     //   (bar area: 4 MMA + 4 obs-load mbarriers, TMEM base)
 constexpr int kSmemTotal = kSmemObs + kGroups * kObsTileBytes;      // 225,344 of the 232,448 B
 static_assert(kSmemTotal <= 227 * 1024, "shared memory budget");
-
-#if DD_K5_TRACE
-constexpr int kTraceSteps = 24, kTracePts = 12;
-__device__ long long g_k5_trace[4][kTraceSteps][kTracePts];
-#define DD_TRACE(pt) do { if (blockIdx.x == 0 && (threadIdx.x & 127) == 0 && t >= 100 && t < 100 + kTraceSteps) g_k5_trace[g][t - 100][pt] = clock64(); } while (0)
-#else
-#define DD_TRACE(pt) do { } while (0)
-#endif
 
 struct PArgs {
     DDPolicyConsts pc;     // per-column LN parameters + last layer: constant bank -> uniform operands
@@ -243,7 +214,6 @@ __host__ __device__ constexpr uint32_t umma_idesc(int M, int N, bool f16) {
     return (1u << 4) | (f16 ? 0u : ((1u << 7) | (1u << 10))) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if (DD_K5_ABLATE & 1) return;
     asm volatile("{\n\t.reg .pred p;\n\t"
                  "setp.ne.b32 p, %4, 0;\n\t"
                  "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
@@ -252,7 +222,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
 // A operand from tensor memory ("TS" form): row r of the 128 x 16 A block is TMEM lane r, its 16 sixteen-bit elements are
 // the 8 thirty-two-bit columns starting at `tmem_a` (element 2j in the low half of column j).
 __device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if (DD_K5_ABLATE & 1) return;
     asm volatile("{\n\t.reg .pred p;\n\t"
                  "setp.ne.b32 p, %4, 0;\n\t"
                  "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
@@ -268,7 +237,7 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
 }
-// CH (16 or 32) consecutive fp32 columns of this thread's TMEM lane.  Issue and wait are split so the next
+// CH (8 or 16) consecutive fp32 columns of this thread's TMEM lane.  Issue and wait are split so the next
 // chunk can be in flight while this one is processed.  `tcgen05.wait::ld` covers every load the thread has
 // issued; the registers are threaded through the wait statements as in/out operands so the compiler
 // cannot schedule a consumer above the wait.
@@ -298,29 +267,6 @@ template <> struct TmemChunk<16> {
         asm volatile("tcgen05.wait::ld.sync.aligned;"
                      : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
                        "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-                     :: "memory");
-    }
-};
-template <> struct TmemChunk<32> {
-    uint32_t r[32];
-    __device__ __forceinline__ void issue(uint32_t taddr) {
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-                     "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-                     "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                       "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-                       "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-                       "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-                     : "r"(taddr) : "memory");
-    }
-    __device__ __forceinline__ void wait() {
-        asm volatile("tcgen05.wait::ld.sync.aligned;"
-                     : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]),
-                       "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-                     :: "memory");
-        asm volatile(""
-                     : "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]),
-                       "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
                      :: "memory");
     }
 };
@@ -367,7 +313,6 @@ __device__ __forceinline__ void ln_epilogue(uint32_t trow, const float (&beta)[N
 #pragma unroll
     for (int j = 0; j < 4; ++j) q[j] = make_float2(0.f, 0.f);
     buf[0].issue(trow);
-    if (!(DD_K5_ABLATE & 16)) {
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
         buf[c & 1].wait();
@@ -378,13 +323,11 @@ __device__ __forceinline__ void ln_epilogue(uint32_t trow, const float (&beta)[N
             q[j & 3] = __ffma2_rn(t, t, q[j & 3]);
         }
     }
-    }
     const float2 qs = __fadd2_rn(__fadd2_rn(q[0], q[1]), __fadd2_rn(q[2], q[3]));     // packed adds: 4 instructions instead of 7
     const float sq = qs.x + qs.y;
     float rstd;                                                            // biased variance, like nn.LayerNorm; the argument is
     asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(rstd) : "f"(fmaf(sq, 1.0f / N, 1e-5f)));   //   >= 1e-5: one MUFU.RSQ, no denormal fix-up
     const float2 r2 = make_float2(rstd, rstd);
-    if (DD_K5_ABLATE & 32) { buf[0].wait(); return; }
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
         buf[c & 1].wait();
@@ -392,7 +335,7 @@ __device__ __forceinline__ void ln_epilogue(uint32_t trow, const float (&beta)[N
         float y[CH];
 #pragma unroll
         for (int j = 0; j < CH / 4; ++j) {
-            const int col = (DD_K5_ABLATE & 64) ? 0 : c * CH + 4 * j;   // compile-time after unrolling: c[0][imm] -> uniform registers
+            const int col = c * CH + 4 * j;                  // compile-time after unrolling: c[0][imm] -> uniform registers
             const float2 y0 = __ffma2_rn(f2_of(buf[c & 1], 2 * j), r2, make_float2(beta[col], beta[col + 1]));
             const float2 y1 = __ffma2_rn(f2_of(buf[c & 1], 2 * j + 1), r2, make_float2(beta[col + 2], beta[col + 3]));
             y[4 * j] = y0.x; y[4 * j + 1] = y0.y; y[4 * j + 2] = y1.x; y[4 * j + 3] = y1.y;
@@ -438,7 +381,7 @@ __device__ __forceinline__ void store_a_chunk_relu_tmem(uint32_t ta, int c, cons
 // probabilities) -- with every launch-constant switch a compile-time constant: predicated-off stores, their address
 // arithmetic and the selects between modes still cost issue slots, and this kernel is bound by them.
 // F16: the operand images in the blob and the activations are fp16 (else bf16); chosen by dd_policy_pack.
-template <bool DEF, int CH, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false>
+template <bool DEF, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false>
 __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __grid_constant__ PArgs pa)
 {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -564,7 +507,6 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
     StatsAcc st;
     struct Pending { float p0, p1, p2, reward, shaped; uint32_t act, oflags; } pend = {};
     auto flush_pending = [&](size_t o_prev) {
-        if (DD_K5_ABLATE & 8) return;
         if (live) {
             if (shaping) pa.shaped_tn[o_prev] = pend.shaped;
             if (out_act) pa.actions_tn[o_prev] = (uint8_t)pend.act;
@@ -584,7 +526,6 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
     for (int32_t t = 0; t < T_mine; ++t) {
         const size_t o = FWD ? (size_t)i : (size_t)t * a.n + i;
         // ---------------- observation -> A0 (bf16, K = 16: 15 inputs + constant 1 for the bias) -------
-        DD_TRACE(0);                                         // step start
         float ob[16];
         const bool tile_in = FWD && tile_bulk_in(tile0);     // warp-uniform: this tile's rows are in s_obs (or on their way)
         if (forward_only) {
@@ -617,9 +558,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
             *reinterpret_cast<uint4*>(s_a + (2 + q) * (kTile * 16) + row * 16) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
         }
         // ---------------- layer 1: D[128x128] = A0[128x16] * W0''^T, split bf16 (3 MMAs) ---------------
-        DD_TRACE(1);                                         // A0 written
         fence_async_smem(); tc_fence_before(); group_bar(g);
-        DD_TRACE(2);                                         // past barrier 1
         if (issuer_warp && elect_one()) {
             tc_fence_after();
             umma_bf16(tmem_d, umma_desc(a_addr, kTile * 16, 128), umma_desc(w0_addr, kH1 * 16, 128), umma_idesc(128, kH1, F16), 0u);      // x_hi W_hi
@@ -633,7 +572,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         }
         // under the first MMA: the observation leaves (staged for the TMA store issued after the next barrier, or
         // directly for ragged / unaligned tiles), and the previous step's deferred outputs
-        if (obs_bulk && !(DD_K5_ABLATE & 8)) {
+        if (obs_bulk) {
 #pragma unroll
             for (int j = 0; j < kIn; ++j) s_obs[row * kIn + j] = ob[j];
         }
@@ -642,14 +581,11 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
 #pragma unroll
             for (int j = 0; j < kIn; ++j) dst[j] = ob[j];
         }
-        if (DD_K5_FLUSH_AT == 1 && !forward_only && t > 0) flush_pending(o - a.n);   // (under the second MMA instead: measured slower, 1.270 vs 1.257 ms)
-        DD_TRACE(3);                                         // shadow work 1 done
+        if (!forward_only && t > 0) flush_pending(o - a.n);   // (under the second MMA instead: measured slower, 1.270 vs 1.257 ms)
         wait_mma(bar, phase, issuer_warp, g);
-        DD_TRACE(4);                                         // MMA1 done
-        ln_epilogue<kH1, CH>(trow, pc.beta0,
-                             [&](int c, const float (&y)[CH]) { store_a_chunk_relu<CH, F16>(s_a, row, c, y); });
+        ln_epilogue<kH1, kChunk>(trow, pc.beta0,
+                             [&](int c, const float (&y)[kChunk]) { store_a_chunk_relu<kChunk, F16>(s_a, row, c, y); });
         // ---------------- layer 2: D[128x128] = A1[128x128] * W1''^T + ones * bias1''^T -----------------
-        DD_TRACE(5);                                         // epilogue 1 done
         fence_async_smem(); tc_fence_before(); group_bar(g);
         if (issuer_warp && elect_one()) {
             tc_fence_after();
@@ -667,27 +603,23 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         }
         U4 rnd = {0u, 0u, 0u, 0u};                           // under the second MMA: this step's Philox draws
         if (!forward_only && need_spawn) { draw_next_spawn(); need_spawn = false; }   // refill after a reset (off the chain)
-        if (!forward_only && !thresholded && !(DD_K5_ABLATE & 4)) {
+        if (!forward_only && !thresholded) {
             // (7 Philox rounds instead of 10: -0.7 %, not taken; one block per pair of steps with 21-bit uniforms, or the ten
             // rounds under / split with MMA3: no gain; the log-prob under MMA2 instead of MMA1: +1.6 %)
             rnd = philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), pa.t0 + (uint32_t)t, 2u,
                                 (uint32_t)a.seed, (uint32_t)(a.seed >> 32));
             pin(rnd.a); pin(rnd.b); pin(rnd.c);
         }
-        DD_TRACE(6);                                         // shadow work 2 done
         wait_mma(bar, phase, issuer_warp, g);
-        DD_TRACE(7);                                         // MMA2 done
-#if DD_K5_TS_LAYER3
         // The activations of layer 2 go to TENSOR memory, not shared memory: A2 (128 lanes x 64 columns of packed 16-bit
         // pairs) overlays the columns [0, 64) of D2 that pass 2 has already consumed (chunk c reads D2 columns
         // [16c, 16c+16) and writes A2 columns [8c, 8c+8)), layer 3 reads its A operand from there (TS form) and
         // accumulates D3 in columns [64, 128).  Shared memory is what bounds this kernel (each SS-form K-block streams
         // 4 KB of A + 4 KB of B through the 128 B/clk port, on top of the epilogues' stores): this takes the 32 KB A2
         // store and the 32 KB A2 operand read of every tile-step off it.
-        ln_epilogue<kH2, CH>(trow, pc.beta1,
-                             [&](int c, const float (&y)[CH]) { store_a_chunk_relu_tmem<CH, F16>(trow, c, y); });
+        ln_epilogue<kH2, kChunk>(trow, pc.beta1,
+                             [&](int c, const float (&y)[kChunk]) { store_a_chunk_relu_tmem<kChunk, F16>(trow, c, y); });
         tmem_st_wait();
-        DD_TRACE(8);                                         // epilogue 2 done
         // ---------------- layer 3: D[128x64] = A2[128x128] (TMEM) * W2''^T + ones * bias2''^T --------------
         if (obs_bulk && issuer_warp && elect_one()) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging tile reusable after this barrier
         tc_fence_before(); group_bar(g);
@@ -700,29 +632,10 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
             umma_bf16(tmem_d + 64u, umma_desc(ones_addr, kTile * 16, 128), umma_desc(w2b_addr, kH3 * 16, 128), umma_idesc(128, kH3, F16), 1u);
             umma_commit(bar);
         }
-#else
-        ln_epilogue<kH2, CH>(trow, pc.beta1,
-                             [&](int c, const float (&y)[CH]) { store_a_chunk_relu<CH, F16>(s_a, row, c, y); });
-        // ---------------- layer 3: D[128x64] = A2[128x128] * W2''^T + ones * bias2''^T ------------------
-        if (obs_bulk && issuer_warp && elect_one()) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging tile reusable after this barrier
-        fence_async_smem(); tc_fence_before(); group_bar(g);
-        if (issuer_warp && elect_one()) {
-            tc_fence_after();
-#pragma unroll
-            for (int j = 0; j < kH2 / 16; ++j)
-                umma_bf16(tmem_d, umma_desc(a_addr + j * 2 * (kTile * 16), kTile * 16, 128),
-                          umma_desc(w2_addr + j * 2 * (kH3 * 16), kH3 * 16, 128), umma_idesc(128, kH3, F16), j > 0 ? 1u : 0u);
-            umma_bf16(tmem_d, umma_desc(ones_addr, kTile * 16, 128), umma_desc(w2b_addr, kH3 * 16, 128), umma_idesc(128, kH3, F16), 1u);
-            umma_commit(bar);
-        }
-#endif
-        constexpr bool mma_head = DD_K5_MMA_HEAD && DD_K5_TS_LAYER3 && HEAD == 3;
+        constexpr bool mma_head = HEAD == 3;                 // the critic's one-row head stays on the CUDA cores, in fp32
         float s_pre = 0.f, c_pre = 1.f;                      // under the third MMA (the fourth with the tensor-core head): sin / cos of the pre-update angle
         if (!forward_only && !mma_head) { Arith<float>::sincos_deg(e.angle, s_pre, c_pre); pin(s_pre); pin(c_pre); }   // (main thrust, drone.py:58-66)
-        if (DD_K5_FLUSH_AT == 3 && !forward_only && t > 0) flush_pending(o - a.n);
-        DD_TRACE(9);                                         // shadow work 3 done
         wait_mma(bar, phase, issuer_warp, g);
-        DD_TRACE(10);                                        // MMA3 done
         float z0, z1, z2;
         if constexpr (mma_head) {
             // ---------------- epilogue 3, then the policy head as a fourth MMA ----------------------------------
@@ -731,7 +644,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
             // accumulates in columns [32, 48): image rows 0-2 hold the high halves of w3 |gamma2|, rows 3-5 the low halves, so
             // logit_o = D4[o] + D4[3 + o] + b3[o] carries only the rounding of the activations.  That replaces 96 FFMA2 + 64
             // FMNMX + 48 LDCU per env-step (15 % of the kernel's instructions) with one more hand-off.
-            ln_epilogue<kH3, CH>(trow + 64u, pc.beta2, [&](int c, const float (&y)[CH]) { store_a_chunk_relu_tmem<CH, F16>(trow, c, y); });
+            ln_epilogue<kH3, kChunk>(trow + 64u, pc.beta2, [&](int c, const float (&y)[kChunk]) { store_a_chunk_relu_tmem<kChunk, F16>(trow, c, y); });
             tmem_st_wait();
             tc_fence_before(); group_bar(g);
             if (issuer_warp && elect_one()) {
@@ -753,12 +666,12 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         } else {
         // ---------------- epilogue 3 + layer 4 (64 -> 3) on the CUDA cores ------------------------------
         float2 za = make_float2(0.f, 0.f), zb = za, zc = za;
-        ln_epilogue<kH3, CH>(trow + (DD_K5_TS_LAYER3 ? 64u : 0u), pc.beta2, [&](int c, const float (&y)[CH]) {
+        ln_epilogue<kH3, kChunk>(trow + 64u, pc.beta2, [&](int c, const float (&y)[kChunk]) {
 #pragma unroll
-            for (int j = 0; j < CH / 4; ++j) {
+            for (int j = 0; j < kChunk / 4; ++j) {
                 const float2 h0 = make_float2(fmaxf(y[4 * j], 0.f), fmaxf(y[4 * j + 1], 0.f));      // ReLU
                 const float2 h1 = make_float2(fmaxf(y[4 * j + 2], 0.f), fmaxf(y[4 * j + 3], 0.f));
-                const int col = (DD_K5_ABLATE & 128) ? 0 : c * CH + 4 * j;
+                const int col = c * kChunk + 4 * j;
                 za = __ffma2_rn(h0, make_float2(pc.w3[0][col], pc.w3[0][col + 1]), za); za = __ffma2_rn(h1, make_float2(pc.w3[0][col + 2], pc.w3[0][col + 3]), za);
                 if (HEAD == 3) {
                     zb = __ffma2_rn(h0, make_float2(pc.w3[1][col], pc.w3[1][col + 1]), zb); zb = __ffma2_rn(h1, make_float2(pc.w3[1][col + 2], pc.w3[1][col + 3]), zb);
@@ -768,7 +681,6 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         });
         z0 = za.x + za.y + pc.b3[0]; z1 = zb.x + zb.y + pc.b3[1]; z2 = zc.x + zc.y + pc.b3[2];
         }
-        DD_TRACE(11);                                        // epilogue 3 + last Linear done
         tc_fence_before();                                   // my TMEM reads are done before the next MMA may overwrite
         // sigmoid with the approximate reciprocal (MUFU.RCP, ~1 ulp): the IEEE division sequence costs ~8 issue slots
         // per output on the chain; the same expression serves the rollout and the forward-only instantiation
@@ -804,7 +716,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         // ---------------- environment step (same code as K1) -------------------------------------------
         uint32_t oflags = pflags;
         float reward = 0.f, shaped = 0.f;
-        if (live && !(pflags & DD_DONE) && !(DD_K5_ABLATE & 2)) {
+        if (live && !(pflags & DD_DONE)) {
             uint32_t f = step_core<float, true, true>(e, act, k, reward, speed, dist, s_pre, c_pre);
             if (!f && max_steps > 0 && e.steps >= max_steps) f = DD_DONE | DD_TRUNCATED;
             oflags = f;
@@ -1011,8 +923,8 @@ static int policy_launch(PArgs& pa, const DDParams& p, int64_t n, bool forward, 
     if (guard.err != cudaSuccess) return (int)guard.err;
     const bool f16 = pa.pc.operands == DD_OPERANDS_FP16;
     if (forward) {
-        kern = pa.head == 1 ? (f16 ? policy_rollout_kernel<true, kChunk, true, 1, false, true> : policy_rollout_kernel<true, kChunk, true, 1, false, false>)
-                            : (f16 ? policy_rollout_kernel<true, kChunk, true, 3, false, true> : policy_rollout_kernel<true, kChunk, true, 3, false, false>);
+        kern = pa.head == 1 ? (f16 ? policy_rollout_kernel<true, true, 1, false, true> : policy_rollout_kernel<true, true, 1, false, false>)
+                            : (f16 ? policy_rollout_kernel<true, true, 3, false, true> : policy_rollout_kernel<true, true, 3, false, false>);
         int sms = 0;
         const cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, guard.dev);
         if (e != cudaSuccess) return (int)e;
@@ -1025,7 +937,7 @@ static int policy_launch(PArgs& pa, const DDParams& p, int64_t n, bool forward, 
         grid = rollout_grid(n, sms);
         const bool fast = pa.mode == DD_ACTION_SAMPLE && pa.inv_temperature == 1.0f && pa.auto_reset && pa.a.stats &&
                           pa.actions_tn && pa.logp_tn && pa.reward_tn && pa.done_tn && pa.obs_tn && !pa.shaped_tn && !pa.probs_tn;
-#define DD_K5(DEF_, FAST_) (f16 ? policy_rollout_kernel<DEF_, kChunk, false, 3, FAST_, true> : policy_rollout_kernel<DEF_, kChunk, false, 3, FAST_, false>)
+#define DD_K5(DEF_, FAST_) (f16 ? policy_rollout_kernel<DEF_, false, 3, FAST_, true> : policy_rollout_kernel<DEF_, false, 3, FAST_, false>)
         kern = def ? (fast ? DD_K5(true, true) : DD_K5(true, false)) : (fast ? DD_K5(false, true) : DD_K5(false, false));
 #undef DD_K5
     }
@@ -1075,10 +987,6 @@ static int forward_common(const void* blob, const DDPolicyConsts* consts, const 
 }  // namespace dd
 
 extern "C" {
-
-#if DD_K5_TRACE
-int dd_k5_trace_read(long long* host_out) { return (int)cudaMemcpyFromSymbol(host_out, dd::g_k5_trace, sizeof(dd::g_k5_trace)); }
-#endif
 
 int dd_policy_pack(const DDPolicy* p, void* blob, DDPolicyConsts* consts, void* stream)
 {

@@ -11,22 +11,13 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "../../include/drone_b200.h"
+#include "drone_device.cuh"
 #include "host_guard.h"
 
 namespace dd {
 
 constexpr int kRedBlock = 256;
 constexpr int kSMs = 148;
-
-// Programmatic dependent launch (same scheme as the step kernels, drone_device.cuh)
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 __global__ void __launch_bounds__(kRedBlock) moments_kernel(const float* __restrict__ x, int64_t n, double* out)
 {
@@ -60,14 +51,14 @@ __global__ void __launch_bounds__(kRedBlock) moments_kernel(const float* __restr
     const int64_t tail0 = head + 4 * n4;
     if (tid < n - tail0) { const double v = x[tail0 + tid]; s += v; q += v * v; }
 
-    s = warp_sum_d(s); q = warp_sum_d(q);
+    s = warp_sum(s); q = warp_sum(q);
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     if (lane == 0) { s_s[w] = s; s_q[w] = q; }
     __syncthreads();
     if (w == 0) {
         s = lane < kRedBlock / 32 ? s_s[lane] : 0.0;
         q = lane < kRedBlock / 32 ? s_q[lane] : 0.0;
-        s = warp_sum_d(s); q = warp_sum_d(q);
+        s = warp_sum(s); q = warp_sum(q);
         if (lane == 0) {
             atomicAdd(out + 1, s);
             atomicAdd(out + 2, q);
@@ -127,28 +118,20 @@ __global__ void __launch_bounds__(kRedBlock) normalize_kernel(const float* __res
 // the launch is bound by DRAM latency / kGaeUnroll instead of DRAM latency per step.
 // Chunks are double-buffered in registers: the loads of chunk c+1 are issued BEFORE chunk c is scanned, so loads
 // stay in flight during the dependent arithmetic and the stores (round 1 issued them only after the scan of the
-// previous chunk: 4.4 TB/s).  A thread owns V adjacent envs (V = 1, 2, 4): one 4V-byte load per array and step
+// previous chunk: 4.4 TB/s).  A thread owns V adjacent envs: one 4V-byte load per array and step
 // instead of V scalar ones, V independent scan chains per thread.  Measured on B200 at 65,536 envs x 250 steps
-// (profiles/r02_gae_variants.jsonl): V = 2, 16-step chunks, 32-thread CTAs is the best register configuration
-// (a thread then keeps 2 x 16 x 18 B in flight); a cp.async shared-memory ring with 4-6 stages per 64-env CTA
+// (profiles/r02_gae_variants.jsonl, V = 1 / 2 / 4 x block x chunk): V = 2, 16-step chunks, 32-thread CTAs is the best
+// register configuration (a thread then keeps 2 x 16 x 18 B in flight); V = 1 serves buffers that are not aligned
+// to the pair or an odd number of envs.  A cp.async shared-memory ring with 4-6 stages per 64-env CTA
 // was tried and is SLOWER (47 us against 39.5: at this size the kernel is a ~33 us stream plus a fixed ~4 us
 // of launch ramp and drain; at 262,144 envs the same kernel runs at 89 % of the measured HBM bandwidth).
 // The launches carry the programmatic-dependent-launch attribute: the CTAs become resident while the previous
 // kernel of the stream drains and wait (griddepcontrol.wait) before their first global access.
 // MOM: the advantage moments (n, sum, sum of squares; K4) are accumulated in the same pass -- the normalisation
 // that follows (Actor_Critic_PPO.ipynb c21:L105) then needs no separate read of the advantage buffer.
-#ifndef DD_GAE_BLOCK
-#define DD_GAE_BLOCK 32
-#endif
-#ifndef DD_GAE_UNROLL
-#define DD_GAE_UNROLL 16
-#endif
-#ifndef DD_GAE_VEC
-#define DD_GAE_VEC 2
-#endif
-constexpr int kGaeBlock = DD_GAE_BLOCK;
-constexpr int kGaeUnroll = DD_GAE_UNROLL;
-constexpr int kGaeVec = DD_GAE_VEC;
+constexpr int kGaeBlock = 32;     // threads per CTA
+constexpr int kGaeUnroll = 16;    // steps per register chunk
+constexpr int kGaeVec = 2;        // envs per thread when every row is aligned to the pair
 
 template <int V> struct VecLd;
 template <> struct VecLd<1> {
@@ -160,11 +143,6 @@ template <> struct VecLd<2> {
     static __device__ __forceinline__ void f(const float* p, float (&o)[2]) { const float2 t = __ldg(reinterpret_cast<const float2*>(p)); o[0] = t.x; o[1] = t.y; }
     static __device__ __forceinline__ void b(const uint8_t* p, uint8_t (&o)[2]) { const uchar2 t = __ldg(reinterpret_cast<const uchar2*>(p)); o[0] = t.x; o[1] = t.y; }
     static __device__ __forceinline__ void st(float* p, const float (&v)[2]) { *reinterpret_cast<float2*>(p) = make_float2(v[0], v[1]); }
-};
-template <> struct VecLd<4> {
-    static __device__ __forceinline__ void f(const float* p, float (&o)[4]) { const float4 t = __ldg(reinterpret_cast<const float4*>(p)); o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w; }
-    static __device__ __forceinline__ void b(const uint8_t* p, uint8_t (&o)[4]) { const uchar4 t = __ldg(reinterpret_cast<const uchar4*>(p)); o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w; }
-    static __device__ __forceinline__ void st(float* p, const float (&v)[4]) { *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]); }
 };
 
 template <int V, int U>
@@ -222,7 +200,7 @@ __global__ void __launch_bounds__(kGaeBlock) gae_kernel(const float* __restrict_
 #pragma unroll
         for (int e = 0; e < V; ++e) gae[e] = 0.0f;
         VecLd<V>::f(val + (int64_t)T * n + i, v_next);
-        constexpr int U = V == 4 ? (kGaeUnroll + 1) / 2 : kGaeUnroll;     // 2 x U x 9V bytes of registers per thread
+        constexpr int U = kGaeUnroll;                                     // 2 x U x 9V bytes of registers per thread
         GaeChunk<V, U> a, b;
         a.load(rew, val, done, T, n, i);
         for (int32_t t1 = T; t1 > 0; t1 -= 2 * U) {                // two chunks per trip: a = [t1-U, t1), b = [t1-2U, t1-U)
@@ -235,7 +213,7 @@ __global__ void __launch_bounds__(kGaeBlock) gae_kernel(const float* __restrict_
     }
     if (MOM) {                                             // block-level sums, one atomic pair per CTA
         __shared__ double s_s[kGaeBlock / 32 > 0 ? kGaeBlock / 32 : 1], s_q[kGaeBlock / 32 > 0 ? kGaeBlock / 32 : 1];
-        s = warp_sum_d(s); q = warp_sum_d(q);
+        s = warp_sum(s); q = warp_sum(q);
         const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
         if (lane == 0) { s_s[w] = s; s_q[w] = q; }
         __syncthreads();
@@ -294,19 +272,6 @@ __global__ void __launch_bounds__(kGaeBlock) returns_kernel(const float* __restr
     }
 }
 
-// One launch as a programmatic dependent of the previous kernel in the stream.
-template <typename... KP, typename... AP>
-static int launch_pdl(void (*kern)(KP...), int grid, int block, cudaStream_t st, AP... args)
-{
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    return (int)cudaLaunchKernelEx(&cfg, kern, args...);
-}
-
 static inline int wave_grid(int64_t work_items, int per_block, int max_waves_ctas)
 {
     int64_t g = (work_items + per_block - 1) / per_block;
@@ -328,7 +293,7 @@ int dd_moments(const float* x, int64_t n, double* out, void* stream)
     const int grid = dd::wave_grid(n / 4 + 1, dd::kRedBlock * 4, dd::kSMs * 8);    // (4 CTAs per SM measured slower: 16.7 vs 15 us at 16.4 M elements)
     dd::DeviceGuard guard((cudaStream_t)stream, x);
     if (guard.err != cudaSuccess) return (int)guard.err;
-    return dd::launch_pdl(dd::moments_kernel, grid, dd::kRedBlock, (cudaStream_t)stream, x, n, out);
+    return dd::launch(dd::moments_kernel, grid, dd::kRedBlock, (cudaStream_t)stream, true, x, n, out);
 }
 
 int dd_normalize(const float* x, float* y, const double* moments, double eps, int64_t n, void* stream)
@@ -339,7 +304,7 @@ int dd_normalize(const float* x, float* y, const double* moments, double eps, in
     const int grid = dd::wave_grid(n / 4 + 1, dd::kRedBlock * 2, dd::kSMs * 8);
     dd::DeviceGuard guard((cudaStream_t)stream, x);
     if (guard.err != cudaSuccess) return (int)guard.err;
-    return dd::launch_pdl(dd::normalize_kernel, grid, dd::kRedBlock, (cudaStream_t)stream, x, y, moments, eps, n);
+    return dd::launch(dd::normalize_kernel, grid, dd::kRedBlock, (cudaStream_t)stream, true, x, y, moments, eps, n);
 }
 
 int dd_gae_moments(const float* rewards_tn, const float* values_t1n, const uint8_t* dones_tn, float* adv_tn,
@@ -361,10 +326,10 @@ int dd_gae_moments(const float* rewards_tn, const float* values_t1n, const uint8
     const int64_t threads = (n + V - 1) / V;
     const int grid = (int)((threads + dd::kGaeBlock - 1) / dd::kGaeBlock);
     double* const no_mom = nullptr;
-#define DD_GAE_LAUNCH(V_) (moments ? dd::launch_pdl(dd::gae_kernel<V_, true>, grid, dd::kGaeBlock, st, rewards_tn, values_t1n, dones_tn, adv_tn, returns_tn, moments, g, gl, T, n) \
-                                   : dd::launch_pdl(dd::gae_kernel<V_, false>, grid, dd::kGaeBlock, st, rewards_tn, values_t1n, dones_tn, adv_tn, returns_tn, no_mom, g, gl, T, n))
-    return V == 4 ? DD_GAE_LAUNCH(4) : (V == 2 ? DD_GAE_LAUNCH(2) : DD_GAE_LAUNCH(1));
-#undef DD_GAE_LAUNCH
+#define GAE_LAUNCH(V_) (moments ? dd::launch(dd::gae_kernel<V_, true>, grid, dd::kGaeBlock, st, true, rewards_tn, values_t1n, dones_tn, adv_tn, returns_tn, moments, g, gl, T, n) \
+                                : dd::launch(dd::gae_kernel<V_, false>, grid, dd::kGaeBlock, st, true, rewards_tn, values_t1n, dones_tn, adv_tn, returns_tn, no_mom, g, gl, T, n))
+    return V == 2 ? GAE_LAUNCH(2) : GAE_LAUNCH(1);
+#undef GAE_LAUNCH
 }
 
 int dd_gae(const float* rewards_tn, const float* values_t1n, const uint8_t* dones_tn, float* adv_tn,
@@ -382,7 +347,7 @@ int dd_discounted_returns(const float* rewards_tn, const uint8_t* dones_tn, floa
     const int grid = (int)((n + dd::kGaeBlock - 1) / dd::kGaeBlock);
     dd::DeviceGuard guard((cudaStream_t)stream, rewards_tn);
     if (guard.err != cudaSuccess) return (int)guard.err;
-    return dd::launch_pdl(dd::returns_kernel, grid, dd::kGaeBlock, (cudaStream_t)stream, rewards_tn, dones_tn, returns_tn, gamma, T, n);
+    return dd::launch(dd::returns_kernel, grid, dd::kGaeBlock, (cudaStream_t)stream, true, rewards_tn, dones_tn, returns_tn, gamma, T, n);
 }
 
 }  // extern "C"

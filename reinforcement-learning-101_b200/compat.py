@@ -152,7 +152,7 @@ class DroneGamePool:
             e = self.env
             self._h_mask.zero_()
             self._h_mask[i] = 1
-            nv.check(e._lib.dd_reset(C.byref(e._state), C.byref(e.params), C.byref(e._cfg), self._h_mask.data_ptr(),
+            nv.check(e._lib.dd_reset(C.byref(e._state), C.byref(e._params), C.byref(e._cfg), self._h_mask.data_ptr(),
                                      e.obs.data_ptr(), e.obs_stride, self.num_games, e._stream()), "dd_reset")
             e._needs_reset = False
             self._rec_ok[i] = False

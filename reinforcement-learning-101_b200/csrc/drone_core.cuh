@@ -101,6 +101,18 @@ inline R speed2_threshold(R limit) {
     return s;
 }
 
+// Decision margin of step_core's PRE_SC landing shortcut (px): the shortcut and the exact evaluation can round the
+// bottom centre to neighbouring floats -- one ulp of the largest coordinate the world allows apart -- and differ by the
+// polynomial's error (< 1e-6 of half_h) besides.  8 ulps + 1e-5 half_h covers both; 1e-3 is the floor, which is the
+// value for config.py's world (8 ulps of 850 = 4.9e-4 px), so the default-parameter kernels keep it as an immediate.
+inline float pre_sc_margin(const DDParams& p) {
+    const double far = std::fmax(p.width + p.oob_margin, p.height + p.oob_margin);
+    int ex = 0;
+    std::frexp(far, &ex);                                  // far in [2^(ex-1), 2^ex): one float ulp there is 2^(ex-24)
+    const double m = 8.0 * std::ldexp(1.0, ex - 24) + 1e-5 * std::fabs(p.drone_height / 2);
+    return m > 1e-3 ? (float)m : 1e-3f;
+}
+
 template <typename R>
 inline Consts<R> make_consts(const DDParams& p) {
     Consts<R> k = make_consts_base<R>(p);
@@ -195,10 +207,11 @@ struct Env {
 //
 // PRE_SC: the caller already holds (s_pre, c_pre) = sincos_deg(e.angle) of the PRE-update angle -- it does not
 // depend on the action, so the fused policy kernel evaluates it while the network runs.  Same function of
-// the same input: results are bit-identical to the PRE_SC = false instantiation.
+// the same input: results are bit-identical to the PRE_SC = false instantiation, provided `pre_margin` is
+// pre_sc_margin() of the parameters (1e-3 for config.py's).
 template <typename R, bool WANT_SPEED, bool PRE_SC = false>
 DD_HD uint32_t step_core(Env<R>& e, uint32_t act, const Consts<R>& k, R& reward, R& speed, R& dist,
-                         R s_pre = (R)0, R c_pre = (R)0)
+                         R s_pre = (R)0, R c_pre = (R)0, R pre_margin = (R)1e-3)
 {
     using A = Arith<R>;
     R vx = e.vx, vy = e.vy, w = e.angvel, fuel = e.fuel;
@@ -257,10 +270,13 @@ DD_HD uint32_t step_core(Env<R>& e, uint32_t act, const Consts<R>& k, R& reward,
             // The caller holds sin / cos of the PRE-update angle (computed off the critical path).  The post-update
             // angle is that plus w_add (|w_add| is a few degrees), so sin / cos of it follow from the angle-addition
             // formulas and two short polynomials -- no range reduction, no MUFU -- to ~2e-7.  That is only used to
-            // DECIDE: if the bottom-centre point so obtained is farther than 1e-3 px from every edge of the platform
-            // box (the exact evaluation below differs from it by < 1e-4 px), inside / outside is certain and equals the
-            // exact decision bit for bit; otherwise (probability ~1e-5 per test) the exact path runs.  The landing test
-            // sits on the serial chain of the fused policy kernel, where sincospif's latency is paid by the whole tile.
+            // DECIDE: if the bottom-centre point so obtained is farther than pre_margin from every edge of the platform
+            // box, inside / outside is certain and equals the exact decision bit for bit; otherwise the exact path runs.
+            // The exact evaluation below can differ from the shortcut by one float ulp of the coordinates plus the
+            // polynomial's error: < 1e-4 px while |x|, |y| < 2048 (config.py's world: pre_margin = 1e-3, the exact path
+            // runs with probability ~1e-5 per test), but 1.95e-3 px at |x| >= 16384 -- pre_sc_margin() scales the
+            // margin with the world.  The landing test sits on the serial chain of the fused policy kernel, where
+            // sincospif's latency is paid by the whole tile.
             if (A::abs_(w_add) <= (R)8) {
                 const R th = w_add * (R)0.017453292519943295, t2 = th * th;
                 const R sn = th * ((R)1 + t2 * ((R)-0.16666666666666666 + t2 * (R)0.008333333333333333));
@@ -269,7 +285,7 @@ DD_HD uint32_t step_core(Env<R>& e, uint32_t act, const Consts<R>& k, R& reward,
                 const R bxa = x - k.half_h * sa, bya = y + k.half_h * ca;
                 const R x0 = e.px - k.plat_half_w, x1 = e.px + k.plat_half_w, y0 = e.py - k.plat_half_h, y1 = e.py + k.plat_half_h;
                 const R mx = fminf(A::abs_(bxa - x0), A::abs_(bxa - x1)), my = fminf(A::abs_(bya - y0), A::abs_(bya - y1));
-                if (fminf(mx, my) > (R)1e-3) {
+                if (fminf(mx, my) > pre_margin) {
                     decided = true;
                     inside = (x0 <= bxa) && (bxa <= x1) && (y0 <= bya) && (bya <= y1);
                 }

@@ -55,7 +55,8 @@
 //     chain is a few moves; the 10 Philox rounds of the spawn after it run under the second MMA of the following
 //     step), and the landing test -- which a trained policy enters on most tile-steps -- decides from the angle-addition
 //     formulas on the pre-update sin / cos already held, falling back to sincospif only within 1e-3 px of a platform
-//     edge (step_core<.., PRE_SC>: same decisions bit for bit): 1.250 -> 1.220 ms.
+//     edge in config.py's world, a few float ulps of the coordinates in a larger one (step_core<.., PRE_SC>, pre_sc_margin:
+//     same decisions bit for bit): 1.250 -> 1.220 ms.
 // The four tiles of a CTA are independent pipelines, so while one waits for its MMAs the other three
 // keep the CUDA cores busy; work that is not on the chain obs -> network -> action -> env step -> obs runs in
 // the shadow of an MMA, where the warp would otherwise sleep: the previous step's log-prob / output stores
@@ -146,6 +147,7 @@ struct PArgs {
     const float* obs_in;       // forward-only instantiation: [n][15], no env stepping
     int32_t auto_reset;
     int32_t head;              // forward-only: 3 = probs[n][3] (sigmoid, DroneGamerBoi), 1 = values[n] (DroneTeacherBoi)
+    float pre_margin;          // dd::pre_sc_margin of the parameters (the DEF instantiations use its default-world 1e-3)
 };
 
 // ---- raw PTX wrappers -----------------------------------------------------------------------
@@ -717,7 +719,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         uint32_t oflags = pflags;
         float reward = 0.f, shaped = 0.f;
         if (live && !(pflags & DD_DONE)) {
-            uint32_t f = step_core<float, true, true>(e, act, k, reward, speed, dist, s_pre, c_pre);
+            uint32_t f = step_core<float, true, true>(e, act, k, reward, speed, dist, s_pre, c_pre, DEF ? 1e-3f : pa.pre_margin);
             if (!f && max_steps > 0 && e.steps >= max_steps) f = DD_DONE | DD_TRUNCATED;
             oflags = f;
             if (shaping) {
@@ -1044,6 +1046,7 @@ int dd_policy_rollout(const DDState* s, const DDParams* p, const DDEnvConfig* c,
     pa.a.n = (uint32_t)n; pa.a.seed = c->seed; pa.a.env_id_base = c->env_id_base; pa.a.max_steps = c->max_steps; pa.a.shaping = c->shaping;
     pa.a.rand_drone = c->randomize_drone; pa.a.rand_platform = c->randomize_platform;
     pa.a.k = dd::make_consts<float>(*p);
+    pa.pre_margin = dd::pre_sc_margin(*p);
     pa.blob = (const uint8_t*)blob; pa.mode = mode; pa.t0 = t0; pa.T = T;
     pa.inv_temperature = mode == DD_ACTION_SAMPLE ? 1.0f / temperature : 1.0f;
     pa.actions_tn = actions_tn; pa.logp_tn = logp_tn; pa.reward_tn = reward_tn; pa.done_tn = done_tn;

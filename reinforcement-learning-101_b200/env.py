@@ -125,7 +125,7 @@ class BatchedDroneEnv:
         self.num_envs = n = int(num_envs)
         self.dtype = dtype
         self.obs_stride = int(obs_stride)
-        self.params = params if params is not None else nv.default_params()
+        self._params = nv.DDParams.from_buffer_copy(params if params is not None else nv.default_params())
         dev = self.device
         # ---- state in HBM (layout: include/drone_b200.h DDState) ----
         self.pos_vel = torch.zeros(n, 4, dtype=dtype, device=dev)      # x, y, vx, vy
@@ -179,6 +179,21 @@ class BatchedDroneEnv:
         self._plans.clear()
 
     @property
+    def params(self) -> "nv.DDParams":
+        """A COPY of the physics parameters (``DDParams``).  Writing a field of the returned struct changes nothing;
+        assign a whole struct instead (``p = env.params; p.gravity = 0.5; env.params = p``): the setter copies it and
+        drops the resolved step launches, which carry the derived constants, so that every later call -- ``step``,
+        ``reset``, ``observe``, the rollouts -- runs with the new values."""
+        return nv.DDParams.from_buffer_copy(self._params)
+
+    @params.setter
+    def params(self, p: "nv.DDParams") -> None:
+        if not isinstance(p, nv.DDParams):
+            raise TypeError("params must be a DDParams struct")
+        self._params = nv.DDParams.from_buffer_copy(p)
+        self._plans.clear()
+
+    @property
     def launch_flags(self) -> int:
         return self._cfg.launch_flags
 
@@ -207,7 +222,7 @@ class BatchedDroneEnv:
                 m = mask.to(device=self.device).ne(0).to(torch.uint8).contiguous()
                 if m.shape != (self.num_envs,):
                     raise ValueError("mask must have shape [num_envs]")
-            nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self.params), C.byref(self._cfg), _ptr(m),
+            nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self._params), C.byref(self._cfg), _ptr(m),
                                         None, self.obs_stride, self.num_envs, self._stream()), "dd_reset")
             self._needs_reset = False
             return None
@@ -217,7 +232,7 @@ class BatchedDroneEnv:
             if m.shape != (self.num_envs,):
                 raise ValueError("mask must have shape [num_envs]")
             self.observe()                     # rows of unmasked envs: current state
-        nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self.params), C.byref(self._cfg), _ptr(m),
+        nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self._params), C.byref(self._cfg), _ptr(m),
                                     self.obs.data_ptr(), self.obs_stride, self.num_envs, self._stream()), "dd_reset")
         self._needs_reset = False
         return self.obs
@@ -225,7 +240,7 @@ class BatchedDroneEnv:
     def observe(self) -> torch.Tensor:
         """``get_state()`` (game_engine.py:140-177) of every env without stepping."""
         self._packed.fill_(nv.ACT_SKIP)
-        nv.check(self._lib.dd_step(C.byref(self._state), C.byref(self.params), C.byref(self._cfg),
+        nv.check(self._lib.dd_step(C.byref(self._state), C.byref(self._params), C.byref(self._cfg),
                                    self._packed.data_ptr(), self.obs.data_ptr(), self.obs_stride, None, None, None,
                                    None, self.num_envs, self._stream()), "dd_step(observe)")
         return self.obs
@@ -277,7 +292,7 @@ class BatchedDroneEnv:
         pinned host memory for ``step_host(zero_copy=True)``)."""
         plan = nv.DDStepPlan()
         nv.check(self._lib.dd_step_plan(
-            C.byref(self._state), C.byref(self.params), C.byref(self._cfg),
+            C.byref(self._state), C.byref(self._params), C.byref(self._cfg),
             (self.obs.data_ptr() if obs is None else obs) if want_obs else None, self.obs_stride,
             self.reward.data_ptr() if reward is None else reward, self.step_flags.data_ptr() if flags is None else flags,
             _ptr(self.final_obs), self.stats_slots.data_ptr() if stats else None, self.num_envs, C.byref(plan)), "dd_step_plan")
@@ -344,7 +359,7 @@ class BatchedDroneEnv:
             self._fresh_prev_dist()
         t0 = self._take_t0(t0, T) if pol == nv.POLICY_RANDOM else int(t0 or 0)
         nv.check(self._lib.dd_rollout_shaped(
-            C.byref(self._state), C.byref(self.params), C.byref(self._cfg), pol, _ptr(actions), int(t0), int(T),
+            C.byref(self._state), C.byref(self._params), C.byref(self._cfg), pol, _ptr(actions), int(t0), int(T),
             _ptr(reward_out), _ptr(done_out), _ptr(obs_out), self.obs_stride, _ptr(shaped_out),
             self.stats_slots.data_ptr() if stats else None, n, self._stream()), "dd_rollout")
 
@@ -415,7 +430,7 @@ class BatchedDroneEnv:
         self.set_state({
             "x": x, "y": y, "platform_x": platform_x, "platform_y": platform_y,
             "vx": z, "vy": z, "angle": z, "angular_velocity": z, "total_reward": z,
-            "fuel": torch.full((n,), float(self.params.max_fuel), dtype=self.dtype, device=dev),
+            "fuel": torch.full((n,), float(self._params.max_fuel), dtype=self.dtype, device=dev),
             "steps": torch.zeros(n, dtype=torch.int32, device=dev),
             "flags": torch.zeros(n, dtype=torch.uint8, device=dev),
             "episode": self.episode + 1,

@@ -165,7 +165,7 @@ def policy_rollout(env: BatchedDroneEnv, blob: PolicyBlob, T: int, sample: bool 
         env._fresh_prev_dist()
     t0 = env._take_t0(t0, T)
     nv.check(nv.lib().dd_policy_rollout(
-        C.byref(env._state), C.byref(env.params), C.byref(env._cfg), blob.blob.data_ptr(), C.byref(blob.consts),
+        C.byref(env._state), C.byref(env._params), C.byref(env._cfg), blob.blob.data_ptr(), C.byref(blob.consts),
         ACTION_SAMPLE if sample else ACTION_THRESHOLD, float(temperature), int(t0), int(T), ptr("actions"), ptr("logp"), ptr("reward"),
         ptr("done"), ptr("obs"), ptr("probs"), ptr("shaped"), env.stats_slots.data_ptr() if stats else None, n,
         env._stream()),

@@ -222,6 +222,20 @@ class ShardedDroneEnv:
             e.max_steps = v
         self._drop_graphs()
 
+    @property
+    def params(self) -> "nv.DDParams":
+        """A copy of the physics parameters of the shards (``BatchedDroneEnv.params``)."""
+        return self.shards[0].params
+
+    @params.setter
+    def params(self, p: "nv.DDParams") -> None:
+        """New physics parameters for every shard; the captured graphs embed the old constants and are dropped.  Set
+        them here, not on one shard: the graphs of this class would keep replaying a shard's old launches."""
+        self.join()
+        for e in self.shards:
+            e.params = p
+        self._drop_graphs()
+
     # ---- statistics / state -------------------------------------------------------------------------------------
     def stats_tensor(self) -> torch.Tensor:
         self.join()

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define DD_ABI_VERSION 5
+#define DD_ABI_VERSION 6
 
 /* ---- flag byte (per-step output and persistent state) ---------------------- */
 #define DD_DONE        0x01u   /* game_engine.py:53  self.done            */
@@ -67,6 +67,18 @@ extern "C" {
                                        kernel itself waits (griddepcontrol.wait) before its first load */
 #define DD_LAUNCH_BLOCK_128  0x10   /* dd_step CTA size (default 256) */
 #define DD_LAUNCH_BLOCK_512  0x20
+
+/* ---- DDEnvConfig.obs_format ---------------------------------------------------- */
+/* Element format of the observation outputs (obs, final_obs, obs_tn) of dd_reset, dd_step, dd_step_plan and
+ * dd_rollout / dd_rollout_shaped.  A 16-bit format writes uint16 bit patterns: every value is the one the same env
+ * writes with DD_OBS_NATIVE, converted float -> 16 bit with round-to-nearest-even (what torch's .to(torch.float16) /
+ * .to(torch.bfloat16) produce).  State, rewards, flags and statistics are unchanged.  DD_F32 state only (DD_F64 with a
+ * 16-bit format: DD_E_DTYPE); an unknown value: DD_E_RANGE.  With obs_stride 16 the `steps` column is converted too,
+ * so it is exact only up to 2048 (fp16) or 256 (bf16).
+ * dd_policy_rollout and dd_gather_env ignore the field: their observations are always in the state precision. */
+#define DD_OBS_NATIVE 0     /* the state precision (R) -- what a zero-initialised DDEnvConfig selects */
+#define DD_OBS_F16    1     /* IEEE binary16 */
+#define DD_OBS_BF16   2     /* bfloat16 */
 
 /* error codes */
 #define DD_E_NULL    (-1)
@@ -136,6 +148,8 @@ typedef struct DDEnvConfig {
     int32_t randomize_platform; /* DroneGame(randomize_platform=...) */
     int32_t launch_flags;    /* DD_LAUNCH_* bits; 0 = plain stream-ordered launch */
     int32_t shaping;         /* which notebook's client-side calc_reward the `shaped` outputs follow: DD_SHAPING_* */
+    int32_t obs_format;      /* DD_OBS_*: element format of the observation outputs */
+    int32_t reserved2;
 } DDEnvConfig;
 
 int  dd_abi_version(void);
@@ -143,7 +157,8 @@ void dd_default_params(DDParams *p);                 /* config.py defaults */
 const char *dd_error_string(int code);
 
 /* DroneGame.reset (game_engine.py:59-93) for every env with mask[i] != 0 (mask == NULL: all).
- * obs (nullable): R[n][obs_stride] first observation of the new episode. */
+ * obs (nullable): R[n][obs_stride] first observation of the new episode (uint16[n][obs_stride] under a 16-bit
+ * c->obs_format, as for every obs / final_obs / obs_tn below). */
 int dd_reset(const DDState *s, const DDParams *p, const DDEnvConfig *c, const uint8_t *mask,
              void *obs, int32_t obs_stride, int64_t n, void *stream);
 
@@ -212,7 +227,8 @@ int dd_stats_collapse(const uint64_t *stats, const int32_t *steps, const uint8_t
  * socket API costs one small copy instead of ten:  [0..15] obs row of env i (obs_stride 15: [15] = steps),
  * [16] reward and [17] flags of the last dd_step, [18] persistent flags, [19] steps, [20] episode,
  * [21..24] pos_vel, [25..28] att_fuel, [29..30] platform, [31] 0.   `out` may be device memory or pinned
- * (device-mapped) host memory; obs / reward / step_flags may be NULL (zeros). */
+ * (device-mapped) host memory; obs / reward / step_flags may be NULL (zeros).  `obs` is in the state precision (there
+ * is no DDEnvConfig here: 16-bit observation rows cannot be read). */
 #define DD_ENV_RECORD_DOUBLES 32
 int dd_gather_env(const DDState *s, const void *obs, int32_t obs_stride, const void *reward,
                   const uint8_t *step_flags, int64_t i, int64_t n, double *out, void *stream);
@@ -301,7 +317,8 @@ int dd_value_forward(const void *blob, const DDPolicyConsts *consts, const float
 /* `temperature` (DD_ACTION_SAMPLE, > 0): actions ~ Bernoulli(p^(1/tau) / (p^(1/tau) + (1-p)^(1/tau))) = Bernoulli(sigmoid(logit / tau)),
  * the evaluation sampling of evaluate_policy_simple (Actor_Critic_PPO.ipynb c18); 1 = the policy's own distribution
  * (collect_episodes_ppo).  probs / logp outputs always describe the untempered policy. */
-/* T steps of {observe, policy, act, step} in one launch; DD_F32 state only.  Optional [T][n] outputs:
+/* T steps of {observe, policy, act, step} in one launch; DD_F32 state only; c->obs_format is ignored (obs_tn is fp32:
+ * the critic's first layer reads these rows at full precision).  Optional [T][n] outputs:
  * actions (DD_ACT_* bits), logp (sum of the 3 Bernoulli log-probs), reward, done flags, obs [T][n][15],
  * probs [T][n][3], shaped (the notebook's training reward; needs s->prev_dist; c->shaping must be a DD_SHAPING_*
  * value, else DD_E_RANGE).

@@ -16,6 +16,8 @@
  *   - DD_F32: bit-identical to the device kernels except where sin / cos enter (the device uses sincospif,
  *     the host rounds a float64 libm result; <= 1 ulp apart) and expf of the `pg` shaping.
  *     DD_F64: every product and sum rounded separately like the device path; libm sin / cos.
+ *   - c->obs_format is honoured as on the device: 16-bit rows are the fp32 rows converted by the portable
+ *     round-to-nearest-even routine that stands in for the kernels' hardware conversion.
  */
 #ifndef DRONE_B200_HOST_H
 #define DRONE_B200_HOST_H
@@ -39,6 +41,9 @@ int dd_rollout_host(const DDState *s, const DDParams *p, const DDEnvConfig *c, i
                     const uint8_t *actions_tn, uint32_t t0, int32_t T,
                     void *reward_tn, uint8_t *done_tn, void *obs_tn, int32_t obs_stride, void *shaped_tn,
                     uint64_t *stats, int64_t n);
+
+/* out[i] = x[i] as DD_OBS_F16 / DD_OBS_BF16 bits (fmt): the conversion of the 16-bit observation formats. */
+int dd_obs16_convert_host(int32_t fmt, const float *x, uint16_t *out, int64_t n);
 
 #ifdef __cplusplus
 }

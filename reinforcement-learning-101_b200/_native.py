@@ -27,7 +27,7 @@ HOST_TWIN_SOURCE = "host_twin.cpp"
 HOST_TWIN_FLAGS = ("-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared")
 
 # ---- constants of include/drone_b200.h ------------------------------------------------------
-ABI_VERSION = 5
+ABI_VERSION = 6
 DONE, LANDED, CRASHED, TRUNCATED = 0x01, 0x02, 0x04, 0x08
 CAUSE_MASK, CAUSE_GROUND, CAUSE_FUEL, CAUSE_OOB = 0x30, 0x10, 0x20, 0x30
 ACT_MAIN, ACT_LEFT, ACT_RIGHT, ACT_SKIP = 0x01, 0x02, 0x04, 0x80
@@ -40,6 +40,7 @@ SHAPING_PPO, SHAPING_PG = 0, 1
 RETURN_FIXED_SCALE = 1048576.0
 LAUNCH_PDL, LAUNCH_BLOCK_128, LAUNCH_BLOCK_512 = 0x01, 0x10, 0x20
 OPERANDS_AUTO, OPERANDS_BF16, OPERANDS_FP16 = 0, 1, 2
+OBS_NATIVE, OBS_F16, OBS_BF16 = 0, 1, 2
 
 _PARAM_FIELDS = (
     "width", "height", "gravity", "drag", "angular_drag", "drone_height", "main_thrust", "side_thrust",
@@ -70,6 +71,7 @@ class DDEnvConfig(C.Structure):
         ("max_steps", C.c_int32), ("auto_reset", C.c_int32),
         ("randomize_drone", C.c_int32), ("randomize_platform", C.c_int32),
         ("launch_flags", C.c_int32), ("shaping", C.c_int32),
+        ("obs_format", C.c_int32), ("reserved2", C.c_int32),
     ]
 
 
@@ -223,4 +225,4 @@ EXPORTS = (
     "dd_fill_random_actions", "dd_pack_actions", "dd_stats_collapse", "dd_moments", "dd_normalize", "dd_gae", "dd_gae_moments",
     "dd_policy_pack", "dd_policy_pack_ex", "dd_policy_forward", "dd_policy_rollout", "dd_policy_rollout_grid", "dd_value_pack", "dd_value_forward", "dd_gather_env", "dd_discounted_returns",
 )
-HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host")
+HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host", "dd_obs16_convert_host")

@@ -10,6 +10,7 @@
 //   game_engine.py:140-177  observation normalisation
 #pragma once
 #include <stdint.h>
+#include <string.h>
 #include <math.h>
 #include <cmath>
 #include "../../include/drone_b200.h"
@@ -328,6 +329,79 @@ DD_HD void write_obs(const Env<R>& e, uint32_t flags, R speed, R dist, const Con
     put(12, A::div(speed, k.vel_norm, k.inv_vel));
     put(13, (flags & DD_LANDED) ? (R)1 : (R)0);
     put(14, (flags & DD_CRASHED) ? (R)1 : (R)0);
+}
+
+// ---------------------------------------------------------------------------------------
+// 16-bit observation formats (DDEnvConfig.obs_format): float -> binary16 / bfloat16 bits, round to nearest even --
+// the bits torch's .to(torch.float16) / .to(torch.bfloat16) give.  The kernels convert a pair per instruction
+// (cvt.rn.f16x2.f32 / cvt.rn.bf16x2.f32, SASS F2FP); the host twin uses the portable routines below, which give the
+// same bits for every input but NaN (a quiet NaN either way).
+// ---------------------------------------------------------------------------------------
+inline uint16_t f16_bits_rn_portable(float f)
+{
+    uint32_t x;
+    memcpy(&x, &f, 4);
+    const uint32_t sign = (x >> 16) & 0x8000u, ax = x & 0x7fffffffu;
+    if (ax >= 0x7f800000u) return (uint16_t)(sign | (ax > 0x7f800000u ? 0x7e00u : 0x7c00u));   // NaN / inf
+    if (ax >= 0x477ff000u) return (uint16_t)(sign | 0x7c00u);          // >= 65520 (the 65504 / 65536 tie) -> inf
+    if (ax < 0x38800000u) {                                            // |f| < 2^-14: subnormal or zero, units of 2^-24
+        if (ax <= 0x33000000u) return (uint16_t)sign;                  // <= 2^-25 (the tie goes to the even 0)
+        const uint32_t e = ax >> 23, m = (ax & 0x7fffffu) | 0x800000u, sh = 126u - e;   // sh in [14, 24]
+        uint32_t r = m >> sh;
+        const uint32_t rem = m & ((1u << sh) - 1u), half = 1u << (sh - 1u);
+        if (rem > half || (rem == half && (r & 1u))) ++r;
+        return (uint16_t)(sign | r);
+    }
+    const uint32_t y = ax - 0x38000000u;                               // re-bias the exponent: 127 -> 15
+    uint32_t r = y >> 13;
+    const uint32_t rem = y & 0x1fffu;
+    if (rem > 0x1000u || (rem == 0x1000u && (r & 1u))) ++r;            // a carry into the exponent is correct
+    return (uint16_t)(sign | r);
+}
+
+inline uint16_t bf16_bits_rn_portable(float f)
+{
+    uint32_t x;
+    memcpy(&x, &f, 4);
+    if ((x & 0x7fffffffu) > 0x7f800000u) return (uint16_t)0x7fc0u;    // NaN
+    return (uint16_t)((x + 0x7fffu + ((x >> 16) & 1u)) >> 16);
+}
+
+// Bits 0-15: lo, bits 16-31: hi, in format FMT (DD_OBS_F16 / DD_OBS_BF16).
+template <int FMT>
+DD_HD uint32_t obs16_pack2(float lo, float hi)
+{
+    static_assert(FMT == DD_OBS_F16 || FMT == DD_OBS_BF16, "16-bit observation format");
+#if defined(__CUDA_ARCH__)
+    uint32_t r;
+    if (FMT == DD_OBS_F16) asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    else asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+#else
+    if (FMT == DD_OBS_F16) return (uint32_t)f16_bits_rn_portable(lo) | ((uint32_t)f16_bits_rn_portable(hi) << 16);
+    return (uint32_t)bf16_bits_rn_portable(lo) | ((uint32_t)bf16_bits_rn_portable(hi) << 16);
+#endif
+}
+
+// One observation row in a 16-bit format: write_obs's 15 values (+ `steps_col`: column 15 = `steps`) converted in pairs.
+// `put16(j, bits)` stores element j.
+template <int FMT, typename Put16>
+DD_HD void write_obs16(const Env<float>& e, uint32_t flags, float speed, float dist, const Consts<float>& k,
+                       bool steps_col, float steps, Put16 put16)
+{
+    float v[16];
+    write_obs(e, flags, speed, dist, k, [&](int j, float x) { v[j] = x; });
+    v[15] = steps;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int j = 0; j < 14; j += 2) {
+        const uint32_t w = obs16_pack2<FMT>(v[j], v[j + 1]);
+        put16(j, (uint16_t)w); put16(j + 1, (uint16_t)(w >> 16));
+    }
+    const uint32_t w = obs16_pack2<FMT>(v[14], v[15]);
+    put16(14, (uint16_t)w);
+    if (steps_col) put16(DD_OBS_DIM, (uint16_t)(w >> 16));
 }
 
 template <typename R>

@@ -47,13 +47,25 @@ __device__ __forceinline__ void obs_tile_store(const R* s_obs, R* g_tile, int ro
     }
 }
 
+// ---- observation element format (DDEnvConfig.obs_format) ---------------------------------------
+// OF = DD_OBS_NATIVE: elements of type R, stored as the kernels always have.  OF = DD_OBS_F16 / DD_OBS_BF16 (float
+// state only): uint16 bit patterns, converted in pairs by write_obs16; the KArgs / RArgs pointers (obs, final_obs,
+// obs_tn) then hold uint16 buffers and are cast here.
+template <typename R, int OF> struct ObsElem { using type = uint16_t; };
+template <typename R> struct ObsElem<R, DD_OBS_NATIVE> { using type = R; };
+template <typename R, int OF> using obs_elem_t = typename ObsElem<R, OF>::type;
+
+template <int OF, typename R>
+__device__ __forceinline__ obs_elem_t<R, OF>* obs_ptr(R* p) { return reinterpret_cast<obs_elem_t<R, OF>*>(p); }
+
 // =================================================================================================
 // K1: one step per env per launch.
 // =================================================================================================
-template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK>
+template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK, int OF>
 __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KArgs<R> a)
 {
-    __shared__ __align__(128) R s_obs[OBS ? BLOCK * kMaxObsStride : 1];
+    using O = obs_elem_t<R, OF>;
+    __shared__ __align__(128) O s_obs[OBS ? BLOCK * kMaxObsStride : 1];
     const Consts<R> k = consts_of<R, DEF>(a);
 
     const uint32_t tile0 = blockIdx.x * BLOCK;
@@ -82,9 +94,10 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
             if (f) {                                           // rare: ~1 % of env-steps
                 f_stat = f; ret_stat = e.ret; len_stat = e.steps;
                 if (a.final_obs) {                             // terminal observation (scattered rows)
-                    R* fo = a.final_obs + (size_t)i * a.obs_stride;
+                    O* fo = obs_ptr<OF>(a.final_obs) + (size_t)i * a.obs_stride;
                     if (!OBS) speed = Arith<R>::sqrt_(Arith<R>::fma_(e.vx, e.vx, Arith<R>::mul(e.vy, e.vy)));
-                    write_obs(e, f, speed, dist, k, [&](int j, R v) { fo[j] = v; });
+                    if constexpr (OF == DD_OBS_NATIVE) write_obs(e, f, speed, dist, k, [&](int j, R v) { fo[j] = v; });
+                    else write_obs16<OF>(e, f, speed, dist, k, false, 0.0f, [&](int j, O v) { fo[j] = v; });
                 }
                 if (AUTO) {                                    // same-step reset
                     const uint32_t ep = a.episode[i];
@@ -106,9 +119,14 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
         if (a.reward) a.reward[i] = reward;
         if (a.done_flags) a.done_flags[i] = (uint8_t)oflags;
         if (OBS) {
-            R* row = s_obs + threadIdx.x * a.obs_stride;
-            write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
-            if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;     // 16th key: 'steps'
+            O* row = s_obs + threadIdx.x * a.obs_stride;
+            if constexpr (OF == DD_OBS_NATIVE) {
+                write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
+                if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;     // 16th key: 'steps'
+            } else {
+                write_obs16<OF>(e, pflags, speed, dist, k, a.obs_stride > DD_OBS_DIM, (float)e.steps,
+                                [&](int j, O v) { row[j] = v; });
+            }
         }
     } else {
         pdl_launch_dependents();
@@ -118,7 +136,7 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
     if (OBS) {
         const uint32_t rem = a.n - tile0;
         const int rows = rem < (uint32_t)BLOCK ? (int)rem : BLOCK;
-        obs_tile_store<R, BLOCK>(s_obs, a.obs + (size_t)tile0 * a.obs_stride, rows, a.obs_stride);
+        obs_tile_store<O, BLOCK>(s_obs, obs_ptr<OF>(a.obs) + (size_t)tile0 * a.obs_stride, rows, a.obs_stride);
     }
 }
 
@@ -127,7 +145,7 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
 // =================================================================================================
 constexpr int kBlock = 256;
 
-template <typename R>
+template <typename R, int OF>
 __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ KArgs<R> a, const uint8_t* mask)
 {
     const uint32_t i = blockIdx.x * kBlock + threadIdx.x;
@@ -145,9 +163,13 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ K
     if (a.obs) {
         R speed, dist;
         speed_dist(e, speed, dist);
-        R* row = a.obs + (size_t)i * a.obs_stride;
-        write_obs(e, 0u, speed, dist, a.k, [&](int j, R v) { row[j] = v; });
-        if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)0;
+        obs_elem_t<R, OF>* row = obs_ptr<OF>(a.obs) + (size_t)i * a.obs_stride;
+        if constexpr (OF == DD_OBS_NATIVE) {
+            write_obs(e, 0u, speed, dist, a.k, [&](int j, R v) { row[j] = v; });
+            if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)0;
+        } else {
+            write_obs16<OF>(e, 0u, speed, dist, a.k, a.obs_stride > DD_OBS_DIM, 0.0f, [&](int j, uint16_t v) { row[j] = v; });
+        }
     }
 }
 
@@ -171,10 +193,11 @@ struct RArgs {
 // per-step path is throughput.
 // OUTS = false: no per-step [T][n] outputs (reward / done / shaped) -- the pure statistics rollout of the curriculum
 // sweep and the throughput bench -- compiles their address arithmetic and predicated stores away.
-template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS>
+template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS, int OF>
 __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__ RArgs<R> ra)
 {
-    __shared__ __align__(128) R s_obs[OBS ? kBlock * kMaxObsStride : 1];
+    using O = obs_elem_t<R, OF>;
+    __shared__ __align__(128) O s_obs[OBS ? kBlock * kMaxObsStride : 1];
     const KArgs<R>& a = ra.a;
     const Consts<R> k = consts_of<R, DEF>(a);
     const uint32_t tile0 = blockIdx.x * kBlock;
@@ -261,13 +284,18 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
             if (out_rew) ra.reward_tn[o] = reward;
             if (out_done) ra.done_tn[o] = (uint8_t)oflags;
             if (OBS) {
-                R* row = s_obs + threadIdx.x * a.obs_stride;
-                write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
-                if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;
+                O* row = s_obs + threadIdx.x * a.obs_stride;
+                if constexpr (OF == DD_OBS_NATIVE) {
+                    write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
+                    if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;
+                } else {
+                    write_obs16<OF>(e, pflags, speed, dist, k, a.obs_stride > DD_OBS_DIM, (float)e.steps,
+                                    [&](int j, O v) { row[j] = v; });
+                }
             }
         }
         if (OBS) {
-            obs_tile_store<R, kBlock>(s_obs, ra.obs_tn + ((size_t)t * a.n + tile0) * a.obs_stride, rows, a.obs_stride);
+            obs_tile_store<O, kBlock>(s_obs, obs_ptr<OF>(ra.obs_tn) + ((size_t)t * a.n + tile0) * a.obs_stride, rows, a.obs_stride);
             __syncthreads();                                   // tile is reused next step
         }
     };
@@ -401,6 +429,17 @@ static inline int check_stride(int32_t stride) {
     return (stride == DD_OBS_DIM || stride == kMaxObsStride) ? 0 : DD_E_RANGE;
 }
 
+// DDEnvConfig.obs_format, checked before any CUDA call: DD_E_RANGE for an unknown value, DD_E_DTYPE for a 16-bit format
+// with float64 state (the exact-parity instantiation writes its own precision only).  NULL structs are left to the
+// callee's checks.
+static int check_obs_format(const DDState* s, const DDEnvConfig* c)
+{
+    if (!s || !c) return 0;
+    if (c->obs_format < DD_OBS_NATIVE || c->obs_format > DD_OBS_BF16) return DD_E_RANGE;
+    if (c->obs_format != DD_OBS_NATIVE && s->dtype != DD_F32) return DD_E_DTYPE;
+    return 0;
+}
+
 template <typename R>
 static int reset_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask,
                       void* obs, int32_t obs_stride, int64_t n, cudaStream_t st)
@@ -412,7 +451,12 @@ static int reset_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c,
     if (n == 0) return 0;
     DeviceGuard g(st, s->pos_vel);
     if (g.err != cudaSuccess) return (int)g.err;
-    return launch(reset_kernel<R>, grid_for(n, kBlock), kBlock, st, (c->launch_flags & DD_LAUNCH_PDL) != 0, a, mask);
+    const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0;
+    if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
+        if (c->obs_format == DD_OBS_F16) return launch(reset_kernel<R, DD_OBS_F16>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+        if (c->obs_format == DD_OBS_BF16) return launch(reset_kernel<R, DD_OBS_BF16>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+    }
+    return launch(reset_kernel<R, DD_OBS_NATIVE>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
 }
 
 // The resolved launch of one dd_step call: what dd_step_plan stores in the caller's DDStepPlan.
@@ -427,14 +471,25 @@ constexpr uint32_t kPlanMagic = 0x44445034u;               // "DDP4"
 static_assert(sizeof(StepPlanT<double>) <= DD_STEP_PLAN_BYTES && sizeof(StepPlanT<float>) <= DD_STEP_PLAN_BYTES,
               "DD_STEP_PLAN_BYTES too small for the argument block");
 
-template <typename R, bool AUTO, bool OBS, bool DEF>
+template <typename R, bool AUTO, bool OBS, bool DEF, int OF>
 static void (*step_kernel_of(int block))(KArgs<R>)
 {
     if constexpr (sizeof(R) == 4) {                        // CTA-size variants: float only (tuning knob)
-        if (block == 128) return step_kernel<R, AUTO, OBS, DEF, 128>;
-        if (block == 512) return step_kernel<R, AUTO, OBS, DEF, 512>;
+        if (block == 128) return step_kernel<R, AUTO, OBS, DEF, 128, OF>;
+        if (block == 512) return step_kernel<R, AUTO, OBS, DEF, 512, OF>;
     }
-    return step_kernel<R, AUTO, OBS, DEF, 256>;
+    return step_kernel<R, AUTO, OBS, DEF, 256, OF>;
+}
+
+template <typename R, int OF>
+static void (*step_kernel_sel(bool au, bool ob, bool def, int block))(KArgs<R>)
+{
+#define DD_STEP(AU, OB, DF) step_kernel_of<R, AU, OB, DF, OF>(block)
+    if (def) return au ? (ob ? DD_STEP(true, true, true) : DD_STEP(true, false, true))
+                       : (ob ? DD_STEP(false, true, true) : DD_STEP(false, false, true));
+    return au ? (ob ? DD_STEP(true, true, false) : DD_STEP(true, false, false))
+              : (ob ? DD_STEP(false, true, false) : DD_STEP(false, false, false));
+#undef DD_STEP
 }
 
 // Validate a dd_step call and resolve it to (kernel, grid, block, argument block).
@@ -454,12 +509,11 @@ static int step_resolve(StepPlanT<R>& pl, const DDState* s, const DDParams* p, c
     if (sizeof(R) != 4) block = 256;
     pl.magic = kPlanMagic; pl.dtype = sizeof(R) == 4 ? DD_F32 : DD_F64; pl.device = -1;
     pl.block = block; pl.grid = grid_for(n, block); pl.pdl = (c->launch_flags & DD_LAUNCH_PDL) ? 1 : 0;
-#define DD_STEP(AU, OB, DF) step_kernel_of<R, AU, OB, DF>(block)
-    if (def) pl.kern = au ? (ob ? DD_STEP(true, true, true) : DD_STEP(true, false, true))
-                          : (ob ? DD_STEP(false, true, true) : DD_STEP(false, false, true));
-    else     pl.kern = au ? (ob ? DD_STEP(true, true, false) : DD_STEP(true, false, false))
-                          : (ob ? DD_STEP(false, true, false) : DD_STEP(false, false, false));
-#undef DD_STEP
+    pl.kern = step_kernel_sel<R, DD_OBS_NATIVE>(au, ob, def, block);
+    if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
+        if (c->obs_format == DD_OBS_F16) pl.kern = step_kernel_sel<R, DD_OBS_F16>(au, ob, def, block);
+        if (c->obs_format == DD_OBS_BF16) pl.kern = step_kernel_sel<R, DD_OBS_BF16>(au, ob, def, block);
+    }
     return 0;
 }
 
@@ -513,13 +567,17 @@ static int rollout_impl(const DDState* s, const DDParams* p, const DDEnvConfig* 
     const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0, def = params_are_default(*p);
     const int g = grid_for(n, kBlock);
     const bool outs = reward_tn || done_tn || shaped_tn;
-#define DD_ROLL2(OBS_, DEF_, OUTS_)                                                                                          \
-    (policy == DD_POLICY_TRACE    ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_TRACE, OUTS_>, g, kBlock, st, pdl, ra)    \
-     : policy == DD_POLICY_RANDOM ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_RANDOM, OUTS_>, g, kBlock, st, pdl, ra)   \
-                                  : launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_BANGBANG, OUTS_>, g, kBlock, st, pdl, ra))
-#define DD_ROLL(OBS_, DEF_) (outs ? DD_ROLL2(OBS_, DEF_, true) : DD_ROLL2(OBS_, DEF_, false))
-    if (def) return obs_tn ? DD_ROLL(true, true) : DD_ROLL(false, true);
-    return obs_tn ? DD_ROLL(true, false) : DD_ROLL(false, false);
+#define DD_ROLL2(OBS_, DEF_, OUTS_, OF_)                                                                                          \
+    (policy == DD_POLICY_TRACE    ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_TRACE, OUTS_, OF_>, g, kBlock, st, pdl, ra)    \
+     : policy == DD_POLICY_RANDOM ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_RANDOM, OUTS_, OF_>, g, kBlock, st, pdl, ra)   \
+                                  : launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_BANGBANG, OUTS_, OF_>, g, kBlock, st, pdl, ra))
+#define DD_ROLL(OBS_, DEF_, OF_) (outs ? DD_ROLL2(OBS_, DEF_, true, OF_) : DD_ROLL2(OBS_, DEF_, false, OF_))
+    if constexpr (sizeof(R) == 4) {                        // 16-bit obs_tn: float state only
+        if (obs_tn && c->obs_format == DD_OBS_F16) return def ? DD_ROLL(true, true, DD_OBS_F16) : DD_ROLL(true, false, DD_OBS_F16);
+        if (obs_tn && c->obs_format == DD_OBS_BF16) return def ? DD_ROLL(true, true, DD_OBS_BF16) : DD_ROLL(true, false, DD_OBS_BF16);
+    }
+    if (def) return obs_tn ? DD_ROLL(true, true, DD_OBS_NATIVE) : DD_ROLL(false, true, DD_OBS_NATIVE);
+    return obs_tn ? DD_ROLL(true, false, DD_OBS_NATIVE) : DD_ROLL(false, false, DD_OBS_NATIVE);
 #undef DD_ROLL
 #undef DD_ROLL2
 }
@@ -552,6 +610,7 @@ int dd_reset(const DDState* s, const DDParams* p, const DDEnvConfig* c, const ui
              void* obs, int32_t obs_stride, int64_t n, void* stream)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32) return dd::reset_impl<float>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
     if (s->dtype == DD_F64) return dd::reset_impl<double>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
     return DD_E_DTYPE;
@@ -562,6 +621,7 @@ int dd_step(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uin
             uint64_t* stats, int64_t n, void* stream)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
         return dd::step_impl<float>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
     if (s->dtype == DD_F64)
@@ -574,6 +634,7 @@ int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void
 {
     if (!s || !plan) return DD_E_NULL;
     if (s->dtype != DD_F32 && s->dtype != DD_F64) return DD_E_DTYPE;
+    if (int rc = dd::check_obs_format(s, c)) { memset(plan, 0, sizeof *plan); return rc; }
     memset(plan, 0, sizeof *plan);
     int rc, *device;
     if (s->dtype == DD_F32) {
@@ -607,6 +668,7 @@ int dd_rollout_shaped(const DDState* s, const DDParams* p, const DDEnvConfig* c,
                       void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n, void* stream)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
         return dd::rollout_impl<float>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
     if (s->dtype == DD_F64)

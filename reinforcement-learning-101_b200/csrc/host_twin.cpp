@@ -68,6 +68,35 @@ void stats_commit(uint64_t* st, uint32_t f, R ret, int32_t steps)
 
 inline int check_stride(int32_t stride) { return (stride == DD_OBS_DIM || stride == 16) ? 0 : DD_E_RANGE; }
 
+// check_obs_format of drone_kernels.cu
+inline int check_obs_format(const DDState* s, const DDEnvConfig* c)
+{
+    if (!s || !c) return 0;
+    if (c->obs_format < DD_OBS_NATIVE || c->obs_format > DD_OBS_BF16) return DD_E_RANGE;
+    if (c->obs_format != DD_OBS_NATIVE && s->dtype != DD_F32) return DD_E_DTYPE;
+    return 0;
+}
+
+// Row r of an observation buffer in format `fmt` (DD_OBS_*; 16-bit formats: float state only): write_obs, or
+// write_obs16 as the kernels' 16-bit instantiations call it.  steps_col: column 15 = `steps`.
+template <typename R>
+void obs_row(void* base, int64_t r, int32_t stride, int32_t fmt, const Env<R>& e, uint32_t flags, R speed, R dist,
+             const Consts<R>& k, bool steps_col, R steps)
+{
+    if constexpr (sizeof(R) == 4) {
+        if (fmt != DD_OBS_NATIVE) {
+            uint16_t* row = (uint16_t*)base + r * stride;
+            auto put = [&](int j, uint16_t v) { row[j] = v; };
+            if (fmt == DD_OBS_F16) write_obs16<DD_OBS_F16>(e, flags, speed, dist, k, steps_col, steps, put);
+            else write_obs16<DD_OBS_BF16>(e, flags, speed, dist, k, steps_col, steps, put);
+            return;
+        }
+    }
+    R* row = (R*)base + r * stride;
+    write_obs(e, flags, speed, dist, k, [&](int j, R v) { row[j] = v; });
+    if (steps_col) row[DD_OBS_DIM] = steps;
+}
+
 template <typename R>
 int reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask, void* obs_, int32_t stride, int64_t n)
 {
@@ -75,7 +104,7 @@ int reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const 
     if (int rc = bind(h, s, p, c, n)) return rc;
     if (obs_) if (int rc = check_stride(stride)) return rc;
     const Consts<R> k = make_consts<R>(*p);
-    R* obs = (R*)obs_;
+    void* obs = obs_;
     for (int64_t i = 0; i < n; ++i) {                                  // reset_kernel
         if (mask && !mask[i]) continue;
         Env<R> e;
@@ -89,9 +118,7 @@ int reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const 
         if (obs) {
             R speed, dist;
             speed_dist(e, speed, dist);
-            R* row = obs + i * stride;
-            write_obs(e, 0u, speed, dist, k, [&](int j, R v) { row[j] = v; });
-            if (stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)0;
+            obs_row(obs, i, stride, c->obs_format, e, 0u, speed, dist, k, stride > DD_OBS_DIM, (R)0);
         }
     }
     return 0;
@@ -106,7 +133,8 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
     if (!actions && n > 0) return DD_E_NULL;
     if (obs_ || final_obs_) if (int rc = check_stride(stride)) return rc;
     const Consts<R> k = make_consts<R>(*p);
-    R *obs = (R*)obs_, *reward_out = (R*)reward_, *final_obs = (R*)final_obs_;
+    void *obs = obs_, *final_obs = final_obs_;
+    R* reward_out = (R*)reward_;
     const bool AUTO = c->auto_reset != 0, OBS = obs != nullptr;
     for (int64_t i = 0; i < n; ++i) {                                  // step_kernel, one "thread" at a time
         Env<R> e;
@@ -122,10 +150,7 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
             oflags = f;
             if (f) {
                 stats_commit(stats, f, e.ret, e.steps);
-                if (final_obs) {
-                    R* fo = final_obs + i * stride;
-                    write_obs(e, f, speed, dist, k, [&](int j, R v) { fo[j] = v; });
-                }
+                if (final_obs) obs_row(final_obs, i, stride, c->obs_format, e, f, speed, dist, k, false, (R)0);
                 if (AUTO) {
                     const uint32_t ep = h.episode[i];
                     spawn(e, k, c->seed, c->env_id_base + (uint64_t)i, ep, c->randomize_drone != 0, c->randomize_platform != 0);
@@ -144,11 +169,7 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
         }
         if (reward_out) reward_out[i] = reward;
         if (done_flags) done_flags[i] = (uint8_t)oflags;
-        if (OBS) {
-            R* row = obs + i * stride;
-            write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
-            if (stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;
-        }
+        if (OBS) obs_row(obs, i, stride, c->obs_format, e, pflags, speed, dist, k, stride > DD_OBS_DIM, (R)e.steps);
     }
     return 0;
 }
@@ -167,7 +188,8 @@ int rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, int3
     if (shaped_tn_ && !s->prev_dist && n > 0) return DD_E_NULL;
     if (shaped_tn_ && c->shaping != DD_SHAPING_PPO && c->shaping != DD_SHAPING_PG) return DD_E_RANGE;
     const Consts<R> k = make_consts<R>(*p);
-    R *reward_tn = (R*)reward_tn_, *obs_tn = (R*)obs_tn_, *shaped_tn = (R*)shaped_tn_;
+    R *reward_tn = (R*)reward_tn_, *shaped_tn = (R*)shaped_tn_;
+    void* obs_tn = obs_tn_;
     const bool OBS = obs_tn != nullptr, shaping = shaped_tn != nullptr, auto_reset = c->auto_reset != 0;
     const int32_t max_steps = c->max_steps;
     const R nan = std::numeric_limits<R>::quiet_NaN();
@@ -219,11 +241,7 @@ int rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, int3
             if (shaping) shaped_tn[o] = shaped;
             if (reward_tn) reward_tn[o] = reward;
             if (done_tn) done_tn[o] = (uint8_t)oflags;
-            if (OBS) {
-                R* row = obs_tn + o * stride;
-                write_obs(e, pflags, speed, dist, k, [&](int j, R v) { row[j] = v; });
-                if (stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)e.steps;
-            }
+            if (OBS) obs_row(obs_tn, o, stride, c->obs_format, e, pflags, speed, dist, k, stride > DD_OBS_DIM, (R)e.steps);
         }
         store_env(h, i, e);
         h.flags[i] = (uint8_t)pflags;
@@ -243,6 +261,7 @@ int dd_host_abi_version(void) { return DD_ABI_VERSION; }
 int dd_reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask, void* obs, int32_t obs_stride, int64_t n)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32) return reset_host<float>(s, p, c, mask, obs, obs_stride, n);
     if (s->dtype == DD_F64) return reset_host<double>(s, p, c, mask, obs, obs_stride, n);
     return DD_E_DTYPE;
@@ -252,6 +271,7 @@ int dd_step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, cons
                  void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32) return step_host<float>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
     if (s->dtype == DD_F64) return step_host<double>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
     return DD_E_DTYPE;
@@ -261,11 +281,21 @@ int dd_rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, i
                     int32_t T, void* reward_tn, uint8_t* done_tn, void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n)
 {
     if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
         return rollout_host<float>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
     if (s->dtype == DD_F64)
         return rollout_host<double>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
     return DD_E_DTYPE;
+}
+
+int dd_obs16_convert_host(int32_t fmt, const float* x, uint16_t* out, int64_t n)
+{
+    if ((!x || !out) && n > 0) return DD_E_NULL;
+    if ((fmt != DD_OBS_F16 && fmt != DD_OBS_BF16) || n < 0) return DD_E_RANGE;
+    for (int64_t i = 0; i < n; ++i)
+        out[i] = (uint16_t)(fmt == DD_OBS_F16 ? obs16_pack2<DD_OBS_F16>(x[i], 0.0f) : obs16_pack2<DD_OBS_BF16>(x[i], 0.0f));
+    return 0;
 }
 
 }  // extern "C"

@@ -28,6 +28,8 @@ from . import _native as nv
 _STATE_KEYS = ("x", "y", "vx", "vy", "angle", "angular_velocity", "fuel", "total_reward",
                "platform_x", "platform_y", "steps", "episode", "flags", "prev_dist")
 POLICIES = {"trace": nv.POLICY_TRACE, "random": nv.POLICY_RANDOM, "bangbang": nv.POLICY_BANGBANG}
+# observation element dtype -> DDEnvConfig.obs_format (16-bit formats: float32 state only)
+_OBS_FORMATS = {torch.float16: nv.OBS_F16, torch.bfloat16: nv.OBS_BF16}
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -46,19 +48,23 @@ def _current_stream_handle(device: torch.device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
-def _out_layout(n: int, stride: int, dtype: torch.dtype):
-    """Byte offsets of (obs, reward, step_flags, end) inside the packed per-step output block."""
+def _out_layout(n: int, stride: int, dtype: torch.dtype, obs_dtype: Optional[torch.dtype] = None):
+    """Byte offsets of (obs, reward, step_flags, end) inside the packed per-step output block.  ``dtype`` is the state
+    (and reward) dtype, ``obs_dtype`` the observation's (default: ``dtype``)."""
     isz = 4 if dtype == torch.float32 else 8
+    osz = torch.empty((), dtype=obs_dtype or dtype).element_size()
     up = lambda b: -(-b // 256) * 256
-    o_rew = up(n * stride * isz)
+    o_rew = up(n * stride * osz)
     o_flg = o_rew + up(n * isz)
     return 0, o_rew, o_flg, max(o_flg + up(n), 256)
 
 
-def _carve(block: torch.Tensor, layout, n: int, stride: int, dtype: torch.dtype):
+def _carve(block: torch.Tensor, layout, n: int, stride: int, dtype: torch.dtype, obs_dtype: Optional[torch.dtype] = None):
     isz = 4 if dtype == torch.float32 else 8
+    obs_dtype = obs_dtype or dtype
+    osz = torch.empty((), dtype=obs_dtype).element_size()
     o_obs, o_rew, o_flg, _ = layout
-    obs = block[o_obs:o_obs + n * stride * isz].view(dtype).view(n, stride)
+    obs = block[o_obs:o_obs + n * stride * osz].view(obs_dtype).view(n, stride)
     reward = block[o_rew:o_rew + n * isz].view(dtype)
     flags = block[o_flg:o_flg + n]
     return obs, reward, flags
@@ -100,15 +106,30 @@ class BatchedDroneEnv:
     ``DroneGame(render_mode=None, randomize_drone=False, randomize_platform=True)`` defaults are
     kept (game_engine.py:14).  ``dtype=torch.float64`` selects the exact-parity instantiation of the
     kernels (the reference computes in float64); ``torch.float32`` is the throughput one.
+
+    ``obs_dtype``: element dtype of the observations the env hands out (``obs``, ``final_obs``, ``step_host``'s
+    ``io['obs']``, ``rollout(obs_out=...)``).  ``None`` / ``torch.float32``: the state dtype.  ``torch.float16`` /
+    ``torch.bfloat16`` (float32 state only): the kernels write 16-bit rows, each value exactly the float32 one
+    rounded to nearest even (``obs32.to(obs_dtype)``, bit for bit), at half the observation bytes; state, rewards,
+    flags and statistics stay as they are.  With ``obs_stride=16`` the ``steps`` column is converted too: exact up to
+    2048 steps in float16, 256 in bfloat16.  ``policy_rollout`` ignores it (its ``obs`` rows are always float32).
     """
 
     def __init__(self, num_envs: int, device="cuda", seed: int = 0, randomize_drone: bool = False,
                  randomize_platform: bool = True, max_steps: Optional[int] = None, auto_reset: bool = True,
                  dtype: torch.dtype = torch.float32, env_id_base: int = 0, obs_stride: int = nv.OBS_DIM,
                  want_final_obs: bool = False, params: Optional[nv.DDParams] = None, launch_flags: int = 0,
-                 shaping: str = "ppo"):
+                 shaping: str = "ppo", obs_dtype: Optional[torch.dtype] = None):
         if dtype not in (torch.float32, torch.float64):
             raise ValueError("dtype must be torch.float32 or torch.float64")
+        if obs_dtype is None or obs_dtype == dtype or (obs_dtype == torch.float32 and dtype == torch.float32):
+            obs_dtype, obs_format = dtype, nv.OBS_NATIVE
+        elif obs_dtype in _OBS_FORMATS:
+            if dtype != torch.float32:
+                raise ValueError("16-bit observations (obs_dtype float16 / bfloat16) need dtype=torch.float32")
+            obs_format = _OBS_FORMATS[obs_dtype]
+        else:
+            raise ValueError("obs_dtype must be None, torch.float32, torch.float16 or torch.bfloat16")
         if obs_stride not in (15, 16):
             raise ValueError("obs_stride must be 15 or 16")
         if num_envs < 0:
@@ -124,6 +145,7 @@ class BatchedDroneEnv:
         self._lib = nv.lib()
         self.num_envs = n = int(num_envs)
         self.dtype = dtype
+        self.obs_dtype = obs_dtype
         self.obs_stride = int(obs_stride)
         self._params = nv.DDParams.from_buffer_copy(params if params is not None else nv.default_params())
         dev = self.device
@@ -137,10 +159,10 @@ class BatchedDroneEnv:
         self.prev_dist = torch.full((n,), float("nan"), dtype=dtype, device=dev)   # N2 shaping bookkeeping
         # ---- per-step outputs: ONE block [obs | reward | step_flags] (256-byte aligned parts), so that the
         #      host-buffer step moves them with a single device->host copy ----
-        self._out_layout = _out_layout(n, self.obs_stride, dtype)
+        self._out_layout = _out_layout(n, self.obs_stride, dtype, obs_dtype)
         self._out_block = torch.zeros(self._out_layout[-1], dtype=torch.uint8, device=dev)
-        self.obs, self.reward, self.step_flags = _carve(self._out_block, self._out_layout, n, self.obs_stride, dtype)
-        self.final_obs = torch.zeros(n, self.obs_stride, dtype=dtype, device=dev) if want_final_obs else None
+        self.obs, self.reward, self.step_flags = _carve(self._out_block, self._out_layout, n, self.obs_stride, dtype, obs_dtype)
+        self.final_obs = torch.zeros(n, self.obs_stride, dtype=obs_dtype, device=dev) if want_final_obs else None
         self._packed = torch.zeros(n, dtype=torch.uint8, device=dev)
         # ---- episode statistics (K3) ----
         self.stats_slots = torch.zeros(nv.STATS_SLOTS, nv.STATS_WORDS, dtype=torch.int64, device=dev)
@@ -151,7 +173,7 @@ class BatchedDroneEnv:
                                  nv.F32 if dtype == torch.float32 else nv.F64, 0, self.prev_dist.data_ptr())
         self._cfg = nv.DDEnvConfig(int(seed) & (2 ** 64 - 1), int(env_id_base), int(max_steps or 0),
                                    int(bool(auto_reset)), int(bool(randomize_drone)), int(bool(randomize_platform)),
-                                   int(launch_flags), nv.SHAPING_PG if shaping == "pg" else nv.SHAPING_PPO)
+                                   int(launch_flags), nv.SHAPING_PG if shaping == "pg" else nv.SHAPING_PPO, obs_format)
         self.shaping = shaping
         self._needs_reset = True
         self._plans: Dict[tuple, "nv.DDStepPlan"] = {}       # resolved dd_step launches (dd_step_plan), by (want_obs, stats)
@@ -335,7 +357,8 @@ class BatchedDroneEnv:
         """T steps per launch with the env state in registers (one state round trip per launch).
         ``policy``: 'trace' (``actions`` uint8 ``[T,N]``), 'random' (Philox, p=0.5 per thruster;
         examples/random_agent.py:27-31; ``t0=None`` continues this env's noise stream, see ``_take_t0``) or
-        'bangbang' (main = vy > 1.5).  Optional ``[T,N]`` outputs (``obs_out[t]`` = observation AFTER step t);
+        'bangbang' (main = vy > 1.5).  Optional ``[T,N]`` outputs (``obs_out[t]`` = observation AFTER step t, in
+        ``obs_dtype``; ``reward_out`` / ``shaped_out`` in the state dtype);
         ``shaped_out`` receives the PPO notebook's client-side training reward (``calc_reward`` +
         time-out penalty, Actor_Critic_PPO.ipynb c7, c16:L89-93) computed in the same launch."""
         if self._needs_reset:
@@ -350,9 +373,11 @@ class BatchedDroneEnv:
                                ("shaped_out", shaped_out, (T, n)), ("obs_out", obs_out, (T, n, self.obs_stride))):
             if t is not None and (tuple(t.shape) != shape or not t.is_contiguous() or t.device != self.device):
                 raise ValueError(f"{name} must be a contiguous {shape} tensor on {self.device}")
-        for t in (reward_out, obs_out, shaped_out):
+        for t in (reward_out, shaped_out):
             if t is not None and t.dtype != self.dtype:
-                raise ValueError("reward_out / obs_out / shaped_out must have the env dtype")
+                raise ValueError("reward_out / shaped_out must have the env dtype")
+        if obs_out is not None and obs_out.dtype != self.obs_dtype:
+            raise ValueError("obs_out must have the env's obs_dtype")
         if done_out is not None and done_out.dtype != torch.uint8:
             raise ValueError("done_out must be uint8")
         if shaped_out is not None:
@@ -444,7 +469,7 @@ class BatchedDroneEnv:
         same layout as the device's, of which ``obs`` / ``reward`` / ``flags`` are views."""
         n = self.num_envs
         block = torch.zeros(self._out_layout[-1], dtype=torch.uint8, pin_memory=True)
-        obs, reward, flags = _carve(block, self._out_layout, n, self.obs_stride, self.dtype)
+        obs, reward, flags = _carve(block, self._out_layout, n, self.obs_stride, self.dtype, self.obs_dtype)
         return {"actions": torch.zeros(n, dtype=torch.uint8, pin_memory=True), "block": block,
                 "obs": obs, "reward": reward, "flags": flags}
 
@@ -457,7 +482,8 @@ class BatchedDroneEnv:
         (call it under ``torch.cuda.stream(...)`` with one stream per env in flight).
 
         ``mode='copy'``      the kernel writes its packed output block in HBM, ONE device->host copy brings it back
-                             (65 B per env-step: this copy is what bounds the call, PCIe);
+                             (65 B per env-step with float32 observations, 35 B with 16-bit ones: this copy is what
+                             bounds the call, PCIe);
         ``mode='zero_copy'`` the kernel's obs / reward / flags destinations ARE the pinned host buffers (device-mapped
                              under UVA): the observation tile of each CTA leaves the SM as one TMA bulk store straight
                              over PCIe, there is no HBM round trip and no separate copy."""

@@ -22,6 +22,9 @@ c16:L42-108), for both kinds of caller:
     in that order (tested).  ``run`` / ``step_all`` return as soon as the work is enqueued on the env's own chain
     streams; ``join()`` orders the caller's stream behind it.
 
+``env_kw`` goes to every shard's ``BatchedDroneEnv`` (``obs_dtype=torch.bfloat16`` etc.): the observation format is
+part of each shard's resolved step launch, so the graphs replay it like any other argument.
+
 Global env ids are contiguous over the shards (``env_id_base + s * N + i``), so a ShardedDroneEnv of S x N envs is the
 same set of trajectories as one BatchedDroneEnv of S * N envs (Philox is keyed by the global id).
 """

@@ -156,6 +156,42 @@ int  dd_abi_version(void);
 void dd_default_params(DDParams *p);                 /* config.py defaults */
 const char *dd_error_string(int code);
 
+/* ---- per-environment physics parameter sets (domain randomisation, per-group curricula) ----------------------------
+ * The _sets entry points below take a DDParamSets instead of one DDParams: a table of up to DD_MAX_PARAM_SETS derived
+ * parameter sets and a per-env set index.
+ *   Selection.  Env i steps, resets and observes exactly as the same env would under DDParams sets[min(index[i], count-1)]
+ *     through the single-set entry point: spawn ranges and default spawn, max_fuel at reset, terminal rewards, shaping
+ *     constants and observation normalisation.  An out-of-range index is clamped to count-1, never read out of bounds.
+ *   Resampling (flags & DD_PARAM_SETS_RESAMPLE).  Each reset of env i -- masked resets of dd_reset_sets, same-step
+ *     auto-resets of dd_step_sets / dd_rollout_sets -- draws s = mulhi32(r.a, count) with
+ *     r = Philox4x32-10(counter = (env_id lo, env_id hi, episode, 3), key = seed), writes index[i] = s and spawns under
+ *     set s.  `episode` is the counter the spawn itself uses (read before the increment); counter word 3 = 3 is a stream
+ *     no other draw uses (spawns 0, random actions 1, dd_policy_rollout's Bernoulli uniforms 2).  The step that ends an
+ *     episode runs under the old set (its reward, flags and final_obs row); the observation after the auto-reset is
+ *     normalised by the new one.  Without the flag `index` is only read.
+ *   Validation, before any CUDA call: NULL ps, or NULL table / index with n > 0: DD_E_NULL; count outside
+ *     [1, DD_MAX_PARAM_SETS] or unknown flag bits: DD_E_RANGE; ps->dtype != s->dtype: DD_E_DTYPE; table not 16-byte
+ *     aligned: DD_E_ALIGN; and every check of the single-set entry point, with the same codes.
+ *   Plans.  dd_step_plan_sets keeps the table and index POINTERS: in-place edits of index[] or of the table contents
+ *     reach the next dd_step_planned and captured graphs.  A different count or flags value needs a new plan.
+ * dd_policy_rollout and dd_gather_env take no parameter sets. */
+#define DD_MAX_PARAM_SETS      64
+#define DD_PARAM_TABLE_BYTES   32768     /* fixed size: room for 64 sets of the float64 derived constants */
+#define DD_PARAM_SETS_RESAMPLE 0x01
+
+typedef struct DDParamSets {
+    const void *table;       /* device, 16-byte aligned, DD_PARAM_TABLE_BYTES: the bytes dd_param_sets_build wrote */
+    uint8_t *index;          /* device uint8[n]: the set env i runs under (written at resets under RESAMPLE) */
+    int32_t count;           /* 1 .. DD_MAX_PARAM_SETS */
+    int32_t dtype;           /* DD_F32 / DD_F64 the table was built for; must equal DDState.dtype */
+    int32_t flags;           /* DD_PARAM_SETS_* */
+    int32_t reserved;
+} DDParamSets;
+
+/* Pure host function, no CUDA call: derive `count` parameter sets (including the speed-threshold search) in `dtype` into
+ * host_out (DD_PARAM_TABLE_BYTES; unused slots are zero), to be copied to the device table.  The layout is private. */
+int dd_param_sets_build(const DDParams *sets, int32_t count, int32_t dtype, void *host_out);
+
 /* DroneGame.reset (game_engine.py:59-93) for every env with mask[i] != 0 (mask == NULL: all).
  * obs (nullable): R[n][obs_stride] first observation of the new episode (uint16[n][obs_stride] under a 16-bit
  * c->obs_format, as for every obs / final_obs / obs_tn below). */
@@ -206,6 +242,21 @@ int dd_rollout_shaped(const DDState *s, const DDParams *p, const DDEnvConfig *c,
                       const uint8_t *actions_tn, uint32_t t0, int32_t T,
                       void *reward_tn, uint8_t *done_tn, void *obs_tn, int32_t obs_stride, void *shaped_tn,
                       uint64_t *stats, int64_t n, void *stream);
+
+/* dd_reset / dd_step / dd_step_plan / dd_rollout_shaped with per-env parameter sets (DDParamSets above) in place of
+ * DDParams.  A plan made by dd_step_plan_sets is launched by dd_step_planned.  dd_rollout_sets with shaped_tn NULL is
+ * dd_rollout. */
+int dd_reset_sets(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, const uint8_t *mask,
+                  void *obs, int32_t obs_stride, int64_t n, void *stream);
+int dd_step_sets(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, const uint8_t *actions,
+                 void *obs, int32_t obs_stride, void *reward, uint8_t *done_flags, void *final_obs,
+                 uint64_t *stats, int64_t n, void *stream);
+int dd_step_plan_sets(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, void *obs, int32_t obs_stride,
+                      void *reward, uint8_t *done_flags, void *final_obs, uint64_t *stats, int64_t n, DDStepPlan *plan);
+int dd_rollout_sets(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, int32_t policy,
+                    const uint8_t *actions_tn, uint32_t t0, int32_t T,
+                    void *reward_tn, uint8_t *done_tn, void *obs_tn, int32_t obs_stride, void *shaped_tn,
+                    uint64_t *stats, int64_t n, void *stream);
 
 /* [T][n] synthetic random action trace (same bits DD_POLICY_RANDOM uses in-kernel). */
 int dd_fill_random_actions(uint8_t *actions_tn, uint64_t seed, uint64_t env_id_base,

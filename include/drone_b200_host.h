@@ -42,6 +42,20 @@ int dd_rollout_host(const DDState *s, const DDParams *p, const DDEnvConfig *c, i
                     void *reward_tn, uint8_t *done_tn, void *obs_tn, int32_t obs_stride, void *shaped_tn,
                     uint64_t *stats, int64_t n);
 
+/* The _sets entry points of drone_b200.h over host memory: `ps->table` holds the bytes dd_param_sets_build_host (or
+ * the device library's dd_param_sets_build) wrote, `ps->index` is host memory, written at resets under
+ * DD_PARAM_SETS_RESAMPLE.  Same selection, resampling rule and argument codes as on the device. */
+int dd_param_sets_build_host(const DDParams *sets, int32_t count, int32_t dtype, void *host_out);
+int dd_reset_sets_host(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, const uint8_t *mask,
+                       void *obs, int32_t obs_stride, int64_t n);
+int dd_step_sets_host(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, const uint8_t *actions,
+                      void *obs, int32_t obs_stride, void *reward, uint8_t *done_flags, void *final_obs,
+                      uint64_t *stats, int64_t n);
+int dd_rollout_sets_host(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, int32_t policy,
+                         const uint8_t *actions_tn, uint32_t t0, int32_t T,
+                         void *reward_tn, uint8_t *done_tn, void *obs_tn, int32_t obs_stride, void *shaped_tn,
+                         uint64_t *stats, int64_t n);
+
 /* out[i] = x[i] as DD_OBS_F16 / DD_OBS_BF16 bits (fmt): the conversion of the 16-bit observation formats. */
 int dd_obs16_convert_host(int32_t fmt, const float *x, uint16_t *out, int64_t n);
 

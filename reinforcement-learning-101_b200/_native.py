@@ -41,6 +41,7 @@ RETURN_FIXED_SCALE = 1048576.0
 LAUNCH_PDL, LAUNCH_BLOCK_128, LAUNCH_BLOCK_512 = 0x01, 0x10, 0x20
 OPERANDS_AUTO, OPERANDS_BF16, OPERANDS_FP16 = 0, 1, 2
 OBS_NATIVE, OBS_F16, OBS_BF16 = 0, 1, 2
+MAX_PARAM_SETS, PARAM_TABLE_BYTES, PARAM_SETS_RESAMPLE = 64, 32768, 0x01
 
 _PARAM_FIELDS = (
     "width", "height", "gravity", "drag", "angular_drag", "drone_height", "main_thrust", "side_thrust",
@@ -73,6 +74,12 @@ class DDEnvConfig(C.Structure):
         ("launch_flags", C.c_int32), ("shaping", C.c_int32),
         ("obs_format", C.c_int32), ("reserved2", C.c_int32),
     ]
+
+
+class DDParamSets(C.Structure):
+    """Per-env parameter sets of the _sets entry points: device table (dd_param_sets_build's bytes) + uint8 index [n]."""
+    _fields_ = [("table", C.c_void_p), ("index", C.c_void_p), ("count", C.c_int32), ("dtype", C.c_int32),
+                ("flags", C.c_int32), ("reserved", C.c_int32)]
 
 
 class DDStepPlan(C.Structure):
@@ -169,6 +176,17 @@ def lib():
     L.dd_rollout.argtypes = [PS, PP, PC, i32, vp, u32, i32, vp, vp, vp, i32, vp, i64, vp]
     L.dd_rollout_shaped.restype = C.c_int
     L.dd_rollout_shaped.argtypes = [PS, PP, PC, i32, vp, u32, i32, vp, vp, vp, i32, vp, vp, i64, vp]
+    PSS = C.POINTER(DDParamSets)
+    L.dd_param_sets_build.restype = C.c_int
+    L.dd_param_sets_build.argtypes = [PP, i32, i32, vp]
+    L.dd_reset_sets.restype = C.c_int
+    L.dd_reset_sets.argtypes = [PS, PSS, PC, vp, vp, i32, i64, vp]
+    L.dd_step_sets.restype = C.c_int
+    L.dd_step_sets.argtypes = [PS, PSS, PC, vp, vp, i32, vp, vp, vp, vp, i64, vp]
+    L.dd_step_plan_sets.restype = C.c_int
+    L.dd_step_plan_sets.argtypes = [PS, PSS, PC, vp, i32, vp, vp, vp, vp, i64, C.POINTER(DDStepPlan)]
+    L.dd_rollout_sets.restype = C.c_int
+    L.dd_rollout_sets.argtypes = [PS, PSS, PC, i32, vp, u32, i32, vp, vp, vp, i32, vp, vp, i64, vp]
     L.dd_fill_random_actions.restype = C.c_int
     L.dd_fill_random_actions.argtypes = [vp, u64, u64, u32, i32, i64, vp]
     L.dd_pack_actions.restype = C.c_int
@@ -219,10 +237,25 @@ def default_params() -> DDParams:
     return p
 
 
+def build_param_table(sets, dtype: int) -> bytes:
+    """dd_param_sets_build: the DD_PARAM_TABLE_BYTES of 1..64 DDParams structs in DD_F32 / DD_F64 (host bytes)."""
+    sets = list(sets)
+    if not 1 <= len(sets) <= MAX_PARAM_SETS:
+        raise ValueError(f"param_sets must hold 1 to {MAX_PARAM_SETS} DDParams structs")
+    if not all(isinstance(p, DDParams) for p in sets):
+        raise TypeError("param_sets must be DDParams structs")
+    arr = (DDParams * len(sets))(*sets)
+    out = C.create_string_buffer(PARAM_TABLE_BYTES)
+    check(lib().dd_param_sets_build(arr, len(sets), int(dtype), out), "dd_param_sets_build")
+    return out.raw
+
+
 EXPORTS = (
     "dd_abi_version", "dd_default_params", "dd_error_string", "dd_reset", "dd_step", "dd_step_plan", "dd_step_planned",
     "dd_rollout", "dd_rollout_shaped",
+    "dd_param_sets_build", "dd_reset_sets", "dd_step_sets", "dd_step_plan_sets", "dd_rollout_sets",
     "dd_fill_random_actions", "dd_pack_actions", "dd_stats_collapse", "dd_moments", "dd_normalize", "dd_gae", "dd_gae_moments",
     "dd_policy_pack", "dd_policy_pack_ex", "dd_policy_forward", "dd_policy_rollout", "dd_policy_rollout_grid", "dd_value_pack", "dd_value_forward", "dd_gather_env", "dd_discounted_returns",
 )
-HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host", "dd_obs16_convert_host")
+HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host", "dd_obs16_convert_host",
+                     "dd_param_sets_build_host", "dd_reset_sets_host", "dd_step_sets_host", "dd_rollout_sets_host")

@@ -609,6 +609,72 @@ DD_HD void spawn(Env<R>& e, const Consts<R>& k, uint64_t seed, uint64_t env_id, 
     e.fuel = k.max_fuel; e.ret = (R)0; e.steps = 0;
 }
 
+// ---------------------------------------------------------------------------------------
+// Per-env parameter sets (DDParamSets, include/drone_b200.h).  The table is Consts<R> of up to DD_MAX_PARAM_SETS sets
+// laid out [word][set]: word j of set s (words of sizeof(R) bytes; the four uint32 counts pack into whole words) sits
+// at j * DD_MAX_PARAM_SETS + s.  A warp's load of one field touches at most 64 * sizeof(R) contiguous bytes -- two
+// 128-byte lines for float -- whatever mix of sets its lanes hold.  param_sets_build is the table's only writer and
+// param_set its only reader, on the device and in the host twin alike.
+// ---------------------------------------------------------------------------------------
+template <typename R> struct ParamWord { using type = unsigned int; };
+template <> struct ParamWord<double> { using type = unsigned long long; };
+template <typename R> constexpr int kParamWords = (int)(sizeof(Consts<R>) / sizeof(R));
+static_assert(sizeof(Consts<float>) == kParamWords<float> * 4 && sizeof(Consts<double>) == kParamWords<double> * 8,
+              "Consts<R> must be whole words of R");
+static_assert(sizeof(Consts<double>) * DD_MAX_PARAM_SETS <= DD_PARAM_TABLE_BYTES, "DD_PARAM_TABLE_BYTES too small");
+
+// The constants of set `s` (already clamped to count - 1).  Fields the caller does not use are never loaded.
+template <typename R>
+DD_HD Consts<R> param_set(const void* table, uint32_t s)
+{
+    using W = typename ParamWord<R>::type;
+    const W* t = static_cast<const W*>(table) + s;
+    W w[kParamWords<R>];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+    for (int j = 0; j < kParamWords<R>; ++j) w[j] = __ldg(t + j * DD_MAX_PARAM_SETS);
+#else
+    for (int j = 0; j < kParamWords<R>; ++j) w[j] = t[j * DD_MAX_PARAM_SETS];
+#endif
+    Consts<R> k;
+    memcpy(&k, w, sizeof k);
+    return k;
+}
+
+DD_HD uint32_t param_set_clamp(uint32_t index, uint32_t count) { return index < count ? index : count - 1u; }
+
+// Host only: make_consts of sets[0 .. count) into the DD_PARAM_TABLE_BYTES at `out` (unused slots zero).
+template <typename R>
+inline void param_sets_build(const DDParams* sets, int count, void* out)
+{
+    using W = typename ParamWord<R>::type;
+    memset(out, 0, DD_PARAM_TABLE_BYTES);
+    for (int s = 0; s < count; ++s) {
+        const Consts<R> k = make_consts<R>(sets[s]);
+        W w[kParamWords<R>];
+        memcpy(w, &k, sizeof k);
+        for (int j = 0; j < kParamWords<R>; ++j) static_cast<W*>(out)[j * DD_MAX_PARAM_SETS + s] = w[j];
+    }
+}
+
+// dd_param_sets_build (both libraries)
+inline int param_sets_build_checked(const DDParams* sets, int32_t count, int32_t dtype, void* out)
+{
+    if (!sets || !out) return DD_E_NULL;
+    if (count < 1 || count > DD_MAX_PARAM_SETS) return DD_E_RANGE;
+    if (dtype == DD_F32) { param_sets_build<float>(sets, count, out); return 0; }
+    if (dtype == DD_F64) { param_sets_build<double>(sets, count, out); return 0; }
+    return DD_E_DTYPE;
+}
+
+// The set an env resampling at its reset number `episode` draws (DD_PARAM_SETS_RESAMPLE): Philox stream 3.
+DD_HD uint32_t param_set_draw(uint64_t seed, uint64_t env_id, uint32_t episode, uint32_t count)
+{
+    const U4 r = philox4x32_10((uint32_t)env_id, (uint32_t)(env_id >> 32), episode, 3u,
+                               (uint32_t)seed, (uint32_t)(seed >> 32));
+    return mulhi_u32(r.a, count);
+}
+
 // 3-bit synthetic random action of step t (p = 0.5 per thruster).  One Philox call serves 32
 // consecutive steps: action j = t % 32 is bits [3j, 3j+3) of the 96-bit string a | b<<32 | c<<64.
 DD_HD U4 action_block(uint64_t seed, uint64_t env_id, uint32_t t)

@@ -28,6 +28,19 @@ struct KArgs {
     Consts<R> k;
 };
 
+// The argument block of the per-env parameter-set kernels (SETS = true): KArgs (whose `k` they do not read) + the
+// DDParamSets pointers.  Appended, so that the single-set kernels keep their argument layout.
+template <typename R>
+struct KArgsPS : KArgs<R> {
+    const void* ps_table;                 // Consts<R> [word][set], drone_core.cuh param_set
+    uint8_t* ps_index;
+    uint32_t ps_count;
+    int32_t ps_resample;                  // DD_PARAM_SETS_RESAMPLE
+};
+template <typename R, bool SETS> struct KArgsSel { using type = KArgs<R>; };
+template <typename R> struct KArgsSel<R, true> { using type = KArgsPS<R>; };
+template <typename R, bool SETS> using KArgsOf = typename KArgsSel<R, SETS>::type;
+
 // DEF: the parameters are config.py's defaults -> compile-time constants (immediates); otherwise
 // they come from the kernel argument (constant bank).
 template <typename R, bool DEF>

@@ -61,12 +61,15 @@ __device__ __forceinline__ obs_elem_t<R, OF>* obs_ptr(R* p) { return reinterpret
 // =================================================================================================
 // K1: one step per env per launch.
 // =================================================================================================
-template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK, int OF>
-__global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KArgs<R> a)
+// SETS: per-env parameter sets (KArgsPS): env i's constants are set min(index[i], count - 1) of the table, read through
+// L1 after the index byte arrives; under ps_resample each auto-reset draws a new set (param_set_draw) before it spawns.
+template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK, int OF, bool SETS>
+__global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KArgsOf<R, SETS> a)
 {
     using O = obs_elem_t<R, OF>;
     __shared__ __align__(128) O s_obs[OBS ? BLOCK * kMaxObsStride : 1];
-    const Consts<R> k = consts_of<R, DEF>(a);
+    Consts<R> k;
+    if constexpr (!SETS) k = consts_of<R, DEF>(a);
 
     const uint32_t tile0 = blockIdx.x * BLOCK;
     const uint32_t i = tile0 + threadIdx.x;
@@ -80,7 +83,10 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
         uint32_t act = a.actions[i];
         load_env(a, i, e);
         uint32_t pflags = AUTO ? 0u : (uint32_t)a.flags[i];   // persistent flags are always 0 under auto-reset
+        uint32_t set = 0;
+        if constexpr (SETS) set = a.ps_index[i];
         pin(act); pin(pflags);
+        if constexpr (SETS) { pin(set); k = param_set<R>(a.ps_table, param_set_clamp(set, a.ps_count)); }
         pdl_launch_dependents();
 
         uint32_t oflags = pflags;                              // what this step reports
@@ -101,6 +107,13 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
                 }
                 if (AUTO) {                                    // same-step reset
                     const uint32_t ep = a.episode[i];
+                    if constexpr (SETS) {
+                        if (a.ps_resample) {                   // the new episode's set; final_obs above is the old one's
+                            set = param_set_draw(a.seed, a.env_id_base + (uint64_t)i, ep, a.ps_count);
+                            a.ps_index[i] = (uint8_t)set;
+                            k = param_set<R>(a.ps_table, set);
+                        }
+                    }
                     spawn(e, k, a.seed, a.env_id_base + (uint64_t)i, ep, a.rand_drone != 0, a.rand_platform != 0);
                     a.episode[i] = ep + 1;
                     store2(a.platform, i, e.px, e.py);
@@ -145,8 +158,26 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
 // =================================================================================================
 constexpr int kBlock = 256;
 
-template <typename R, int OF>
-__global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ KArgs<R> a, const uint8_t* mask)
+// The constants env i resets under: the launch's (SETS = false) or its set, drawn anew under ps_resample.
+template <typename R, bool SETS>
+__device__ __forceinline__ Consts<R> reset_consts(const KArgsOf<R, SETS>& a, uint32_t i, uint32_t ep)
+{
+    if constexpr (SETS) {
+        uint32_t s;
+        if (a.ps_resample) {
+            s = param_set_draw(a.seed, a.env_id_base + (uint64_t)i, ep, a.ps_count);
+            a.ps_index[i] = (uint8_t)s;
+        } else {
+            s = param_set_clamp(a.ps_index[i], a.ps_count);
+        }
+        return param_set<R>(a.ps_table, s);
+    } else {
+        return a.k;
+    }
+}
+
+template <typename R, int OF, bool SETS>
+__global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ KArgsOf<R, SETS> a, const uint8_t* mask)
 {
     const uint32_t i = blockIdx.x * kBlock + threadIdx.x;
     pdl_wait();
@@ -154,7 +185,8 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ K
     if (mask && !mask[i]) return;
     Env<R> e;
     const uint32_t ep = a.episode[i];
-    spawn(e, a.k, a.seed, a.env_id_base + (uint64_t)i, ep, a.rand_drone != 0, a.rand_platform != 0);
+    const Consts<R> k = reset_consts<R, SETS>(a, i, ep);
+    spawn(e, k, a.seed, a.env_id_base + (uint64_t)i, ep, a.rand_drone != 0, a.rand_platform != 0);
     a.episode[i] = ep + 1;                                     // game_engine.py:91
     store_env(a, i, e);
     store2(a.platform, i, e.px, e.py);
@@ -165,10 +197,10 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ K
         speed_dist(e, speed, dist);
         obs_elem_t<R, OF>* row = obs_ptr<OF>(a.obs) + (size_t)i * a.obs_stride;
         if constexpr (OF == DD_OBS_NATIVE) {
-            write_obs(e, 0u, speed, dist, a.k, [&](int j, R v) { row[j] = v; });
+            write_obs(e, 0u, speed, dist, k, [&](int j, R v) { row[j] = v; });
             if (a.obs_stride > DD_OBS_DIM) row[DD_OBS_DIM] = (R)0;
         } else {
-            write_obs16<OF>(e, 0u, speed, dist, a.k, a.obs_stride > DD_OBS_DIM, 0.0f, [&](int j, uint16_t v) { row[j] = v; });
+            write_obs16<OF>(e, 0u, speed, dist, k, a.obs_stride > DD_OBS_DIM, 0.0f, [&](int j, uint16_t v) { row[j] = v; });
         }
     }
 }
@@ -176,9 +208,9 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ K
 // =================================================================================================
 // Rollout: T steps per launch, env state in registers, one state round trip per launch.
 // =================================================================================================
-template <typename R>
+template <typename R, typename KA = KArgs<R>>
 struct RArgs {
-    KArgs<R> a;
+    KA a;
     const uint8_t* actions_tn;
     R* reward_tn;
     uint8_t* done_tn;
@@ -193,13 +225,16 @@ struct RArgs {
 // per-step path is throughput.
 // OUTS = false: no per-step [T][n] outputs (reward / done / shaped) -- the pure statistics rollout of the curriculum
 // sweep and the throughput bench -- compiles their address arithmetic and predicated stores away.
-template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS, int OF>
-__global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__ RArgs<R> ra)
+// SETS: as in step_kernel; the env's constants stay in registers over the T steps and are reloaded when a resampling
+// auto-reset draws a new set (index[i] is written back once, at the end).
+template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS, int OF, bool SETS>
+__global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__ RArgs<R, KArgsOf<R, SETS>> ra)
 {
     using O = obs_elem_t<R, OF>;
     __shared__ __align__(128) O s_obs[OBS ? kBlock * kMaxObsStride : 1];
-    const KArgs<R>& a = ra.a;
-    const Consts<R> k = consts_of<R, DEF>(a);
+    const auto& a = ra.a;
+    Consts<R> k;
+    if constexpr (!SETS) k = consts_of<R, DEF>(a);
     const uint32_t tile0 = blockIdx.x * kBlock;
     const uint32_t i = tile0 + threadIdx.x;
     const bool live = i < a.n;
@@ -208,13 +243,15 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
 
     pdl_wait();
     Env<R> e = {};
-    uint32_t pflags = 0, ep = 0;
-    bool platform_dirty = false;
+    uint32_t pflags = 0, ep = 0, set = 0;
+    bool platform_dirty = false, set_dirty = false;
     if (live) {
         load_env(a, i, e);
         pflags = a.flags[i];
         ep = a.episode[i];
+        if constexpr (SETS) set = param_set_clamp(a.ps_index[i], a.ps_count);
     }
+    if constexpr (SETS) k = param_set<R>(a.ps_table, set);
     pdl_launch_dependents();
     const uint64_t gid = a.env_id_base + (uint64_t)i;
     // DD_POLICY_RANDOM: the 96 action bits of the current block of 32 steps (action_block) as a shift register --
@@ -268,6 +305,13 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
                 if (f) {
                     if (do_stats) st.add(f, e.ret, e.steps);          // per-thread totals, committed once after the loop
                     if (auto_reset) {
+                        if constexpr (SETS) {
+                            if (a.ps_resample) {
+                                set = param_set_draw(a.seed, gid, ep, a.ps_count);
+                                set_dirty = true;
+                                k = param_set<R>(a.ps_table, set);
+                            }
+                        }
                         spawn(e, k, a.seed, gid, ep, a.rand_drone != 0, a.rand_platform != 0);
                         ep += 1;
                         platform_dirty = true;
@@ -323,6 +367,7 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
         a.episode[i] = ep;
         if (platform_dirty) store2(a.platform, i, e.px, e.py);
         if (shaping) a.prev_dist[i] = dprev;
+        if constexpr (SETS) { if (set_dirty) a.ps_index[i] = (uint8_t)set; }
     }
 }
 
@@ -406,10 +451,11 @@ static bool params_are_default(const DDParams& p)
            speed2_threshold<double>(p.land_speed) == p.land_speed * p.land_speed;
 }
 
+// Everything of the argument block but the constants.
 template <typename R>
-static int fill_args(KArgs<R>& a, const DDState* s, const DDParams* p, const DDEnvConfig* c, int64_t n)
+static int fill_state(KArgs<R>& a, const DDState* s, const DDEnvConfig* c, int64_t n)
 {
-    if (!s || !p || !c) return DD_E_NULL;
+    if (!s || !c) return DD_E_NULL;
     if (n < 0 || n > (int64_t)0x7fffff00) return DD_E_RANGE;          // 32-bit env index inside one call
     if (n > 0 && (!s->pos_vel || !s->att_fuel || !s->platform || !s->steps || !s->episode || !s->flags)) return DD_E_NULL;
     if ((reinterpret_cast<uintptr_t>(s->pos_vel) | reinterpret_cast<uintptr_t>(s->att_fuel)) & 15u) return DD_E_ALIGN;
@@ -421,9 +467,35 @@ static int fill_args(KArgs<R>& a, const DDState* s, const DDParams* p, const DDE
     a.n = (uint32_t)n; a.seed = c->seed; a.env_id_base = c->env_id_base;
     a.max_steps = c->max_steps; a.obs_stride = DD_OBS_DIM; a.shaping = c->shaping;
     a.rand_drone = c->randomize_drone; a.rand_platform = c->randomize_platform;
+    return 0;
+}
+
+template <typename R>
+static int fill_args(KArgs<R>& a, const DDState* s, const DDParams* p, const DDEnvConfig* c, int64_t n)
+{
+    if (!p) return DD_E_NULL;
+    if (int rc = fill_state(a, s, c, n)) return rc;
     a.k = make_consts<R>(*p);
     return 0;
 }
+
+// The DDParamSets checks of include/drone_b200.h, then the argument block of the per-env kernels.
+template <typename R>
+static int fill_args(KArgsPS<R>& a, const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int64_t n)
+{
+    if (!ps) return DD_E_NULL;
+    if (int rc = fill_state(a, s, c, n)) return rc;
+    if (n > 0 && (!ps->table || !ps->index)) return DD_E_NULL;
+    if (ps->count < 1 || ps->count > DD_MAX_PARAM_SETS || (ps->flags & ~DD_PARAM_SETS_RESAMPLE)) return DD_E_RANGE;
+    if (ps->dtype != s->dtype) return DD_E_DTYPE;
+    if (reinterpret_cast<uintptr_t>(ps->table) & 15u) return DD_E_ALIGN;
+    a.ps_table = ps->table; a.ps_index = ps->index;
+    a.ps_count = (uint32_t)ps->count; a.ps_resample = (ps->flags & DD_PARAM_SETS_RESAMPLE) ? 1 : 0;
+    return 0;
+}
+
+// Kernel mode of a call: single-set calls use the immediates when the parameters are config.py's; per-env sets never.
+static bool params_are_default(const DDParamSets&) { return false; }
 
 static inline int check_stride(int32_t stride) {
     return (stride == DD_OBS_DIM || stride == kMaxObsStride) ? 0 : DD_E_RANGE;
@@ -440,11 +512,11 @@ static int check_obs_format(const DDState* s, const DDEnvConfig* c)
     return 0;
 }
 
-template <typename R>
-static int reset_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask,
+template <typename R, bool SETS, typename P>
+static int reset_impl(const DDState* s, const P* p, const DDEnvConfig* c, const uint8_t* mask,
                       void* obs, int32_t obs_stride, int64_t n, cudaStream_t st)
 {
-    KArgs<R> a;
+    KArgsOf<R, SETS> a;
     if (int rc = fill_args(a, s, p, c, n)) return rc;
     if (obs) { if (int rc = check_stride(obs_stride)) return rc; a.obs_stride = obs_stride; }
     a.obs = (R*)obs;
@@ -453,52 +525,54 @@ static int reset_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c,
     if (g.err != cudaSuccess) return (int)g.err;
     const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0;
     if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
-        if (c->obs_format == DD_OBS_F16) return launch(reset_kernel<R, DD_OBS_F16>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
-        if (c->obs_format == DD_OBS_BF16) return launch(reset_kernel<R, DD_OBS_BF16>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+        if (c->obs_format == DD_OBS_F16) return launch(reset_kernel<R, DD_OBS_F16, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+        if (c->obs_format == DD_OBS_BF16) return launch(reset_kernel<R, DD_OBS_BF16, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
     }
-    return launch(reset_kernel<R, DD_OBS_NATIVE>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+    return launch(reset_kernel<R, DD_OBS_NATIVE, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
 }
 
 // The resolved launch of one dd_step call: what dd_step_plan stores in the caller's DDStepPlan.
-template <typename R>
+template <typename R, bool SETS = false>
 struct StepPlanT {
     uint32_t magic;
     int32_t dtype, device, grid, block, pdl;
-    void (*kern)(KArgs<R>);
-    KArgs<R> a;                                            // everything but `actions`
+    void (*kern)(KArgsOf<R, SETS>);
+    KArgsOf<R, SETS> a;                                    // everything but `actions`
 };
 constexpr uint32_t kPlanMagic = 0x44445034u;               // "DDP4"
-static_assert(sizeof(StepPlanT<double>) <= DD_STEP_PLAN_BYTES && sizeof(StepPlanT<float>) <= DD_STEP_PLAN_BYTES,
+constexpr uint32_t kPlanMagicSets = 0x44445334u;           // "DDS4": a plan of dd_step_plan_sets
+static_assert(sizeof(StepPlanT<double, true>) <= DD_STEP_PLAN_BYTES && sizeof(StepPlanT<float, true>) <= DD_STEP_PLAN_BYTES,
               "DD_STEP_PLAN_BYTES too small for the argument block");
 
-template <typename R, bool AUTO, bool OBS, bool DEF, int OF>
-static void (*step_kernel_of(int block))(KArgs<R>)
+template <typename R, bool AUTO, bool OBS, bool DEF, int OF, bool SETS>
+static void (*step_kernel_of(int block))(KArgsOf<R, SETS>)
 {
     if constexpr (sizeof(R) == 4) {                        // CTA-size variants: float only (tuning knob)
-        if (block == 128) return step_kernel<R, AUTO, OBS, DEF, 128, OF>;
-        if (block == 512) return step_kernel<R, AUTO, OBS, DEF, 512, OF>;
+        if (block == 128) return step_kernel<R, AUTO, OBS, DEF, 128, OF, SETS>;
+        if (block == 512) return step_kernel<R, AUTO, OBS, DEF, 512, OF, SETS>;
     }
-    return step_kernel<R, AUTO, OBS, DEF, 256, OF>;
+    return step_kernel<R, AUTO, OBS, DEF, 256, OF, SETS>;
 }
 
-template <typename R, int OF>
-static void (*step_kernel_sel(bool au, bool ob, bool def, int block))(KArgs<R>)
+template <typename R, int OF, bool SETS>
+static void (*step_kernel_sel(bool au, bool ob, bool def, int block))(KArgsOf<R, SETS>)
 {
-#define DD_STEP(AU, OB, DF) step_kernel_of<R, AU, OB, DF, OF>(block)
-    if (def) return au ? (ob ? DD_STEP(true, true, true) : DD_STEP(true, false, true))
-                       : (ob ? DD_STEP(false, true, true) : DD_STEP(false, false, true));
+#define DD_STEP(AU, OB, DF) step_kernel_of<R, AU, OB, DF, OF, SETS>(block)
+    if (!SETS && def)                                      // per-env sets: DEF = false only
+        return au ? (ob ? DD_STEP(true, true, !SETS) : DD_STEP(true, false, !SETS))
+                  : (ob ? DD_STEP(false, true, !SETS) : DD_STEP(false, false, !SETS));
     return au ? (ob ? DD_STEP(true, true, false) : DD_STEP(true, false, false))
               : (ob ? DD_STEP(false, true, false) : DD_STEP(false, false, false));
 #undef DD_STEP
 }
 
 // Validate a dd_step call and resolve it to (kernel, grid, block, argument block).
-template <typename R>
-static int step_resolve(StepPlanT<R>& pl, const DDState* s, const DDParams* p, const DDEnvConfig* c,
+template <typename R, bool SETS, typename P>
+static int step_resolve(StepPlanT<R, SETS>& pl, const DDState* s, const P* p, const DDEnvConfig* c,
                         void* obs, int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs,
                         uint64_t* stats, int64_t n)
 {
-    KArgs<R>& a = pl.a;
+    KArgsOf<R, SETS>& a = pl.a;
     if (int rc = fill_args(a, s, p, c, n)) return rc;
     if (obs || final_obs) { if (int rc = check_stride(obs_stride)) return rc; a.obs_stride = obs_stride; }
     a.obs = (R*)obs; a.reward = (R*)reward; a.final_obs = (R*)final_obs;
@@ -507,22 +581,22 @@ static int step_resolve(StepPlanT<R>& pl, const DDState* s, const DDParams* p, c
     const int bsel = (c->launch_flags >> 4) & 3;
     int block = bsel == 1 ? 128 : (bsel == 2 ? 512 : 256);
     if (sizeof(R) != 4) block = 256;
-    pl.magic = kPlanMagic; pl.dtype = sizeof(R) == 4 ? DD_F32 : DD_F64; pl.device = -1;
+    pl.magic = SETS ? kPlanMagicSets : kPlanMagic; pl.dtype = sizeof(R) == 4 ? DD_F32 : DD_F64; pl.device = -1;
     pl.block = block; pl.grid = grid_for(n, block); pl.pdl = (c->launch_flags & DD_LAUNCH_PDL) ? 1 : 0;
-    pl.kern = step_kernel_sel<R, DD_OBS_NATIVE>(au, ob, def, block);
+    pl.kern = step_kernel_sel<R, DD_OBS_NATIVE, SETS>(au, ob, def, block);
     if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
-        if (c->obs_format == DD_OBS_F16) pl.kern = step_kernel_sel<R, DD_OBS_F16>(au, ob, def, block);
-        if (c->obs_format == DD_OBS_BF16) pl.kern = step_kernel_sel<R, DD_OBS_BF16>(au, ob, def, block);
+        if (c->obs_format == DD_OBS_F16) pl.kern = step_kernel_sel<R, DD_OBS_F16, SETS>(au, ob, def, block);
+        if (c->obs_format == DD_OBS_BF16) pl.kern = step_kernel_sel<R, DD_OBS_BF16, SETS>(au, ob, def, block);
     }
     return 0;
 }
 
-template <typename R>
-static int step_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* actions,
+template <typename R, bool SETS, typename P>
+static int step_impl(const DDState* s, const P* p, const DDEnvConfig* c, const uint8_t* actions,
                      void* obs, int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs,
                      uint64_t* stats, int64_t n, cudaStream_t st)
 {
-    StepPlanT<R> pl;
+    StepPlanT<R, SETS> pl;
     if (int rc = step_resolve(pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n)) return rc;
     if (!actions && n > 0) return DD_E_NULL;
     if (n == 0) return 0;
@@ -532,24 +606,24 @@ static int step_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c, 
     return launch(pl.kern, pl.grid, pl.block, st, pl.pdl != 0, pl.a);
 }
 
-template <typename R>
-static int step_planned(const StepPlanT<R>& pl, const uint8_t* actions, cudaStream_t st)
+template <typename R, bool SETS>
+static int step_planned(const StepPlanT<R, SETS>& pl, const uint8_t* actions, cudaStream_t st)
 {
     if (pl.a.n == 0) return 0;
     if (!actions) return DD_E_NULL;
     DeviceGuard g(pl.device);
     if (g.err != cudaSuccess) return (int)g.err;
-    KArgs<R> a = pl.a;
+    KArgsOf<R, SETS> a = pl.a;
     a.actions = actions;
     return launch(pl.kern, pl.grid, pl.block, st, pl.pdl != 0, a);
 }
 
-template <typename R>
-static int rollout_impl(const DDState* s, const DDParams* p, const DDEnvConfig* c, int32_t policy,
+template <typename R, bool SETS, typename P>
+static int rollout_impl(const DDState* s, const P* p, const DDEnvConfig* c, int32_t policy,
                         const uint8_t* actions_tn, uint32_t t0, int32_t T, void* reward_tn, uint8_t* done_tn,
                         void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n, cudaStream_t st)
 {
-    RArgs<R> ra{};
+    RArgs<R, KArgsOf<R, SETS>> ra{};
     if (int rc = fill_args(ra.a, s, p, c, n)) return rc;
     if (policy < DD_POLICY_TRACE || policy > DD_POLICY_BANGBANG) return DD_E_RANGE;
     if (policy == DD_POLICY_TRACE && !actions_tn && n > 0 && T > 0) return DD_E_NULL;
@@ -568,15 +642,16 @@ static int rollout_impl(const DDState* s, const DDParams* p, const DDEnvConfig* 
     const int g = grid_for(n, kBlock);
     const bool outs = reward_tn || done_tn || shaped_tn;
 #define DD_ROLL2(OBS_, DEF_, OUTS_, OF_)                                                                                          \
-    (policy == DD_POLICY_TRACE    ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_TRACE, OUTS_, OF_>, g, kBlock, st, pdl, ra)    \
-     : policy == DD_POLICY_RANDOM ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_RANDOM, OUTS_, OF_>, g, kBlock, st, pdl, ra)   \
-                                  : launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_BANGBANG, OUTS_, OF_>, g, kBlock, st, pdl, ra))
+    (policy == DD_POLICY_TRACE    ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_TRACE, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra)  \
+     : policy == DD_POLICY_RANDOM ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_RANDOM, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra) \
+                                  : launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_BANGBANG, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra))
 #define DD_ROLL(OBS_, DEF_, OF_) (outs ? DD_ROLL2(OBS_, DEF_, true, OF_) : DD_ROLL2(OBS_, DEF_, false, OF_))
+    // per-env sets: DEF = false only (DEF = !SETS below instantiates nothing new for them)
     if constexpr (sizeof(R) == 4) {                        // 16-bit obs_tn: float state only
-        if (obs_tn && c->obs_format == DD_OBS_F16) return def ? DD_ROLL(true, true, DD_OBS_F16) : DD_ROLL(true, false, DD_OBS_F16);
-        if (obs_tn && c->obs_format == DD_OBS_BF16) return def ? DD_ROLL(true, true, DD_OBS_BF16) : DD_ROLL(true, false, DD_OBS_BF16);
+        if (obs_tn && c->obs_format == DD_OBS_F16) return def ? DD_ROLL(true, !SETS, DD_OBS_F16) : DD_ROLL(true, false, DD_OBS_F16);
+        if (obs_tn && c->obs_format == DD_OBS_BF16) return def ? DD_ROLL(true, !SETS, DD_OBS_BF16) : DD_ROLL(true, false, DD_OBS_BF16);
     }
-    if (def) return obs_tn ? DD_ROLL(true, true, DD_OBS_NATIVE) : DD_ROLL(false, true, DD_OBS_NATIVE);
+    if (def) return obs_tn ? DD_ROLL(true, !SETS, DD_OBS_NATIVE) : DD_ROLL(false, !SETS, DD_OBS_NATIVE);
     return obs_tn ? DD_ROLL(true, false, DD_OBS_NATIVE) : DD_ROLL(false, false, DD_OBS_NATIVE);
 #undef DD_ROLL
 #undef DD_ROLL2
@@ -611,8 +686,8 @@ int dd_reset(const DDState* s, const DDParams* p, const DDEnvConfig* c, const ui
 {
     if (!s) return DD_E_NULL;
     if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32) return dd::reset_impl<float>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64) return dd::reset_impl<double>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    if (s->dtype == DD_F32) return dd::reset_impl<float, false>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    if (s->dtype == DD_F64) return dd::reset_impl<double, false>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
     return DD_E_DTYPE;
 }
 
@@ -623,14 +698,18 @@ int dd_step(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uin
     if (!s) return DD_E_NULL;
     if (int rc = dd::check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
-        return dd::step_impl<float>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
+        return dd::step_impl<float, false>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
     if (s->dtype == DD_F64)
-        return dd::step_impl<double>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
+        return dd::step_impl<double, false>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
     return DD_E_DTYPE;
 }
 
-int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
-                 void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
+}  // extern "C"
+
+namespace dd {
+template <bool SETS, typename P>
+static int step_plan_impl(const DDState* s, const P* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
+                          void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
 {
     if (!s || !plan) return DD_E_NULL;
     if (s->dtype != DD_F32 && s->dtype != DD_F64) return DD_E_DTYPE;
@@ -638,11 +717,11 @@ int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void
     memset(plan, 0, sizeof *plan);
     int rc, *device;
     if (s->dtype == DD_F32) {
-        auto* pl = reinterpret_cast<dd::StepPlanT<float>*>(plan);
+        auto* pl = reinterpret_cast<dd::StepPlanT<float, SETS>*>(plan);
         rc = dd::step_resolve(*pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n);
         device = &pl->device;
     } else {
-        auto* pl = reinterpret_cast<dd::StepPlanT<double>*>(plan);
+        auto* pl = reinterpret_cast<dd::StepPlanT<double, SETS>*>(plan);
         rc = dd::step_resolve(*pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n);
         device = &pl->device;
     }
@@ -652,11 +731,72 @@ int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void
     if (e != cudaSuccess) { memset(plan, 0, sizeof *plan); return (int)e; }
     return 0;
 }
+}  // namespace dd
+
+extern "C" {
+
+int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
+                 void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
+{
+    return dd::step_plan_impl<false>(s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n, plan);
+}
+
+int dd_step_plan_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, void* obs, int32_t obs_stride,
+                      void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
+{
+    return dd::step_plan_impl<true>(s, ps, c, obs, obs_stride, reward, done_flags, final_obs, stats, n, plan);
+}
+
+int dd_param_sets_build(const DDParams* sets, int32_t count, int32_t dtype, void* host_out)
+{
+    return dd::param_sets_build_checked(sets, count, dtype, host_out);
+}
+
+int dd_reset_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* mask,
+                  void* obs, int32_t obs_stride, int64_t n, void* stream)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32) return dd::reset_impl<float, true>(s, ps, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    if (s->dtype == DD_F64) return dd::reset_impl<double, true>(s, ps, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    return DD_E_DTYPE;
+}
+
+int dd_step_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* actions,
+                 void* obs, int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs,
+                 uint64_t* stats, int64_t n, void* stream)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32)
+        return dd::step_impl<float, true>(s, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
+    if (s->dtype == DD_F64)
+        return dd::step_impl<double, true>(s, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
+    return DD_E_DTYPE;
+}
+
+int dd_rollout_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int32_t policy,
+                    const uint8_t* actions_tn, uint32_t t0, int32_t T, void* reward_tn, uint8_t* done_tn,
+                    void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n, void* stream)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = dd::check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32)
+        return dd::rollout_impl<float, true>(s, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
+    if (s->dtype == DD_F64)
+        return dd::rollout_impl<double, true>(s, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
+    return DD_E_DTYPE;
+}
 
 int dd_step_planned(const DDStepPlan* plan, const uint8_t* actions, void* stream)
 {
     if (!plan) return DD_E_NULL;
     const auto* hdr = reinterpret_cast<const dd::StepPlanT<float>*>(plan);
+    if (hdr->magic == dd::kPlanMagicSets) {                           // dd_step_plan_sets
+        if (hdr->dtype == DD_F32) return dd::step_planned(*reinterpret_cast<const dd::StepPlanT<float, true>*>(plan), actions, (cudaStream_t)stream);
+        if (hdr->dtype == DD_F64) return dd::step_planned(*reinterpret_cast<const dd::StepPlanT<double, true>*>(plan), actions, (cudaStream_t)stream);
+        return DD_E_DTYPE;
+    }
     if (hdr->magic != dd::kPlanMagic) return DD_E_RANGE;             // not (or no longer) a plan
     if (hdr->dtype == DD_F32) return dd::step_planned(*hdr, actions, (cudaStream_t)stream);
     if (hdr->dtype == DD_F64) return dd::step_planned(*reinterpret_cast<const dd::StepPlanT<double>*>(plan), actions, (cudaStream_t)stream);
@@ -670,9 +810,9 @@ int dd_rollout_shaped(const DDState* s, const DDParams* p, const DDEnvConfig* c,
     if (!s) return DD_E_NULL;
     if (int rc = dd::check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
-        return dd::rollout_impl<float>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
+        return dd::rollout_impl<float, false>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
     if (s->dtype == DD_F64)
-        return dd::rollout_impl<double>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
+        return dd::rollout_impl<double, false>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
     return DD_E_DTYPE;
 }
 

@@ -25,9 +25,9 @@ struct HostState {
 };
 
 template <typename R>
-int bind(HostState<R>& h, const DDState* s, const DDParams* p, const DDEnvConfig* c, int64_t n)
+int bind(HostState<R>& h, const DDState* s, const DDEnvConfig* c, int64_t n)
 {
-    if (!s || !p || !c) return DD_E_NULL;
+    if (!s || !c) return DD_E_NULL;
     if (n < 0 || n > (int64_t)DD_MAX_ENVS_PER_CALL) return DD_E_RANGE;
     if (n > 0 && (!s->pos_vel || !s->att_fuel || !s->platform || !s->steps || !s->episode || !s->flags)) return DD_E_NULL;
     h.pos_vel = (R*)s->pos_vel; h.att_fuel = (R*)s->att_fuel; h.platform = (R*)s->platform; h.prev_dist = (R*)s->prev_dist;
@@ -66,6 +66,35 @@ void stats_commit(uint64_t* st, uint32_t f, R ret, int32_t steps)
     st[5] += (uint64_t)steps;
 }
 
+// Where env i's constants come from: the call's DDParams, or its entry of a DDParamSets table (the _sets twins).
+template <typename R>
+struct ConstSource {
+    Consts<R> k0{};
+    const DDParamSets* ps = nullptr;
+    int init(const DDState* s, const DDParams* p, const DDParamSets* sets, int64_t n)     // fill_args of drone_kernels.cu
+    {
+        if (!sets) { if (!p) return DD_E_NULL; k0 = make_consts<R>(*p); return 0; }
+        if (n > 0 && (!sets->table || !sets->index)) return DD_E_NULL;
+        if (sets->count < 1 || sets->count > DD_MAX_PARAM_SETS || (sets->flags & ~DD_PARAM_SETS_RESAMPLE)) return DD_E_RANGE;
+        if (sets->dtype != s->dtype) return DD_E_DTYPE;
+        if (reinterpret_cast<uintptr_t>(sets->table) & 15u) return DD_E_ALIGN;
+        ps = sets;
+        return 0;
+    }
+    Consts<R> of(int64_t i) const
+    {
+        return ps ? param_set<R>(ps->table, param_set_clamp(ps->index[i], (uint32_t)ps->count)) : k0;
+    }
+    // the constants of env i's reset number `ep`: under DD_PARAM_SETS_RESAMPLE a new set, recorded in index[i]
+    Consts<R> at_reset(int64_t i, const Consts<R>& cur, uint64_t seed, uint64_t gid, uint32_t ep) const
+    {
+        if (!ps || !(ps->flags & DD_PARAM_SETS_RESAMPLE)) return cur;
+        const uint32_t s = param_set_draw(seed, gid, ep, (uint32_t)ps->count);
+        ps->index[i] = (uint8_t)s;
+        return param_set<R>(ps->table, s);
+    }
+};
+
 inline int check_stride(int32_t stride) { return (stride == DD_OBS_DIM || stride == 16) ? 0 : DD_E_RANGE; }
 
 // check_obs_format of drone_kernels.cu
@@ -98,17 +127,20 @@ void obs_row(void* base, int64_t r, int32_t stride, int32_t fmt, const Env<R>& e
 }
 
 template <typename R>
-int reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask, void* obs_, int32_t stride, int64_t n)
+int reset_host(const DDState* s, const DDParams* p, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* mask,
+               void* obs_, int32_t stride, int64_t n)
 {
     HostState<R> h;
-    if (int rc = bind(h, s, p, c, n)) return rc;
+    if (int rc = bind(h, s, c, n)) return rc;
+    ConstSource<R> src;
+    if (int rc = src.init(s, p, ps, n)) return rc;
     if (obs_) if (int rc = check_stride(stride)) return rc;
-    const Consts<R> k = make_consts<R>(*p);
     void* obs = obs_;
     for (int64_t i = 0; i < n; ++i) {                                  // reset_kernel
         if (mask && !mask[i]) continue;
         Env<R> e;
         const uint32_t ep = h.episode[i];
+        const Consts<R> k = src.at_reset(i, src.of(i), c->seed, c->env_id_base + (uint64_t)i, ep);
         spawn(e, k, c->seed, c->env_id_base + (uint64_t)i, ep, c->randomize_drone != 0, c->randomize_platform != 0);
         h.episode[i] = ep + 1;
         store_env(h, i, e);
@@ -125,14 +157,15 @@ int reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const 
 }
 
 template <typename R>
-int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* actions, void* obs_, int32_t stride,
-              void* reward_, uint8_t* done_flags, void* final_obs_, uint64_t* stats, int64_t n)
+int step_host(const DDState* s, const DDParams* p, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* actions,
+              void* obs_, int32_t stride, void* reward_, uint8_t* done_flags, void* final_obs_, uint64_t* stats, int64_t n)
 {
     HostState<R> h;
-    if (int rc = bind(h, s, p, c, n)) return rc;
+    if (int rc = bind(h, s, c, n)) return rc;
+    ConstSource<R> src;
+    if (int rc = src.init(s, p, ps, n)) return rc;
     if (!actions && n > 0) return DD_E_NULL;
     if (obs_ || final_obs_) if (int rc = check_stride(stride)) return rc;
-    const Consts<R> k = make_consts<R>(*p);
     void *obs = obs_, *final_obs = final_obs_;
     R* reward_out = (R*)reward_;
     const bool AUTO = c->auto_reset != 0, OBS = obs != nullptr;
@@ -140,6 +173,7 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
         Env<R> e;
         const uint32_t act = actions[i];
         load_env(h, i, e);
+        Consts<R> k = src.of(i);
         uint32_t pflags = AUTO ? 0u : (uint32_t)h.flags[i];
         uint32_t oflags = pflags;
         R reward = (R)0, speed = (R)0, dist = (R)0;
@@ -153,6 +187,7 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
                 if (final_obs) obs_row(final_obs, i, stride, c->obs_format, e, f, speed, dist, k, false, (R)0);
                 if (AUTO) {
                     const uint32_t ep = h.episode[i];
+                    k = src.at_reset(i, k, c->seed, c->env_id_base + (uint64_t)i, ep);
                     spawn(e, k, c->seed, c->env_id_base + (uint64_t)i, ep, c->randomize_drone != 0, c->randomize_platform != 0);
                     h.episode[i] = ep + 1;
                     h.platform[2 * i] = e.px; h.platform[2 * i + 1] = e.py;
@@ -175,19 +210,20 @@ int step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, const u
 }
 
 template <typename R>
-int rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, int32_t policy, const uint8_t* actions_tn,
-                 uint32_t t0, int32_t T, void* reward_tn_, uint8_t* done_tn, void* obs_tn_, int32_t stride, void* shaped_tn_,
-                 uint64_t* stats, int64_t n)
+int rollout_host(const DDState* s, const DDParams* p, const DDParamSets* ps, const DDEnvConfig* c, int32_t policy,
+                 const uint8_t* actions_tn, uint32_t t0, int32_t T, void* reward_tn_, uint8_t* done_tn, void* obs_tn_,
+                 int32_t stride, void* shaped_tn_, uint64_t* stats, int64_t n)
 {
     HostState<R> h;
-    if (int rc = bind(h, s, p, c, n)) return rc;
+    if (int rc = bind(h, s, c, n)) return rc;
+    ConstSource<R> src;
+    if (int rc = src.init(s, p, ps, n)) return rc;
     if (policy < DD_POLICY_TRACE || policy > DD_POLICY_BANGBANG) return DD_E_RANGE;
     if (policy == DD_POLICY_TRACE && !actions_tn && n > 0 && T > 0) return DD_E_NULL;
     if (T < 0) return DD_E_RANGE;
     if (obs_tn_) if (int rc = check_stride(stride)) return rc;
     if (shaped_tn_ && !s->prev_dist && n > 0) return DD_E_NULL;
     if (shaped_tn_ && c->shaping != DD_SHAPING_PPO && c->shaping != DD_SHAPING_PG) return DD_E_RANGE;
-    const Consts<R> k = make_consts<R>(*p);
     R *reward_tn = (R*)reward_tn_, *shaped_tn = (R*)shaped_tn_;
     void* obs_tn = obs_tn_;
     const bool OBS = obs_tn != nullptr, shaping = shaped_tn != nullptr, auto_reset = c->auto_reset != 0;
@@ -196,6 +232,7 @@ int rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, int3
     for (int64_t i = 0; i < n; ++i) {                                  // rollout_kernel, one "thread" at a time
         Env<R> e;
         load_env(h, i, e);
+        Consts<R> k = src.of(i);
         uint32_t pflags = h.flags[i], ep = h.episode[i];
         bool platform_dirty = false;
         const uint64_t gid = c->env_id_base + (uint64_t)i;
@@ -226,6 +263,7 @@ int rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, int3
                 if (f) {
                     stats_commit(stats, f, e.ret, e.steps);
                     if (auto_reset) {
+                        k = src.at_reset(i, k, c->seed, gid, ep);
                         spawn(e, k, c->seed, gid, ep, c->randomize_drone != 0, c->randomize_platform != 0);
                         ep += 1;
                         platform_dirty = true;
@@ -262,8 +300,8 @@ int dd_reset_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, con
 {
     if (!s) return DD_E_NULL;
     if (int rc = check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32) return reset_host<float>(s, p, c, mask, obs, obs_stride, n);
-    if (s->dtype == DD_F64) return reset_host<double>(s, p, c, mask, obs, obs_stride, n);
+    if (s->dtype == DD_F32) return reset_host<float>(s, p, nullptr, c, mask, obs, obs_stride, n);
+    if (s->dtype == DD_F64) return reset_host<double>(s, p, nullptr, c, mask, obs, obs_stride, n);
     return DD_E_DTYPE;
 }
 
@@ -272,8 +310,8 @@ int dd_step_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, cons
 {
     if (!s) return DD_E_NULL;
     if (int rc = check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32) return step_host<float>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
-    if (s->dtype == DD_F64) return step_host<double>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
+    if (s->dtype == DD_F32) return step_host<float>(s, p, nullptr, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
+    if (s->dtype == DD_F64) return step_host<double>(s, p, nullptr, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
     return DD_E_DTYPE;
 }
 
@@ -283,9 +321,47 @@ int dd_rollout_host(const DDState* s, const DDParams* p, const DDEnvConfig* c, i
     if (!s) return DD_E_NULL;
     if (int rc = check_obs_format(s, c)) return rc;
     if (s->dtype == DD_F32)
-        return rollout_host<float>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
+        return rollout_host<float>(s, p, nullptr, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
     if (s->dtype == DD_F64)
-        return rollout_host<double>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
+        return rollout_host<double>(s, p, nullptr, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
+    return DD_E_DTYPE;
+}
+
+int dd_param_sets_build_host(const DDParams* sets, int32_t count, int32_t dtype, void* host_out)
+{
+    return param_sets_build_checked(sets, count, dtype, host_out);
+}
+
+int dd_reset_sets_host(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* mask, void* obs,
+                       int32_t obs_stride, int64_t n)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32) return reset_host<float>(s, nullptr, ps, c, mask, obs, obs_stride, n);
+    if (s->dtype == DD_F64) return reset_host<double>(s, nullptr, ps, c, mask, obs, obs_stride, n);
+    return DD_E_DTYPE;
+}
+
+int dd_step_sets_host(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* actions, void* obs,
+                      int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32) return step_host<float>(s, nullptr, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
+    if (s->dtype == DD_F64) return step_host<double>(s, nullptr, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n);
+    return DD_E_DTYPE;
+}
+
+int dd_rollout_sets_host(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int32_t policy, const uint8_t* actions_tn,
+                         uint32_t t0, int32_t T, void* reward_tn, uint8_t* done_tn, void* obs_tn, int32_t obs_stride,
+                         void* shaped_tn, uint64_t* stats, int64_t n)
+{
+    if (!s) return DD_E_NULL;
+    if (int rc = check_obs_format(s, c)) return rc;
+    if (s->dtype == DD_F32)
+        return rollout_host<float>(s, nullptr, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
+    if (s->dtype == DD_F64)
+        return rollout_host<double>(s, nullptr, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n);
     return DD_E_DTYPE;
 }
 

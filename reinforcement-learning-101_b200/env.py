@@ -30,6 +30,9 @@ _STATE_KEYS = ("x", "y", "vx", "vy", "angle", "angular_velocity", "fuel", "total
 POLICIES = {"trace": nv.POLICY_TRACE, "random": nv.POLICY_RANDOM, "bangbang": nv.POLICY_BANGBANG}
 # observation element dtype -> DDEnvConfig.obs_format (16-bit formats: float32 state only)
 _OBS_FORMATS = {torch.float16: nv.OBS_F16, torch.bfloat16: nv.OBS_BF16}
+# single-set entry point -> its per-env parameter-set counterpart (include/drone_b200.h DDParamSets)
+_SETS_ENTRY = {"dd_reset": "dd_reset_sets", "dd_step": "dd_step_sets", "dd_step_plan": "dd_step_plan_sets",
+               "dd_rollout_shaped": "dd_rollout_sets"}
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -113,13 +116,17 @@ class BatchedDroneEnv:
     rounded to nearest even (``obs32.to(obs_dtype)``, bit for bit), at half the observation bytes; state, rewards,
     flags and statistics stay as they are.  With ``obs_stride=16`` the ``steps`` column is converted too: exact up to
     2048 steps in float16, 256 in bfloat16.  ``policy_rollout`` ignores it (its ``obs`` rows are always float32).
+
+    ``param_sets`` / ``param_index`` / ``resample_param_sets``: per-env physics (domain randomisation, curricula per env
+    group), see ``set_param_sets``.
     """
 
     def __init__(self, num_envs: int, device="cuda", seed: int = 0, randomize_drone: bool = False,
                  randomize_platform: bool = True, max_steps: Optional[int] = None, auto_reset: bool = True,
                  dtype: torch.dtype = torch.float32, env_id_base: int = 0, obs_stride: int = nv.OBS_DIM,
                  want_final_obs: bool = False, params: Optional[nv.DDParams] = None, launch_flags: int = 0,
-                 shaping: str = "ppo", obs_dtype: Optional[torch.dtype] = None):
+                 shaping: str = "ppo", obs_dtype: Optional[torch.dtype] = None, param_sets=None,
+                 param_index: Optional[torch.Tensor] = None, resample_param_sets: bool = False):
         if dtype not in (torch.float32, torch.float64):
             raise ValueError("dtype must be torch.float32 or torch.float64")
         if obs_dtype is None or obs_dtype == dtype or (obs_dtype == torch.float32 and dtype == torch.float32):
@@ -180,6 +187,15 @@ class BatchedDroneEnv:
         self._planned = self._lib.dd_step_planned
         self._prev_dist_stale = False                      # dd_step does not advance prev_dist (include/drone_b200.h)
         self.t_rollout = 0                                 # running step offset of the in-kernel RNG streams (t0 contract)
+        # per-env parameter sets (set_param_sets): None = every env runs under self._params
+        self._sets = None
+        self._ps = None
+        self._ps_table = None
+        self.param_index: Optional[torch.Tensor] = None
+        if param_sets is not None:
+            self.set_param_sets(param_sets, param_index, resample_param_sets)
+        elif param_index is not None or resample_param_sets:
+            raise ValueError("param_index / resample_param_sets need param_sets")
 
     # ---- configuration ------------------------------------------------------------------------
     @property
@@ -212,8 +228,63 @@ class BatchedDroneEnv:
     def params(self, p: "nv.DDParams") -> None:
         if not isinstance(p, nv.DDParams):
             raise TypeError("params must be a DDParams struct")
+        if self._sets is not None:
+            raise RuntimeError("per-env parameter sets are active, so params would not be used: call "
+                               "set_param_sets(None) first, or set_param_sets(...) with the new sets")
         self._params = nv.DDParams.from_buffer_copy(p)
         self._plans.clear()
+
+    # ---- per-env parameter sets --------------------------------------------------------------------
+    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False) -> None:
+        """Give env i the physics of ``sets[min(param_index[i], len(sets) - 1)]`` (include/drone_b200.h, DDParamSets).
+
+        ``sets``: a sequence of 1-64 ``DDParams`` structs (copied), or None to return every env to ``params``.
+        ``index``: the set of each env (``[N]`` integers in [0, 255]); None means ``i % len(sets)``.  The env keeps it as
+        ``param_index`` (uint8 ``[N]`` on the device): editing that tensor in place takes effect at the next call.
+        ``resample``: every reset of an env -- ``reset`` and same-step auto-resets -- draws its next set from
+        Philox(seed, env id, episode, stream 3), writes it to ``param_index`` and spawns under it; the step that ends an
+        episode keeps the old set.  Drops the resolved step launches, like the ``params`` setter."""
+        self._plans.clear()
+        if sets is None:
+            if index is not None or resample:
+                raise ValueError("index / resample need sets")
+            self._sets = self._ps = self._ps_table = self.param_index = None
+            return
+        sets = [nv.DDParams.from_buffer_copy(p) if isinstance(p, nv.DDParams) else p for p in sets]
+        dt = nv.F32 if self.dtype == torch.float32 else nv.F64
+        table = nv.build_param_table(sets, dt)            # validates count and types
+        n = self.num_envs
+        if index is None:
+            idx = (torch.arange(n, device=self.device) % len(sets)).to(torch.uint8)
+        else:
+            idx = torch.as_tensor(index, device=self.device)
+            if tuple(idx.shape) != (n,):
+                raise ValueError("param_index must have shape [num_envs]")
+            if idx.dtype != torch.uint8:
+                if idx.numel() and (int(idx.min()) < 0 or int(idx.max()) > 255):
+                    raise ValueError("param_index values must be in [0, 255]")
+                idx = idx.to(torch.uint8)
+            idx = idx.contiguous().clone()
+        self._ps_table = torch.frombuffer(bytearray(table), dtype=torch.uint8).to(self.device)
+        self._sets = sets
+        self.param_index = idx
+        self._ps = nv.DDParamSets(self._ps_table.data_ptr(), idx.data_ptr(), len(sets), dt,
+                                  nv.PARAM_SETS_RESAMPLE if resample else 0, 0)
+
+    @property
+    def param_sets(self):
+        """Copies of the active ``DDParams`` sets, or None when every env runs under ``params``."""
+        return None if self._sets is None else [nv.DDParams.from_buffer_copy(p) for p in self._sets]
+
+    @property
+    def resample_param_sets(self) -> bool:
+        return self._ps is not None and bool(self._ps.flags & nv.PARAM_SETS_RESAMPLE)
+
+    def _pargs(self, name: str):
+        """The C entry point ``name`` (or its _sets twin while sets are active) and its parameter argument."""
+        if self._ps is None:
+            return getattr(self._lib, name), C.byref(self._params)
+        return getattr(self._lib, _SETS_ENTRY[name]), C.byref(self._ps)
 
     @property
     def launch_flags(self) -> int:
@@ -244,8 +315,9 @@ class BatchedDroneEnv:
                 m = mask.to(device=self.device).ne(0).to(torch.uint8).contiguous()
                 if m.shape != (self.num_envs,):
                     raise ValueError("mask must have shape [num_envs]")
-            nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self._params), C.byref(self._cfg), _ptr(m),
-                                        None, self.obs_stride, self.num_envs, self._stream()), "dd_reset")
+            fn, pa = self._pargs("dd_reset")
+            nv.check(fn(C.byref(self._state), pa, C.byref(self._cfg), _ptr(m),
+                        None, self.obs_stride, self.num_envs, self._stream()), "dd_reset")
             self._needs_reset = False
             return None
         m = None
@@ -254,15 +326,17 @@ class BatchedDroneEnv:
             if m.shape != (self.num_envs,):
                 raise ValueError("mask must have shape [num_envs]")
             self.observe()                     # rows of unmasked envs: current state
-        nv.check(self._lib.dd_reset(C.byref(self._state), C.byref(self._params), C.byref(self._cfg), _ptr(m),
-                                    self.obs.data_ptr(), self.obs_stride, self.num_envs, self._stream()), "dd_reset")
+        fn, pa = self._pargs("dd_reset")
+        nv.check(fn(C.byref(self._state), pa, C.byref(self._cfg), _ptr(m),
+                    self.obs.data_ptr(), self.obs_stride, self.num_envs, self._stream()), "dd_reset")
         self._needs_reset = False
         return self.obs
 
     def observe(self) -> torch.Tensor:
         """``get_state()`` (game_engine.py:140-177) of every env without stepping."""
         self._packed.fill_(nv.ACT_SKIP)
-        nv.check(self._lib.dd_step(C.byref(self._state), C.byref(self._params), C.byref(self._cfg),
+        fn, pa = self._pargs("dd_step")
+        nv.check(fn(C.byref(self._state), pa, C.byref(self._cfg),
                                    self._packed.data_ptr(), self.obs.data_ptr(), self.obs_stride, None, None, None,
                                    None, self.num_envs, self._stream()), "dd_step(observe)")
         return self.obs
@@ -313,8 +387,9 @@ class BatchedDroneEnv:
         a 3-argument call.  ``obs`` / ``reward`` / ``flags`` override the destination addresses (e.g. device-mapped
         pinned host memory for ``step_host(zero_copy=True)``)."""
         plan = nv.DDStepPlan()
-        nv.check(self._lib.dd_step_plan(
-            C.byref(self._state), C.byref(self._params), C.byref(self._cfg),
+        fn, pa = self._pargs("dd_step_plan")
+        nv.check(fn(
+            C.byref(self._state), pa, C.byref(self._cfg),
             (self.obs.data_ptr() if obs is None else obs) if want_obs else None, self.obs_stride,
             self.reward.data_ptr() if reward is None else reward, self.step_flags.data_ptr() if flags is None else flags,
             _ptr(self.final_obs), self.stats_slots.data_ptr() if stats else None, self.num_envs, C.byref(plan)), "dd_step_plan")
@@ -383,8 +458,9 @@ class BatchedDroneEnv:
         if shaped_out is not None:
             self._fresh_prev_dist()
         t0 = self._take_t0(t0, T) if pol == nv.POLICY_RANDOM else int(t0 or 0)
-        nv.check(self._lib.dd_rollout_shaped(
-            C.byref(self._state), C.byref(self._params), C.byref(self._cfg), pol, _ptr(actions), int(t0), int(T),
+        fn, pa = self._pargs("dd_rollout_shaped")
+        nv.check(fn(
+            C.byref(self._state), pa, C.byref(self._cfg), pol, _ptr(actions), int(t0), int(T),
             _ptr(reward_out), _ptr(done_out), _ptr(obs_out), self.obs_stride, _ptr(shaped_out),
             self.stats_slots.data_ptr() if stats else None, n, self._stream()), "dd_rollout")
 
@@ -421,15 +497,18 @@ class BatchedDroneEnv:
     # ---- checkpoint / injection -----------------------------------------------------------------------
     def get_state(self) -> Dict[str, torch.Tensor]:
         """Copies of the raw (un-normalised) state, reference attribute names (drone.py:19-32,
-        platform.py:19-20, game_engine.py:50-53)."""
+        platform.py:19-20, game_engine.py:50-53); with parameter sets active also ``param_index``."""
         pv, af, pf = self.pos_vel, self.att_fuel, self.platform
-        return {
+        st = {
             "x": pv[:, 0].clone(), "y": pv[:, 1].clone(), "vx": pv[:, 2].clone(), "vy": pv[:, 3].clone(),
             "angle": af[:, 0].clone(), "angular_velocity": af[:, 1].clone(), "fuel": af[:, 2].clone(),
             "total_reward": af[:, 3].clone(), "platform_x": pf[:, 0].clone(), "platform_y": pf[:, 1].clone(),
             "steps": self.steps.clone(), "episode": self.episode.clone(), "flags": self.flags.clone(),
             "prev_dist": self.prev_dist.clone(),
         }
+        if self.param_index is not None:
+            st["param_index"] = self.param_index.clone()
+        return st
 
     def set_state(self, state: Dict[str, torch.Tensor]) -> None:
         """Overwrite any subset of the state tensors (each ``[N]``)."""
@@ -437,7 +516,7 @@ class BatchedDroneEnv:
                 "angle": (self.att_fuel, 0), "angular_velocity": (self.att_fuel, 1), "fuel": (self.att_fuel, 2),
                 "total_reward": (self.att_fuel, 3), "platform_x": (self.platform, 0), "platform_y": (self.platform, 1)}
         for k, v in state.items():
-            if k not in _STATE_KEYS:
+            if k not in _STATE_KEYS and not (k == "param_index" and self.param_index is not None):
                 raise KeyError(k)
             v = torch.as_tensor(v, device=self.device)
             if k in cols:
@@ -455,13 +534,20 @@ class BatchedDroneEnv:
         self.set_state({
             "x": x, "y": y, "platform_x": platform_x, "platform_y": platform_y,
             "vx": z, "vy": z, "angle": z, "angular_velocity": z, "total_reward": z,
-            "fuel": torch.full((n,), float(self._params.max_fuel), dtype=self.dtype, device=dev),
+            "fuel": self._max_fuel(),
             "steps": torch.zeros(n, dtype=torch.int32, device=dev),
             "flags": torch.zeros(n, dtype=torch.uint8, device=dev),
             "episode": self.episode + 1,
         })
         self.prev_dist.fill_(float("nan"))
         return self.observe()
+
+    def _max_fuel(self) -> torch.Tensor:
+        """``[N]``: each env's ``max_fuel`` (its parameter set's, when sets are active)."""
+        if self._sets is None:
+            return torch.full((self.num_envs,), float(self._params.max_fuel), dtype=self.dtype, device=self.device)
+        mf = torch.tensor([p.max_fuel for p in self._sets], dtype=self.dtype, device=self.device)
+        return mf[self.param_index.long().clamp(max=len(self._sets) - 1)]
 
     # ---- host-buffer entry point (what a CPU-side caller such as the socket shim uses) -----------------
     def make_host_io(self):

@@ -145,6 +145,9 @@ def policy_rollout(env: BatchedDroneEnv, blob: PolicyBlob, T: int, sample: bool 
         sample, temperature = False, 1.0
     if env.dtype != torch.float32:
         raise ValueError("policy_rollout needs a float32 env")
+    if env.param_sets is not None:
+        raise ValueError("policy_rollout does not take per-env parameter sets: the fused policy kernel runs one DDParams "
+                         "per launch (call env.set_param_sets(None) first)")
     if env._needs_reset:
         raise RuntimeError("call reset() before policy_rollout()")
     n, dev = env.num_envs, env.device

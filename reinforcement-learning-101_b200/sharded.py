@@ -22,8 +22,9 @@ c16:L42-108), for both kinds of caller:
     in that order (tested).  ``run`` / ``step_all`` return as soon as the work is enqueued on the env's own chain
     streams; ``join()`` orders the caller's stream behind it.
 
-``env_kw`` goes to every shard's ``BatchedDroneEnv`` (``obs_dtype=torch.bfloat16`` etc.): the observation format is
-part of each shard's resolved step launch, so the graphs replay it like any other argument.
+``env_kw`` goes to every shard's ``BatchedDroneEnv`` (``obs_dtype=torch.bfloat16``, ``param_sets=[...]`` etc.): the
+observation format and the parameter-set pointers are part of each shard's resolved step launch, so the graphs replay
+them like any other argument.
 
 Global env ids are contiguous over the shards (``env_id_base + s * N + i``), so a ShardedDroneEnv of S x N envs is the
 same set of trajectories as one BatchedDroneEnv of S * N envs (Philox is keyed by the global id).
@@ -237,6 +238,17 @@ class ShardedDroneEnv:
         self.join()
         for e in self.shards:
             e.params = p
+        self._drop_graphs()
+
+    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False) -> None:
+        """Per-env parameter sets for every shard (``BatchedDroneEnv.set_param_sets``); ``index``: ``[S, N]`` (None:
+        env i of each shard runs under set ``i % len(sets)``).  The captured graphs are dropped.  Afterwards in-place
+        edits of ``shards[s].param_index`` reach the graphs as they are (they hold its pointer; ``join()`` first)."""
+        if index is not None and tuple(index.shape) != (self.S, self.N):
+            raise ValueError(f"index must have shape {(self.S, self.N)}")
+        self.join()
+        for s, e in enumerate(self.shards):
+            e.set_param_sets(sets, None if index is None else index[s], resample)
         self._drop_graphs()
 
     # ---- statistics / state -------------------------------------------------------------------------------------

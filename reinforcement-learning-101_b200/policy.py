@@ -92,7 +92,9 @@ def _rows(obs: torch.Tensor) -> torch.Tensor:
 
 
 def policy_forward(blob: PolicyBlob, obs: torch.Tensor) -> torch.Tensor:
-    """probs [..., 3] = sigmoid(policy(obs [..., 15])) on the tensor-core path (persistent over the rows)."""
+    """probs [..., 3] = sigmoid(policy(obs [..., 15])) on the tensor-core path (persistent over the rows).
+    With fp16 operands the observations must lie within the fp16 range (|x| <= 65504; rollout observations are O(10)):
+    the first layer splits each input into fp16 hi + lo halves, and a larger input gives NaN.  Not checked per call."""
     if blob.head != 3:
         raise ValueError("policy_forward needs a policy blob (head=3)")
     rows = _rows(obs)

@@ -18,6 +18,7 @@
 #include <stdint.h>
 #include <string.h>
 #include "drone_device.cuh"
+#include "env_abi.h"
 #include "host_guard.h"
 
 namespace dd {
@@ -442,74 +443,24 @@ __global__ void __launch_bounds__(kBlock) live_steps_kernel(const int32_t* steps
 // =================================================================================================
 static inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
 
-static bool params_are_default(const DDParams& p)
+// f(std::bool_constant<DEF>()): the DEF kernels (config.py's parameters as immediates) exist for single-set calls only.
+template <bool SETS, typename P, typename F>
+static auto with_def(const P& p, F&& f)
 {
-    const DDParams d = kDefaultParams;
-    if (memcmp(&p, &d, sizeof d) != 0) return false;
-    // the compile-time constants assume sqrt thresholds that the search confirms
-    return speed2_threshold<float>((float)p.land_speed) == (float)p.land_speed * (float)p.land_speed &&
-           speed2_threshold<double>(p.land_speed) == p.land_speed * p.land_speed;
+    if constexpr (SETS) return f(std::false_type());
+    else return with_bool(params_are_default(p), f);
 }
 
-// Everything of the argument block but the constants.
-template <typename R>
-static int fill_state(KArgs<R>& a, const DDState* s, const DDEnvConfig* c, int64_t n)
+// f(int_c<BLOCK>()) for the CTA size DDEnvConfig.launch_flags asks for: 128 and 512 exist for float only (tuning knob).
+template <typename R, typename F>
+static auto with_block(int32_t launch_flags, F&& f)
 {
-    if (!s || !c) return DD_E_NULL;
-    if (n < 0 || n > (int64_t)0x7fffff00) return DD_E_RANGE;          // 32-bit env index inside one call
-    if (n > 0 && (!s->pos_vel || !s->att_fuel || !s->platform || !s->steps || !s->episode || !s->flags)) return DD_E_NULL;
-    if ((reinterpret_cast<uintptr_t>(s->pos_vel) | reinterpret_cast<uintptr_t>(s->att_fuel)) & 15u) return DD_E_ALIGN;
-    if (reinterpret_cast<uintptr_t>(s->platform) & (2 * sizeof(R) - 1)) return DD_E_ALIGN;
-    a = KArgs<R>{};
-    a.pos_vel = (R*)s->pos_vel; a.att_fuel = (R*)s->att_fuel; a.platform = (R*)s->platform;
-    a.prev_dist = (R*)s->prev_dist;
-    a.steps = s->steps; a.episode = s->episode; a.flags = s->flags;
-    a.n = (uint32_t)n; a.seed = c->seed; a.env_id_base = c->env_id_base;
-    a.max_steps = c->max_steps; a.obs_stride = DD_OBS_DIM; a.shaping = c->shaping;
-    a.rand_drone = c->randomize_drone; a.rand_platform = c->randomize_platform;
-    return 0;
-}
-
-template <typename R>
-static int fill_args(KArgs<R>& a, const DDState* s, const DDParams* p, const DDEnvConfig* c, int64_t n)
-{
-    if (!p) return DD_E_NULL;
-    if (int rc = fill_state(a, s, c, n)) return rc;
-    a.k = make_consts<R>(*p);
-    return 0;
-}
-
-// The DDParamSets checks of include/drone_b200.h, then the argument block of the per-env kernels.
-template <typename R>
-static int fill_args(KArgsPS<R>& a, const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int64_t n)
-{
-    if (!ps) return DD_E_NULL;
-    if (int rc = fill_state(a, s, c, n)) return rc;
-    if (n > 0 && (!ps->table || !ps->index)) return DD_E_NULL;
-    if (ps->count < 1 || ps->count > DD_MAX_PARAM_SETS || (ps->flags & ~DD_PARAM_SETS_RESAMPLE)) return DD_E_RANGE;
-    if (ps->dtype != s->dtype) return DD_E_DTYPE;
-    if (reinterpret_cast<uintptr_t>(ps->table) & 15u) return DD_E_ALIGN;
-    a.ps_table = ps->table; a.ps_index = ps->index;
-    a.ps_count = (uint32_t)ps->count; a.ps_resample = (ps->flags & DD_PARAM_SETS_RESAMPLE) ? 1 : 0;
-    return 0;
-}
-
-// Kernel mode of a call: single-set calls use the immediates when the parameters are config.py's; per-env sets never.
-static bool params_are_default(const DDParamSets&) { return false; }
-
-static inline int check_stride(int32_t stride) {
-    return (stride == DD_OBS_DIM || stride == kMaxObsStride) ? 0 : DD_E_RANGE;
-}
-
-// DDEnvConfig.obs_format, checked before any CUDA call: DD_E_RANGE for an unknown value, DD_E_DTYPE for a 16-bit format
-// with float64 state (the exact-parity instantiation writes its own precision only).  NULL structs are left to the
-// callee's checks.
-static int check_obs_format(const DDState* s, const DDEnvConfig* c)
-{
-    if (!s || !c) return 0;
-    if (c->obs_format < DD_OBS_NATIVE || c->obs_format > DD_OBS_BF16) return DD_E_RANGE;
-    if (c->obs_format != DD_OBS_NATIVE && s->dtype != DD_F32) return DD_E_DTYPE;
-    return 0;
+    if constexpr (std::is_same<R, float>::value) {
+        const int bsel = (launch_flags >> 4) & 3;
+        if (bsel == 1) return f(int_c<128>());
+        if (bsel == 2) return f(int_c<512>());
+    }
+    return f(int_c<256>());
 }
 
 template <typename R, bool SETS, typename P>
@@ -524,11 +475,9 @@ static int reset_impl(const DDState* s, const P* p, const DDEnvConfig* c, const 
     DeviceGuard g(st, s->pos_vel);
     if (g.err != cudaSuccess) return (int)g.err;
     const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0;
-    if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
-        if (c->obs_format == DD_OBS_F16) return launch(reset_kernel<R, DD_OBS_F16, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
-        if (c->obs_format == DD_OBS_BF16) return launch(reset_kernel<R, DD_OBS_BF16, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
-    }
-    return launch(reset_kernel<R, DD_OBS_NATIVE, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+    return with_obs_format<R>(c->obs_format, [&](auto of) {
+        return launch(reset_kernel<R, of, SETS>, grid_for(n, kBlock), kBlock, st, pdl, a, mask);
+    });
 }
 
 // The resolved launch of one dd_step call: what dd_step_plan stores in the caller's DDStepPlan.
@@ -544,28 +493,6 @@ constexpr uint32_t kPlanMagicSets = 0x44445334u;           // "DDS4": a plan of 
 static_assert(sizeof(StepPlanT<double, true>) <= DD_STEP_PLAN_BYTES && sizeof(StepPlanT<float, true>) <= DD_STEP_PLAN_BYTES,
               "DD_STEP_PLAN_BYTES too small for the argument block");
 
-template <typename R, bool AUTO, bool OBS, bool DEF, int OF, bool SETS>
-static void (*step_kernel_of(int block))(KArgsOf<R, SETS>)
-{
-    if constexpr (sizeof(R) == 4) {                        // CTA-size variants: float only (tuning knob)
-        if (block == 128) return step_kernel<R, AUTO, OBS, DEF, 128, OF, SETS>;
-        if (block == 512) return step_kernel<R, AUTO, OBS, DEF, 512, OF, SETS>;
-    }
-    return step_kernel<R, AUTO, OBS, DEF, 256, OF, SETS>;
-}
-
-template <typename R, int OF, bool SETS>
-static void (*step_kernel_sel(bool au, bool ob, bool def, int block))(KArgsOf<R, SETS>)
-{
-#define DD_STEP(AU, OB, DF) step_kernel_of<R, AU, OB, DF, OF, SETS>(block)
-    if (!SETS && def)                                      // per-env sets: DEF = false only
-        return au ? (ob ? DD_STEP(true, true, !SETS) : DD_STEP(true, false, !SETS))
-                  : (ob ? DD_STEP(false, true, !SETS) : DD_STEP(false, false, !SETS));
-    return au ? (ob ? DD_STEP(true, true, false) : DD_STEP(true, false, false))
-              : (ob ? DD_STEP(false, true, false) : DD_STEP(false, false, false));
-#undef DD_STEP
-}
-
 // Validate a dd_step call and resolve it to (kernel, grid, block, argument block).
 template <typename R, bool SETS, typename P>
 static int step_resolve(StepPlanT<R, SETS>& pl, const DDState* s, const P* p, const DDEnvConfig* c,
@@ -577,17 +504,21 @@ static int step_resolve(StepPlanT<R, SETS>& pl, const DDState* s, const P* p, co
     if (obs || final_obs) { if (int rc = check_stride(obs_stride)) return rc; a.obs_stride = obs_stride; }
     a.obs = (R*)obs; a.reward = (R*)reward; a.final_obs = (R*)final_obs;
     a.done_flags = done_flags; a.stats = (unsigned long long*)stats;
-    const bool au = c->auto_reset != 0, ob = obs != nullptr, def = params_are_default(*p);
-    const int bsel = (c->launch_flags >> 4) & 3;
-    int block = bsel == 1 ? 128 : (bsel == 2 ? 512 : 256);
-    if (sizeof(R) != 4) block = 256;
     pl.magic = SETS ? kPlanMagicSets : kPlanMagic; pl.dtype = sizeof(R) == 4 ? DD_F32 : DD_F64; pl.device = -1;
-    pl.block = block; pl.grid = grid_for(n, block); pl.pdl = (c->launch_flags & DD_LAUNCH_PDL) ? 1 : 0;
-    pl.kern = step_kernel_sel<R, DD_OBS_NATIVE, SETS>(au, ob, def, block);
-    if constexpr (sizeof(R) == 4) {                        // 16-bit observations: float state only
-        if (c->obs_format == DD_OBS_F16) pl.kern = step_kernel_sel<R, DD_OBS_F16, SETS>(au, ob, def, block);
-        if (c->obs_format == DD_OBS_BF16) pl.kern = step_kernel_sel<R, DD_OBS_BF16, SETS>(au, ob, def, block);
-    }
+    pl.pdl = (c->launch_flags & DD_LAUNCH_PDL) ? 1 : 0;
+    with_obs_format<R>(c->obs_format, [&](auto of) {
+        with_def<SETS>(*p, [&](auto def) {
+            with_bool(c->auto_reset != 0, [&](auto au) {
+                with_bool(obs != nullptr, [&](auto ob) {
+                    with_block<R>(c->launch_flags, [&](auto block) {
+                        pl.kern = step_kernel<R, au, ob, def, block, of, SETS>;
+                        pl.block = block;
+                    });
+                });
+            });
+        });
+    });
+    pl.grid = grid_for(n, pl.block);
     return 0;
 }
 
@@ -604,6 +535,22 @@ static int step_impl(const DDState* s, const P* p, const DDEnvConfig* c, const u
     if (g.err != cudaSuccess) return (int)g.err;
     pl.a.actions = actions;
     return launch(pl.kern, pl.grid, pl.block, st, pl.pdl != 0, pl.a);
+}
+
+template <bool SETS, typename P>
+static int step_plan_impl(const DDState* s, const P* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
+                          void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
+{
+    if (!plan) return DD_E_NULL;
+    memset(plan, 0, sizeof *plan);
+    const int rc = with_state_type(s, c, [&](auto r) {
+        auto& pl = *reinterpret_cast<StepPlanT<decltype(r), SETS>*>(plan);
+        if (int rc = step_resolve(pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n)) return rc;
+        // the state buffers name the device the planned launches run on
+        return (int)owning_device(nullptr, n > 0 ? s->pos_vel : nullptr, &pl.device);
+    });
+    if (rc) memset(plan, 0, sizeof *plan);                 // a failed call leaves a zeroed plan, which dd_step_planned refuses
+    return rc;
 }
 
 template <typename R, bool SETS>
@@ -638,23 +585,21 @@ static int rollout_impl(const DDState* s, const P* p, const DDEnvConfig* c, int3
     if (n == 0 || T == 0) return 0;
     DeviceGuard guard(st, s->pos_vel);
     if (guard.err != cudaSuccess) return (int)guard.err;
-    const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0, def = params_are_default(*p);
+    const bool pdl = (c->launch_flags & DD_LAUNCH_PDL) != 0, outs = reward_tn || done_tn || shaped_tn;
     const int g = grid_for(n, kBlock);
-    const bool outs = reward_tn || done_tn || shaped_tn;
-#define DD_ROLL2(OBS_, DEF_, OUTS_, OF_)                                                                                          \
-    (policy == DD_POLICY_TRACE    ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_TRACE, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra)  \
-     : policy == DD_POLICY_RANDOM ? launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_RANDOM, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra) \
-                                  : launch(rollout_kernel<R, OBS_, DEF_, DD_POLICY_BANGBANG, OUTS_, OF_, SETS>, g, kBlock, st, pdl, ra))
-#define DD_ROLL(OBS_, DEF_, OF_) (outs ? DD_ROLL2(OBS_, DEF_, true, OF_) : DD_ROLL2(OBS_, DEF_, false, OF_))
-    // per-env sets: DEF = false only (DEF = !SETS below instantiates nothing new for them)
-    if constexpr (sizeof(R) == 4) {                        // 16-bit obs_tn: float state only
-        if (obs_tn && c->obs_format == DD_OBS_F16) return def ? DD_ROLL(true, !SETS, DD_OBS_F16) : DD_ROLL(true, false, DD_OBS_F16);
-        if (obs_tn && c->obs_format == DD_OBS_BF16) return def ? DD_ROLL(true, !SETS, DD_OBS_BF16) : DD_ROLL(true, false, DD_OBS_BF16);
-    }
-    if (def) return obs_tn ? DD_ROLL(true, !SETS, DD_OBS_NATIVE) : DD_ROLL(false, !SETS, DD_OBS_NATIVE);
-    return obs_tn ? DD_ROLL(true, false, DD_OBS_NATIVE) : DD_ROLL(false, false, DD_OBS_NATIVE);
-#undef DD_ROLL
-#undef DD_ROLL2
+    const auto run = [&](auto obs, auto of) {
+        return with_def<SETS>(*p, [&](auto def) {
+            return with_bool(outs, [&](auto out) {
+                const auto go = [&](auto pol) { return launch(rollout_kernel<R, obs, def, pol, out, of, SETS>, g, kBlock, st, pdl, ra); };
+                return policy == DD_POLICY_TRACE    ? go(int_c<DD_POLICY_TRACE>())
+                     : policy == DD_POLICY_RANDOM ? go(int_c<DD_POLICY_RANDOM>())
+                                                  : go(int_c<DD_POLICY_BANGBANG>());
+            });
+        });
+    };
+    // obs_format is the element format of obs_tn: without obs_tn the native kernel runs
+    if (obs_tn) return with_obs_format<R>(c->obs_format, [&](auto of) { return run(std::true_type(), of); });
+    return run(std::false_type(), int_c<DD_OBS_NATIVE>());
 }
 
 }  // namespace dd
@@ -684,56 +629,20 @@ const char* dd_error_string(int code)
 int dd_reset(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* mask,
              void* obs, int32_t obs_stride, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32) return dd::reset_impl<float, false>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64) return dd::reset_impl<double, false>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::reset_impl<decltype(r), false>(s, p, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    });
 }
 
 int dd_step(const DDState* s, const DDParams* p, const DDEnvConfig* c, const uint8_t* actions,
             void* obs, int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs,
             uint64_t* stats, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32)
-        return dd::step_impl<float, false>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64)
-        return dd::step_impl<double, false>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::step_impl<decltype(r), false>(s, p, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n,
+                                                 (cudaStream_t)stream);
+    });
 }
-
-}  // extern "C"
-
-namespace dd {
-template <bool SETS, typename P>
-static int step_plan_impl(const DDState* s, const P* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
-                          void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
-{
-    if (!s || !plan) return DD_E_NULL;
-    if (s->dtype != DD_F32 && s->dtype != DD_F64) return DD_E_DTYPE;
-    if (int rc = dd::check_obs_format(s, c)) { memset(plan, 0, sizeof *plan); return rc; }
-    memset(plan, 0, sizeof *plan);
-    int rc, *device;
-    if (s->dtype == DD_F32) {
-        auto* pl = reinterpret_cast<dd::StepPlanT<float, SETS>*>(plan);
-        rc = dd::step_resolve(*pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n);
-        device = &pl->device;
-    } else {
-        auto* pl = reinterpret_cast<dd::StepPlanT<double, SETS>*>(plan);
-        rc = dd::step_resolve(*pl, s, p, c, obs, obs_stride, reward, done_flags, final_obs, stats, n);
-        device = &pl->device;
-    }
-    if (rc) { memset(plan, 0, sizeof *plan); return rc; }
-    // the state buffers name the device the planned launches run on
-    const cudaError_t e = dd::owning_device(nullptr, n > 0 ? s->pos_vel : nullptr, device);
-    if (e != cudaSuccess) { memset(plan, 0, sizeof *plan); return (int)e; }
-    return 0;
-}
-}  // namespace dd
-
-extern "C" {
 
 int dd_step_plan(const DDState* s, const DDParams* p, const DDEnvConfig* c, void* obs, int32_t obs_stride,
                  void* reward, uint8_t* done_flags, void* final_obs, uint64_t* stats, int64_t n, DDStepPlan* plan)
@@ -755,37 +664,29 @@ int dd_param_sets_build(const DDParams* sets, int32_t count, int32_t dtype, void
 int dd_reset_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* mask,
                   void* obs, int32_t obs_stride, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32) return dd::reset_impl<float, true>(s, ps, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64) return dd::reset_impl<double, true>(s, ps, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::reset_impl<decltype(r), true>(s, ps, c, mask, obs, obs_stride, n, (cudaStream_t)stream);
+    });
 }
 
 int dd_step_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const uint8_t* actions,
                  void* obs, int32_t obs_stride, void* reward, uint8_t* done_flags, void* final_obs,
                  uint64_t* stats, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32)
-        return dd::step_impl<float, true>(s, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64)
-        return dd::step_impl<double, true>(s, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::step_impl<decltype(r), true>(s, ps, c, actions, obs, obs_stride, reward, done_flags, final_obs, stats, n,
+                                                (cudaStream_t)stream);
+    });
 }
 
 int dd_rollout_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int32_t policy,
                     const uint8_t* actions_tn, uint32_t t0, int32_t T, void* reward_tn, uint8_t* done_tn,
                     void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32)
-        return dd::rollout_impl<float, true>(s, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64)
-        return dd::rollout_impl<double, true>(s, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::rollout_impl<decltype(r), true>(s, ps, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride,
+                                                   shaped_tn, stats, n, (cudaStream_t)stream);
+    });
 }
 
 int dd_step_planned(const DDStepPlan* plan, const uint8_t* actions, void* stream)
@@ -807,13 +708,10 @@ int dd_rollout_shaped(const DDState* s, const DDParams* p, const DDEnvConfig* c,
                       const uint8_t* actions_tn, uint32_t t0, int32_t T, void* reward_tn, uint8_t* done_tn,
                       void* obs_tn, int32_t obs_stride, void* shaped_tn, uint64_t* stats, int64_t n, void* stream)
 {
-    if (!s) return DD_E_NULL;
-    if (int rc = dd::check_obs_format(s, c)) return rc;
-    if (s->dtype == DD_F32)
-        return dd::rollout_impl<float, false>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
-    if (s->dtype == DD_F64)
-        return dd::rollout_impl<double, false>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride, shaped_tn, stats, n, (cudaStream_t)stream);
-    return DD_E_DTYPE;
+    return dd::with_state_type(s, c, [&](auto r) {
+        return dd::rollout_impl<decltype(r), false>(s, p, c, policy, actions_tn, t0, T, reward_tn, done_tn, obs_tn, obs_stride,
+                                                    shaped_tn, stats, n, (cudaStream_t)stream);
+    });
 }
 
 int dd_rollout(const DDState* s, const DDParams* p, const DDEnvConfig* c, int32_t policy,
@@ -841,7 +739,7 @@ int dd_gather_env(const DDState* s, const void* obs, int32_t obs_stride, const v
     if (!s || !out) return DD_E_NULL;
     if (!s->pos_vel || !s->att_fuel || !s->platform || !s->steps || !s->episode || !s->flags) return DD_E_NULL;
     if (i < 0 || i >= n) return DD_E_RANGE;
-    if (obs && obs_stride != 15 && obs_stride != 16) return DD_E_RANGE;
+    if (obs) { if (int rc = dd::check_stride(obs_stride)) return rc; }
     if (s->dtype != DD_F32 && s->dtype != DD_F64) return DD_E_DTYPE;
     dd::DeviceGuard g((cudaStream_t)stream, s->pos_vel);
     if (g.err != cudaSuccess) return (int)g.err;

@@ -82,8 +82,8 @@
 #include <cuda_fp16.h>
 #include <stddef.h>
 #include <stdint.h>
-#include <string.h>
 #include "drone_device.cuh"
+#include "env_abi.h"
 #include "host_guard.h"
 
 namespace dd {
@@ -896,12 +896,6 @@ __global__ void __launch_bounds__(256) policy_pack_kernel(DDPolicy p, int head, 
     if (tid < 4) reinterpret_cast<int32_t*>(par)[pFmt + tid] = tid == 0 ? s_fmt : 0;
 }
 
-static bool pol_params_default(const DDParams& p)
-{
-    const DDParams d = kDefaultParams;
-    return memcmp(&p, &d, sizeof d) == 0;
-}
-
 // CTAs of a rollout launch over n envs on a device with `sms` SMs; slot g (0..3) of CTA b runs tile b + grid * g.
 // Per-SM throughput saturates with the number of resident tiles -- measured on B200 with every SM busy: 0.77 / 0.91 /
 // 1.08 / 1.26 ms per 250 steps at 1 / 2 / 3 / 4 tiles per SM -- so up to 3 tiles per SM the tiles are SPREAD over the
@@ -918,30 +912,29 @@ static int rollout_grid(int64_t n, int sms)
 static int policy_launch(PArgs& pa, const DDParams& p, int64_t n, bool forward, cudaStream_t st)
 {
     const int blocks = (int)((n + kTile * kGroups - 1) / (kTile * kGroups));
-    const bool def = pol_params_default(p);
-    void (*kern)(PArgs);
-    int grid = blocks;
     DeviceGuard guard(st, pa.blob);                         // the device that owns the stream (or the blob)
     if (guard.err != cudaSuccess) return (int)guard.err;
+    int sms = 0;
+    const cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, guard.dev);
+    if (e != cudaSuccess) return (int)e;
+    void (*kern)(PArgs);
+    int grid;
     const bool f16 = pa.pc.operands == DD_OPERANDS_FP16;
     if (forward) {
-        kern = pa.head == 1 ? (f16 ? policy_rollout_kernel<true, true, 1, false, true> : policy_rollout_kernel<true, true, 1, false, false>)
-                            : (f16 ? policy_rollout_kernel<true, true, 3, false, true> : policy_rollout_kernel<true, true, 3, false, false>);
-        int sms = 0;
-        const cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, guard.dev);
-        if (e != cudaSuccess) return (int)e;
+        kern = with_bool(f16, [&](auto h) {
+            return pa.head == 1 ? policy_rollout_kernel<true, true, 1, false, h> : policy_rollout_kernel<true, true, 3, false, h>;
+        });
         grid = blocks < sms ? blocks : sms;                 // persistent: one CTA per SM walks the row blocks
         pa.T = (blocks + grid - 1) / grid;
     } else {
-        int sms = 0;
-        const cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, guard.dev);
-        if (e != cudaSuccess) return (int)e;
         grid = rollout_grid(n, sms);
         const bool fast = pa.mode == DD_ACTION_SAMPLE && pa.inv_temperature == 1.0f && pa.auto_reset && pa.a.stats &&
                           pa.actions_tn && pa.logp_tn && pa.reward_tn && pa.done_tn && pa.obs_tn && !pa.shaped_tn && !pa.probs_tn;
-#define DD_K5(DEF_, FAST_) (f16 ? policy_rollout_kernel<DEF_, false, 3, FAST_, true> : policy_rollout_kernel<DEF_, false, 3, FAST_, false>)
-        kern = def ? (fast ? DD_K5(true, true) : DD_K5(true, false)) : (fast ? DD_K5(false, true) : DD_K5(false, false));
-#undef DD_K5
+        kern = with_bool(params_are_default(p), [&](auto def) {
+            return with_bool(fast, [&](auto fa) {
+                return with_bool(f16, [&](auto h) { return policy_rollout_kernel<def, false, 3, fa, h>; });
+            });
+        });
     }
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
     if (err != cudaSuccess) return (int)err;
@@ -1030,27 +1023,20 @@ int dd_policy_rollout(const DDState* s, const DDParams* p, const DDEnvConfig* c,
     if (mode != DD_ACTION_THRESHOLD && mode != DD_ACTION_SAMPLE) return DD_E_RANGE;
     if (consts->operands != DD_OPERANDS_BF16 && consts->operands != DD_OPERANDS_FP16) return DD_E_RANGE;       // not filled by dd_policy_pack
     if (mode == DD_ACTION_SAMPLE && !(temperature > 0.0f)) return DD_E_RANGE;
-    if (T < 0 || n < 0 || n > (int64_t)DD_MAX_ENVS_PER_CALL) return DD_E_RANGE;
-    if (n > 0 && (!s->pos_vel || !s->att_fuel || !s->platform || !s->steps || !s->episode || !s->flags)) return DD_E_NULL;
-    if ((reinterpret_cast<uintptr_t>(s->pos_vel) | reinterpret_cast<uintptr_t>(s->att_fuel) | reinterpret_cast<uintptr_t>(blob)) & 15u) return DD_E_ALIGN;
-    if (reinterpret_cast<uintptr_t>(s->platform) & 7u) return DD_E_ALIGN;
+    if (T < 0) return DD_E_RANGE;
+    dd::PArgs pa{};
+    if (int rc = dd::fill_args(pa.a, s, p, c, n)) return rc;   // the env block of dd_rollout (K5 ignores obs_stride)
+    if (reinterpret_cast<uintptr_t>(blob) & 15u) return DD_E_ALIGN;
     if (shaped_tn && !s->prev_dist && n > 0) return DD_E_NULL;
     if (shaped_tn && c->shaping != DD_SHAPING_PPO && c->shaping != DD_SHAPING_PG) return DD_E_RANGE;
     if (n == 0 || T == 0) return 0;
-    dd::PArgs pa{};
     pa.pc = *consts;
-    pa.a.prev_dist = (float*)s->prev_dist; pa.shaped_tn = shaped_tn;
-    pa.a.pos_vel = (float*)s->pos_vel; pa.a.att_fuel = (float*)s->att_fuel; pa.a.platform = (float*)s->platform;
-    pa.a.steps = s->steps; pa.a.episode = s->episode; pa.a.flags = s->flags;
     pa.a.stats = (unsigned long long*)stats;
-    pa.a.n = (uint32_t)n; pa.a.seed = c->seed; pa.a.env_id_base = c->env_id_base; pa.a.max_steps = c->max_steps; pa.a.shaping = c->shaping;
-    pa.a.rand_drone = c->randomize_drone; pa.a.rand_platform = c->randomize_platform;
-    pa.a.k = dd::make_consts<float>(*p);
     pa.pre_margin = dd::pre_sc_margin(*p);
     pa.blob = (const uint8_t*)blob; pa.mode = mode; pa.t0 = t0; pa.T = T;
     pa.inv_temperature = mode == DD_ACTION_SAMPLE ? 1.0f / temperature : 1.0f;
     pa.actions_tn = actions_tn; pa.logp_tn = logp_tn; pa.reward_tn = reward_tn; pa.done_tn = done_tn;
-    pa.obs_tn = obs_tn; pa.probs_tn = probs_tn; pa.obs_in = nullptr; pa.auto_reset = c->auto_reset;
+    pa.obs_tn = obs_tn; pa.probs_tn = probs_tn; pa.shaped_tn = shaped_tn; pa.obs_in = nullptr; pa.auto_reset = c->auto_reset;
     return dd::policy_launch(pa, *p, n, false, (cudaStream_t)stream);
 }
 

@@ -7,6 +7,7 @@ import os
 import re
 import subprocess
 import sys
+import types
 
 import pytest
 import torch
@@ -87,19 +88,140 @@ def test_default_params_are_the_reference_config(lib):
     assert got == {k: float(v) for k, v in want.items()}
 
 
+NULL, RANGE, DTYPE, ALIGN = -1, -2, -3, -4
+RESET = ("dd_reset", "dd_reset_sets")
+STEP = ("dd_step", "dd_step_sets", "dd_step_plan", "dd_step_plan_sets")
+ROLL = ("dd_rollout", "dd_rollout_shaped", "dd_rollout_sets")
+SHAPED = ("dd_rollout_shaped", "dd_rollout_sets", "dd_policy_rollout")
+ENV = RESET + STEP + ROLL
+SETS = tuple(e for e in ENV if e.endswith("_sets"))
+SINGLE = tuple(e for e in ENV if not e.endswith("_sets"))
+K5, GATHER = ("dd_policy_rollout",), ("dd_gather_env",)
+
+# Each entry point called with the arguments of a namespace `a` (_env_call_args): fake device pointers, real host structs.
+_ENV_CALLS = {
+    "dd_reset": lambda L, a: L.dd_reset(a.s, a.p, a.c, None, a.obs, a.stride, a.n, None),
+    "dd_reset_sets": lambda L, a: L.dd_reset_sets(a.s, a.ps, a.c, None, a.obs, a.stride, a.n, None),
+    "dd_step": lambda L, a: L.dd_step(a.s, a.p, a.c, a.actions, a.obs, a.stride, None, None, a.final_obs, None, a.n, None),
+    "dd_step_sets": lambda L, a: L.dd_step_sets(a.s, a.ps, a.c, a.actions, a.obs, a.stride, None, None, a.final_obs, None,
+                                                a.n, None),
+    "dd_step_plan": lambda L, a: L.dd_step_plan(a.s, a.p, a.c, a.obs, a.stride, None, None, a.final_obs, None, a.n, C.byref(a.plan)),
+    "dd_step_plan_sets": lambda L, a: L.dd_step_plan_sets(a.s, a.ps, a.c, a.obs, a.stride, None, None, a.final_obs, None,
+                                                          a.n, C.byref(a.plan)),
+    "dd_rollout": lambda L, a: L.dd_rollout(a.s, a.p, a.c, a.policy, a.actions_tn, 0, a.T, None, None, a.obs, a.stride,
+                                            None, a.n, None),
+    "dd_rollout_shaped": lambda L, a: L.dd_rollout_shaped(a.s, a.p, a.c, a.policy, a.actions_tn, 0, a.T, None, None, a.obs,
+                                                          a.stride, a.shaped, None, a.n, None),
+    "dd_rollout_sets": lambda L, a: L.dd_rollout_sets(a.s, a.ps, a.c, a.policy, a.actions_tn, 0, a.T, None, None, a.obs,
+                                                      a.stride, a.shaped, None, a.n, None),
+    "dd_policy_rollout": lambda L, a: L.dd_policy_rollout(a.s, a.p, a.c, a.blob, a.consts, a.mode, a.temperature, 0, a.T,
+                                                          None, None, None, None, a.obs, None, a.shaped, None, a.n, None),
+    "dd_gather_env": lambda L, a: L.dd_gather_env(a.s, a.obs, a.stride, None, None, a.i, a.n, a.out, None),
+}
+
+
+def _env_call_args(**kw):
+    """A call that passes validation, but for the single fault in `kw`: `state_<field>`, `sets_<field>`, `cfg_<field>` and
+    `consts_<field>` set one struct field; `s`, `p`, `ps`, `c`, `consts` or `out` = None pass NULL for the struct."""
+    state = nv.DDState(16, 32, 48, 64, 80, 96, kw.get("state_dtype", nv.F32), 0, 112)
+    sets = nv.DDParamSets(4096, 8192, 2, state.dtype, 0, 0)           # the table is built for the state's dtype
+    cfg, consts = nv.DDEnvConfig(), nv.DDPolicyConsts()
+    consts.operands = nv.OPERANDS_BF16
+    for key, v in list(kw.items()):
+        for prefix, struct in (("state_", state), ("sets_", sets), ("cfg_", cfg), ("consts_", consts)):
+            if key.startswith(prefix):
+                setattr(struct, key[len(prefix):], v)
+                del kw[key]
+    a = dict(s=C.byref(state), p=C.byref(nv.default_params()), ps=C.byref(sets), c=C.byref(cfg), consts=C.byref(consts),
+             out=(C.c_double * nv.ENV_RECORD_DOUBLES)(), plan=nv.DDStepPlan(), n=8, T=4, obs=128, stride=15,
+             final_obs=None, actions=192, policy=nv.POLICY_RANDOM, actions_tn=None, shaped=None, blob=16384, mode=1,
+             temperature=1.0, i=0)
+    a.update(kw)
+    return types.SimpleNamespace(**a)
+
+
+_STATE_FIELDS = ("pos_vel", "att_fuel", "platform", "steps", "episode", "flags")
+_ARGUMENT_CASES = [
+    # NULL structs
+    (ENV + K5 + GATHER, dict(s=None), NULL),
+    (SINGLE + K5, dict(p=None), NULL),
+    (SETS, dict(ps=None), NULL),
+    (ENV + K5, dict(c=None), NULL),
+    (K5, dict(blob=None), NULL),
+    (K5, dict(consts=None), NULL),
+    (GATHER, dict(out=None), NULL),
+    # dtypes
+    (ENV + K5 + GATHER, dict(state_dtype=5), DTYPE),
+    (K5, dict(state_dtype=nv.F64), DTYPE),
+    (SETS, dict(sets_dtype=nv.F64), DTYPE),
+    (SETS, dict(state_dtype=nv.F64, sets_dtype=nv.F32), DTYPE),
+    # env counts
+    (ENV + K5, dict(n=-1), RANGE),
+    (ENV + K5, dict(n=0x7fffff01), RANGE),                             # DD_MAX_ENVS_PER_CALL + 1
+    (GATHER, dict(i=-1), RANGE),
+    (GATHER, dict(i=8), RANGE),
+    (GATHER, dict(n=-1), RANGE),
+    # state buffers
+    *[(ENV + K5 + GATHER, {"state_" + f: None}, NULL) for f in _STATE_FIELDS],
+    (ENV + K5, dict(state_pos_vel=24), ALIGN),
+    (ENV + K5, dict(state_att_fuel=40), ALIGN),
+    (ENV + K5, dict(state_platform=52), ALIGN),
+    (ENV, dict(state_dtype=nv.F64, state_platform=56), ALIGN),
+    # observations
+    (ENV + GATHER, dict(stride=14), RANGE),
+    (ENV + GATHER, dict(stride=17), RANGE),
+    (STEP, dict(obs=None, final_obs=256, stride=14), RANGE),
+    (ENV, dict(cfg_obs_format=3), RANGE),
+    (ENV, dict(cfg_obs_format=-1), RANGE),
+    (ENV, dict(state_dtype=nv.F64, cfg_obs_format=nv.OBS_F16), DTYPE),
+    (ENV, dict(state_dtype=nv.F64, cfg_obs_format=nv.OBS_BF16), DTYPE),
+    # actions and policies
+    (("dd_step", "dd_step_sets"), dict(actions=None), NULL),
+    (ROLL, dict(policy=3), RANGE),
+    (ROLL, dict(policy=-1), RANGE),
+    (ROLL + K5, dict(T=-1), RANGE),
+    (ROLL, dict(policy=nv.POLICY_TRACE), NULL),
+    # shaped training reward
+    (SHAPED, dict(shaped=256, state_prev_dist=None), NULL),
+    (SHAPED, dict(shaped=256, cfg_shaping=2), RANGE),
+    # the fused policy rollout
+    (K5, dict(mode=2), RANGE),
+    (K5, dict(mode=-1), RANGE),
+    (K5, dict(temperature=0.0), RANGE),
+    (K5, dict(temperature=-1.0), RANGE),
+    (K5, dict(temperature=float("nan")), RANGE),
+    (K5, dict(consts_operands=nv.OPERANDS_AUTO), RANGE),
+    (K5, dict(consts_operands=3), RANGE),
+    (K5, dict(blob=16392), ALIGN),
+    # parameter sets
+    (SETS, dict(sets_table=None), NULL),
+    (SETS, dict(sets_index=None), NULL),
+    (SETS, dict(sets_count=0), RANGE),
+    (SETS, dict(sets_count=65), RANGE),
+    (SETS, dict(sets_flags=2), RANGE),
+    (SETS, dict(sets_table=4104), ALIGN),
+    # nothing to do: no buffer is needed and no CUDA call is made
+    (RESET + ("dd_step", "dd_step_sets") + ROLL + K5, dict(n=0, **{"state_" + f: None for f in _STATE_FIELDS}), 0),
+    (ROLL + K5, dict(T=0), 0),
+]
+
+
 def test_argument_errors_without_a_gpu(lib):
-    """Validation happens before any CUDA call, so it is testable here."""
+    """Validation happens before any CUDA call, so it is testable here: one call per check, each with a single fault,
+    pins the code every env entry point returns for it."""
+    for entries, fault, want in _ARGUMENT_CASES:
+        for name in entries:
+            a = _env_call_args(**fault)
+            assert _ENV_CALLS[name](lib, a) == want, (name, fault)
+            if name.startswith("dd_step_plan"):
+                assert all(w == 0 for w in a.plan.opaque), (name, fault)
+    assert lib.dd_step_planned(None, 192, None) == NULL
+    assert lib.dd_step_planned(C.byref(nv.DDStepPlan()), 192, None) == RANGE      # zeroed: not a plan
     assert lib.dd_step(None, None, None, None, None, 15, None, None, None, None, 8, None) == -1
     assert lib.dd_reset(None, None, None, None, None, 15, 8, None) == -1
     assert lib.dd_moments(None, 4, None, None) == -1
     assert lib.dd_gae(None, None, None, None, None, 0.99, 0.95, 4, 4, None) == -1
     assert lib.dd_pack_actions(None, None, 4, None) == -1
-    st = nv.DDState(16, 32, 48, 64, 80, 96, 5)
-    assert lib.dd_reset(C.byref(st), C.byref(nv.default_params()), C.byref(nv.DDEnvConfig()), None, None, 15, 8, None) == -3
-    st.dtype = nv.F32
-    assert lib.dd_reset(C.byref(st), C.byref(nv.default_params()), C.byref(nv.DDEnvConfig()), None, None, 15, -1, None) == -2
-    st.pos_vel = 20
-    assert lib.dd_reset(C.byref(st), C.byref(nv.default_params()), C.byref(nv.DDEnvConfig()), None, None, 15, 8, None) == -4
     for code, word in ((0, b"ok"), (-1, b"null"), (-2, b"range"), (-3, b"dtype"), (-4, b"align")):
         assert word in lib.dd_error_string(code)
 

@@ -163,7 +163,7 @@ const char *dd_error_string(int code);
  *     through the single-set entry point: spawn ranges and default spawn, max_fuel at reset, terminal rewards, shaping
  *     constants and observation normalisation.  An out-of-range index is clamped to count-1, never read out of bounds.
  *   Resampling (flags & DD_PARAM_SETS_RESAMPLE).  Each reset of env i -- masked resets of dd_reset_sets, same-step
- *     auto-resets of dd_step_sets / dd_rollout_sets -- draws s = mulhi32(r.a, count) with
+ *     auto-resets of dd_step_sets / dd_rollout_sets / dd_policy_rollout_sets -- draws s = mulhi32(r.a, count) with
  *     r = Philox4x32-10(counter = (env_id lo, env_id hi, episode, 3), key = seed), writes index[i] = s and spawns under
  *     set s.  `episode` is the counter the spawn itself uses (read before the increment); counter word 3 = 3 is a stream
  *     no other draw uses (spawns 0, random actions 1, dd_policy_rollout's Bernoulli uniforms 2).  The step that ends an
@@ -174,7 +174,7 @@ const char *dd_error_string(int code);
  *     aligned: DD_E_ALIGN; and every check of the single-set entry point, with the same codes.
  *   Plans.  dd_step_plan_sets keeps the table and index POINTERS: in-place edits of index[] or of the table contents
  *     reach the next dd_step_planned and captured graphs.  A different count or flags value needs a new plan.
- * dd_policy_rollout and dd_gather_env take no parameter sets. */
+ * The fused policy rollout takes them through dd_policy_rollout_sets (K5 section below); dd_gather_env takes none. */
 #define DD_MAX_PARAM_SETS      64
 #define DD_PARAM_TABLE_BYTES   32768     /* fixed size: room for 64 sets of the float64 derived constants */
 #define DD_PARAM_SETS_RESAMPLE 0x01
@@ -382,6 +382,18 @@ int dd_policy_rollout(const DDState *s, const DDParams *p, const DDEnvConfig *c,
                       const DDPolicyConsts *consts, int32_t mode, float temperature, uint32_t t0, int32_t T, uint8_t *actions_tn, float *logp_tn, float *reward_tn,
                       uint8_t *done_tn, float *obs_tn, float *probs_tn, float *shaped_tn, uint64_t *stats, int64_t n,
                       void *stream);
+
+/* dd_policy_rollout with per-env parameter sets (DDParamSets, "per-environment physics parameter sets" above) in place of
+ * DDParams: domain randomisation while the policy collects.  Env i steps, observes (the network input too), shapes and
+ * resets under set min(index[i], count-1); under DD_PARAM_SETS_RESAMPLE every same-step auto-reset draws the stream-3 set,
+ * writes index[i] and spawns under it, and the observation after it -- the next network input -- is normalised by the
+ * new set.  The Bernoulli uniforms, t0, modes, temperature and outputs are those of dd_policy_rollout.  Validation: the
+ * checks of dd_policy_rollout and the DDParamSets checks, with the same codes, before any CUDA call (DD_F32 state and
+ * table only). */
+int dd_policy_rollout_sets(const DDState *s, const DDParamSets *ps, const DDEnvConfig *c, const void *blob,
+                           const DDPolicyConsts *consts, int32_t mode, float temperature, uint32_t t0, int32_t T,
+                           uint8_t *actions_tn, float *logp_tn, float *reward_tn, uint8_t *done_tn, float *obs_tn,
+                           float *probs_tn, float *shaped_tn, uint64_t *stats, int64_t n, void *stream);
 
 /* Launch shape of dd_policy_rollout (pure host function; what the launcher itself uses): the number of CTAs for n envs on
  * a device with `sms` SMs.  Slot g (0..3) of CTA b runs the tile of 128 envs number b + grid * g (if it exists).  Up to 3

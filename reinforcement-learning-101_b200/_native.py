@@ -217,6 +217,8 @@ def lib():
     L.dd_value_forward.argtypes = [vp, C.POINTER(DDPolicyConsts), vp, vp, i64, vp]
     L.dd_policy_rollout.restype = C.c_int
     L.dd_policy_rollout.argtypes = [PS, PP, PC, vp, C.POINTER(DDPolicyConsts), i32, C.c_float, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
+    L.dd_policy_rollout_sets.restype = C.c_int
+    L.dd_policy_rollout_sets.argtypes = [PS, PSS, PC, vp, C.POINTER(DDPolicyConsts), i32, C.c_float, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
     L.dd_policy_rollout_grid.restype = C.c_int
     L.dd_policy_rollout_grid.argtypes = [i64, i32]
     if L.dd_abi_version() != ABI_VERSION:
@@ -255,7 +257,7 @@ EXPORTS = (
     "dd_rollout", "dd_rollout_shaped",
     "dd_param_sets_build", "dd_reset_sets", "dd_step_sets", "dd_step_plan_sets", "dd_rollout_sets",
     "dd_fill_random_actions", "dd_pack_actions", "dd_stats_collapse", "dd_moments", "dd_normalize", "dd_gae", "dd_gae_moments",
-    "dd_policy_pack", "dd_policy_pack_ex", "dd_policy_forward", "dd_policy_rollout", "dd_policy_rollout_grid", "dd_value_pack", "dd_value_forward", "dd_gather_env", "dd_discounted_returns",
+    "dd_policy_pack", "dd_policy_pack_ex", "dd_policy_forward", "dd_policy_rollout", "dd_policy_rollout_sets", "dd_policy_rollout_grid", "dd_value_pack", "dd_value_forward", "dd_gather_env", "dd_discounted_returns",
 )
 HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host", "dd_obs16_convert_host",
                      "dd_param_sets_build_host", "dd_reset_sets_host", "dd_step_sets_host", "dd_rollout_sets_host")

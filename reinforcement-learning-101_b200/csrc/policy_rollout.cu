@@ -150,6 +150,27 @@ struct PArgs {
     float pre_margin;          // dd::pre_sc_margin of the parameters (the DEF instantiations use its default-world 1e-3)
 };
 
+// The argument block of the per-env parameter-set instantiation (SETS = true): PArgs (whose a.k and pre_margin it does not
+// read) + the DDParamSets fields.  Appended, so that the single-set kernels keep their argument layout.
+struct PArgsPS : PArgs {
+    const void* ps_table;      // Consts<float> [word][set], drone_core.cuh param_set
+    uint8_t* ps_index;
+    uint32_t ps_count;
+    int32_t ps_resample;       // DD_PARAM_SETS_RESAMPLE
+};
+template <bool SETS> using PArgsOf = typename std::conditional<SETS, PArgsPS, PArgs>::type;
+
+// pre_sc_margin (drone_core.cuh) of a set, from its derived constants on the device, rounded up: x_hi / y_hi are the world
+// extent rounded to float (which can only raise its binade), and the sum and product round upwards with a factor above
+// 1e-5 that covers half_h's own rounding -- never below the host's value, so the shortcut decides as the exact path does.
+__device__ __forceinline__ float pre_sc_margin_of(const Consts<float>& k)
+{
+    const float far = fabsf(fmaxf(k.x_hi, k.y_hi));
+    const int e = max((int)((__float_as_uint(far) >> 23) & 0xffu) - 127, -100);   // far in [2^e, 2^(e+1))
+    const float ulp8 = __uint_as_float((uint32_t)(e - 20 + 127) << 23);             // 8 float ulps there: 2^(e-20)
+    return fmaxf(__fadd_ru(ulp8, __fmul_ru(1.0001e-5f, fabsf(k.half_h))), 1e-3f);
+}
+
 // ---- raw PTX wrappers -----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -383,9 +404,15 @@ __device__ __forceinline__ void store_a_chunk_relu_tmem(uint32_t ta, int c, cons
 // probabilities) -- with every launch-constant switch a compile-time constant: predicated-off stores, their address
 // arithmetic and the selects between modes still cost issue slots, and this kernel is bound by them.
 // F16: the operand images in the blob and the activations are fp16 (else bf16); chosen by dd_policy_pack.
-template <bool DEF, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false>
-__global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __grid_constant__ PArgs pa)
+// SETS (rollout, DEF = false only): per-env parameter sets (PArgsPS).  Env i runs under set min(index[i], count - 1); its
+// constants are not held over the step (the 128-register cap leaves no room for them) but read from the [word][set] table
+// through L1 where they are used: the observation's at the top of the step, the env step's (and its landing margin,
+// pre_sc_margin_of) under the head MMA.  Under ps_resample the set of the NEXT episode is drawn with its spawn, ahead of
+// time; the reset switches to it (index[i] is written back once, at the end).
+template <bool DEF, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false, bool SETS = false>
+__global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __grid_constant__ PArgsOf<SETS> pa)
 {
+    static_assert(!SETS || (!DEF && !FWD && HEAD == 3), "parameter sets: rollout instantiations with generic constants only");
     extern __shared__ __align__(1024) uint8_t smem[];
     const KArgs<float>& a = pa.a;
     const Consts<float> k = consts_of<float, DEF>(a);
@@ -459,6 +486,8 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
     Env<float> e = {};
     uint32_t pflags = 0, ep = 0;
     bool platform_dirty = false;
+    uint32_t set = 0, nset = 0;                              // SETS: my set, and the set of my env's next episode
+    bool set_dirty = false;
     if (live && !forward_only) {
         load4(a.pos_vel, i, e.x, e.y, e.vx, e.vy);
         load4(a.att_fuel, i, e.angle, e.angvel, e.fuel, e.ret);
@@ -466,6 +495,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         e.steps = a.steps[i];
         pflags = a.flags[i];
         ep = a.episode[i];
+        if constexpr (SETS) set = param_set_clamp(pa.ps_index[i], pa.ps_count);
     }
     const uint64_t gid = a.env_id_base + (uint64_t)i;
     float speed = 0.f, dist = 0.f;
@@ -475,8 +505,15 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
     // it run under the second MMA of the following step (same spawn_draw as spawn(): bit-identical resets).
     float nsx = 0.f, nsy = 0.f, nspx = 0.f, nspy = 0.f, nsdist = 0.f;
     bool need_spawn = false;
+    // SETS: the next episode's set is a function of (seed, env id, ep) too -- drawn here, and the spawn under its ranges.
     auto draw_next_spawn = [&]() {
-        spawn_draw(k, a.seed, gid, ep, a.rand_drone != 0, a.rand_platform != 0, nsx, nsy, nspx, nspy);
+        if constexpr (SETS) {
+            nset = pa.ps_resample ? param_set_draw(a.seed, gid, ep, pa.ps_count) : set;
+            spawn_draw(param_set<float>(pa.ps_table, nset), a.seed, gid, ep, a.rand_drone != 0, a.rand_platform != 0,
+                       nsx, nsy, nspx, nspy);
+        } else {
+            spawn_draw(k, a.seed, gid, ep, a.rand_drone != 0, a.rand_platform != 0, nsx, nsy, nspx, nspy);
+        }
         const float ddx = nspx - nsx, ddy = nspy - nsy;                       // speed_dist() of the fresh state
         nsdist = Arith<float>::sqrt_(Arith<float>::fma_(ddx, ddx, Arith<float>::mul(ddy, ddy)));
     };
@@ -496,7 +533,9 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
     const uint32_t obs_bytes = (tile0 < a.n ? (a.n - tile0 < (uint32_t)kTile ? a.n - tile0 : (uint32_t)kTile) : 0u) * (kIn * 4u);
     const bool obs_bulk = obs_out && tile0 < a.n && (a.n & 3u) == 0u &&
                           (reinterpret_cast<uintptr_t>(pa.obs_tn) & 15u) == 0u;
-    float dprev = nan_of<float>(), dcur = dist * k.inv_width;
+    float dprev = nan_of<float>(), dcur;
+    if constexpr (SETS) dcur = dist * param_set<float>(pa.ps_table, set).inv_width;
+    else dcur = dist * k.inv_width;
     if (live && shaping) dprev = a.prev_dist[i];
 
     // Outputs of a step that nothing in the NEXT step's network input depends on (log-prob, the action / log-prob /
@@ -539,6 +578,8 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
 #pragma unroll
                 for (int j = 0; j < kIn; ++j) ob[j] = live ? pa.obs_in[(size_t)i * kIn + j] : 0.f;
             }
+        } else if constexpr (SETS) {                         // my set's normalisation (the new set's after a reset)
+            write_obs(e, pflags, speed, dist, param_set<float>(pa.ps_table, set), [&](int j, float v) { ob[j] = v; });
         } else {
             write_obs(e, pflags, speed, dist, k, [&](int j, float v) { ob[j] = v; });
         }
@@ -635,6 +676,8 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
             umma_commit(bar);
         }
         constexpr bool mma_head = HEAD == 3;                 // the critic's one-row head stays on the CUDA cores, in fp32
+        Consts<float> ks;                                    // SETS: this step's constants, read under the head MMA
+        float ks_margin = 0.f, ks_next_fuel = 0.f;
         float s_pre = 0.f, c_pre = 1.f;                      // under the third MMA (the fourth with the tensor-core head): sin / cos of the pre-update angle
         if (!forward_only && !mma_head) { Arith<float>::sincos_deg(e.angle, s_pre, c_pre); pin(s_pre); pin(c_pre); }   // (main thrust, drone.py:58-66)
         wait_mma(bar, phase, issuer_warp, g);
@@ -658,6 +701,11 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
                 umma_commit(bar);
             }
             if (!forward_only) { Arith<float>::sincos_deg(e.angle, s_pre, c_pre); pin(s_pre); pin(c_pre); }   // under the head MMA
+            if constexpr (SETS) {                             // and, for the env step, my set's constants
+                ks = param_set<float>(pa.ps_table, set);
+                ks_margin = pre_sc_margin_of(ks);
+                ks_next_fuel = param_set<float>(pa.ps_table, nset).max_fuel;   // a reset's tank: the next episode's set
+            }
             wait_mma(bar, phase, issuer_warp, g);             // (sin / cos under MMA3 instead, or all four warps on the mbarrier: measured equal or slower)
             TmemChunk<8> d4;
             d4.issue(trow + 32u);
@@ -719,24 +767,48 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         uint32_t oflags = pflags;
         float reward = 0.f, shaped = 0.f;
         if (live && !(pflags & DD_DONE)) {
-            uint32_t f = step_core<float, true, true>(e, act, k, reward, speed, dist, s_pre, c_pre, DEF ? 1e-3f : pa.pre_margin);
+            uint32_t f;
+            if constexpr (SETS) f = step_core<float, true, true>(e, act, ks, reward, speed, dist, s_pre, c_pre, ks_margin);
+            else f = step_core<float, true, true>(e, act, k, reward, speed, dist, s_pre, c_pre, DEF ? 1e-3f : pa.pre_margin);
             if (!f && max_steps > 0 && e.steps >= max_steps) f = DD_DONE | DD_TRUNCATED;
             oflags = f;
             if (shaping) {
-                shaped = shaped_reward(a.shaping, e, f, speed, dist, dprev, max_steps > 0 && e.steps >= max_steps, k);
-                dprev = dcur;
-                dcur = Arith<float>::div(dist, k.width, k.inv_width);
+                if constexpr (SETS) {
+                    shaped = shaped_reward(a.shaping, e, f, speed, dist, dprev, max_steps > 0 && e.steps >= max_steps, ks);
+                    dprev = dcur;
+                    dcur = Arith<float>::div(dist, ks.width, ks.inv_width);
+                } else {
+                    shaped = shaped_reward(a.shaping, e, f, speed, dist, dprev, max_steps > 0 && e.steps >= max_steps, k);
+                    dprev = dcur;
+                    dcur = Arith<float>::div(dist, k.width, k.inv_width);
+                }
             }
             if (f) {
                 if (do_stats) st.add(f, e.ret, e.steps);     // per-thread totals (a few predicated adds in the episode-end branch)
                 if (auto_reset) {
-                    spawn_apply(e, k, nsx, nsy, nspx, nspy);                   // == spawn(e, ..., ep): drawn ahead of time
+                    if constexpr (SETS) {                      // the step above ran under the old set, the new episode under nset
+                        Consts<float> kn = ks;
+                        kn.max_fuel = ks_next_fuel;            // (spawn_apply reads max_fuel only)
+                        spawn_apply(e, kn, nsx, nsy, nspx, nspy);
+                        if (pa.ps_resample) set_dirty = true;
+                        set = nset;
+                    } else {
+                        spawn_apply(e, k, nsx, nsy, nspx, nspy);               // == spawn(e, ..., ep): drawn ahead of time
+                    }
                     ep += 1;
                     need_spawn = true;
                     platform_dirty = true;
                     f = 0;
                     speed = 0.f; dist = nsdist;                               // == speed_dist(e, ...) of a fresh episode (v = 0)
-                    if (shaping) { dprev = nan_of<float>(); dcur = Arith<float>::div(dist, k.width, k.inv_width); }
+                    if (shaping) {
+                        dprev = nan_of<float>();
+                        if constexpr (SETS) {
+                            const Consts<float> kn = param_set<float>(pa.ps_table, set);
+                            dcur = Arith<float>::div(dist, kn.width, kn.inv_width);
+                        } else {
+                            dcur = Arith<float>::div(dist, k.width, k.inv_width);
+                        }
+                    }
                 }
             }
             pflags = f;
@@ -755,6 +827,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         a.episode[i] = ep;
         if (platform_dirty) store2(a.platform, i, e.px, e.py);
         if (shaping) a.prev_dist[i] = dprev;
+        if constexpr (SETS) { if (set_dirty) pa.ps_index[i] = (uint8_t)set; }
     }
     if (obs_bulk && issuer_warp && elect_one()) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     // ---- teardown: everyone is done with TMEM, then the allocating warp frees it ----
@@ -909,37 +982,85 @@ static int rollout_grid(int64_t n, int sms)
     return (int)blocks;
 }
 
-static int policy_launch(PArgs& pa, const DDParams& p, int64_t n, bool forward, cudaStream_t st)
+// On the device that owns the stream (or the blob): pick(sms, grid) chooses the kernel and its grid, then one launch.
+template <typename PA, typename Pick>
+static int policy_launch(PA& pa, cudaStream_t st, Pick&& pick)
 {
-    const int blocks = (int)((n + kTile * kGroups - 1) / (kTile * kGroups));
-    DeviceGuard guard(st, pa.blob);                         // the device that owns the stream (or the blob)
+    DeviceGuard guard(st, pa.blob);
     if (guard.err != cudaSuccess) return (int)guard.err;
     int sms = 0;
     const cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, guard.dev);
     if (e != cudaSuccess) return (int)e;
-    void (*kern)(PArgs);
-    int grid;
-    const bool f16 = pa.pc.operands == DD_OPERANDS_FP16;
-    if (forward) {
-        kern = with_bool(f16, [&](auto h) {
-            return pa.head == 1 ? policy_rollout_kernel<true, true, 1, false, h> : policy_rollout_kernel<true, true, 3, false, h>;
-        });
-        grid = blocks < sms ? blocks : sms;                 // persistent: one CTA per SM walks the row blocks
-        pa.T = (blocks + grid - 1) / grid;
-    } else {
-        grid = rollout_grid(n, sms);
-        const bool fast = pa.mode == DD_ACTION_SAMPLE && pa.inv_temperature == 1.0f && pa.auto_reset && pa.a.stats &&
-                          pa.actions_tn && pa.logp_tn && pa.reward_tn && pa.done_tn && pa.obs_tn && !pa.shaped_tn && !pa.probs_tn;
-        kern = with_bool(params_are_default(p), [&](auto def) {
-            return with_bool(fast, [&](auto fa) {
-                return with_bool(f16, [&](auto h) { return policy_rollout_kernel<def, false, 3, fa, h>; });
-            });
-        });
-    }
+    int grid = 0;
+    void (*kern)(PA) = pick(sms, grid);
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal);
     if (err != cudaSuccess) return (int)err;
     kern<<<grid, kPolThreads, kSmemTotal, st>>>(pa);
     return (int)cudaGetLastError();
+}
+
+// The rollout launch (single set: p; per-env sets: SETS).  FAST is the PPO-collection configuration of the kernel's header.
+template <bool SETS>
+static int rollout_launch(PArgsOf<SETS>& pa, const DDParams* p, int64_t n, cudaStream_t st)
+{
+    const bool fast = pa.mode == DD_ACTION_SAMPLE && pa.inv_temperature == 1.0f && pa.auto_reset && pa.a.stats &&
+                      pa.actions_tn && pa.logp_tn && pa.reward_tn && pa.done_tn && pa.obs_tn && !pa.shaped_tn && !pa.probs_tn;
+    const bool f16 = pa.pc.operands == DD_OPERANDS_FP16;
+    return policy_launch(pa, st, [&](int sms, int& grid) {
+        grid = rollout_grid(n, sms);
+        return with_bool(fast, [&](auto fa) {
+            return with_bool(f16, [&](auto h) {
+                if constexpr (SETS) return policy_rollout_kernel<false, false, 3, fa, h, true>;
+                else return with_bool(params_are_default(*p), [&](auto def) { return policy_rollout_kernel<def, false, 3, fa, h>; });
+            });
+        });
+    });
+}
+
+// The env part of the argument block: fill_args (env_abi.h) of a DDParams, or of a DDParamSets with its fields appended.
+static int fill_env(PArgs& pa, const DDState* s, const DDParams* p, const DDEnvConfig* c, int64_t n)
+{
+    if (int rc = fill_args(pa.a, s, p, c, n)) return rc;    // the env block of dd_rollout (K5 ignores obs_stride)
+    pa.pre_margin = pre_sc_margin(*p);
+    return 0;
+}
+static int fill_env(PArgsPS& pa, const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, int64_t n)
+{
+    KArgsPS<float> a;
+    if (int rc = fill_args(a, s, ps, c, n)) return rc;
+    pa.a = a;
+    pa.ps_table = a.ps_table; pa.ps_index = a.ps_index; pa.ps_count = a.ps_count; pa.ps_resample = a.ps_resample;
+    return 0;
+}
+
+// dd_policy_rollout (P = DDParams) and dd_policy_rollout_sets (P = DDParamSets): the K5 checks, fill_env's, then the launch.
+template <typename P>
+static int policy_rollout_impl(const DDState* s, const P* p, const DDEnvConfig* c, const void* blob, const DDPolicyConsts* consts,
+                               int32_t mode, float temperature, uint32_t t0, int32_t T, uint8_t* actions_tn, float* logp_tn,
+                               float* reward_tn, uint8_t* done_tn, float* obs_tn, float* probs_tn, float* shaped_tn,
+                               uint64_t* stats, int64_t n, cudaStream_t st)
+{
+    constexpr bool SETS = std::is_same<P, DDParamSets>::value;
+    if (!s || !p || !c || !blob || !consts) return DD_E_NULL;
+    if (s->dtype != DD_F32) return DD_E_DTYPE;                 // the fused kernel is the fp32 throughput path
+    if (mode != DD_ACTION_THRESHOLD && mode != DD_ACTION_SAMPLE) return DD_E_RANGE;
+    if (consts->operands != DD_OPERANDS_BF16 && consts->operands != DD_OPERANDS_FP16) return DD_E_RANGE;       // not filled by dd_policy_pack
+    if (mode == DD_ACTION_SAMPLE && !(temperature > 0.0f)) return DD_E_RANGE;
+    if (T < 0) return DD_E_RANGE;
+    PArgsOf<SETS> pa{};
+    if (int rc = fill_env(pa, s, p, c, n)) return rc;
+    if (reinterpret_cast<uintptr_t>(blob) & 15u) return DD_E_ALIGN;
+    if (shaped_tn && !s->prev_dist && n > 0) return DD_E_NULL;
+    if (shaped_tn && c->shaping != DD_SHAPING_PPO && c->shaping != DD_SHAPING_PG) return DD_E_RANGE;
+    if (n == 0 || T == 0) return 0;
+    pa.pc = *consts;
+    pa.a.stats = (unsigned long long*)stats;
+    pa.blob = (const uint8_t*)blob; pa.mode = mode; pa.t0 = t0; pa.T = T;
+    pa.inv_temperature = mode == DD_ACTION_SAMPLE ? 1.0f / temperature : 1.0f;
+    pa.actions_tn = actions_tn; pa.logp_tn = logp_tn; pa.reward_tn = reward_tn; pa.done_tn = done_tn;
+    pa.obs_tn = obs_tn; pa.probs_tn = probs_tn; pa.shaped_tn = shaped_tn; pa.obs_in = nullptr; pa.auto_reset = c->auto_reset;
+    if constexpr (SETS) return rollout_launch<true>(pa, nullptr, n, st);
+    else return rollout_launch<false>(pa, p, n, st);
 }
 
 static int pack_common(const DDPolicy* p, int head, int operands, void* blob, DDPolicyConsts* consts, void* stream)
@@ -975,8 +1096,15 @@ static int forward_common(const void* blob, const DDPolicyConsts* consts, const 
     pa.pc = *consts;
     pa.a.n = (uint32_t)n;
     pa.blob = (const uint8_t*)blob; pa.T = 1; pa.obs_in = obs; pa.probs_tn = out; pa.head = head;
-    DDParams p = kDefaultParams;
-    return policy_launch(pa, p, n, true, (cudaStream_t)stream);
+    const bool f16 = pa.pc.operands == DD_OPERANDS_FP16;
+    const int blocks = (int)((n + kTile * kGroups - 1) / (kTile * kGroups));
+    return policy_launch(pa, (cudaStream_t)stream, [&](int sms, int& grid) {
+        grid = blocks < sms ? blocks : sms;                 // persistent: one CTA per SM walks the row blocks
+        pa.T = (blocks + grid - 1) / grid;
+        return with_bool(f16, [&](auto h) {
+            return pa.head == 1 ? policy_rollout_kernel<true, true, 1, false, h> : policy_rollout_kernel<true, true, 3, false, h>;
+        });
+    });
 }
 
 }  // namespace dd
@@ -1018,26 +1146,17 @@ int dd_policy_rollout(const DDState* s, const DDParams* p, const DDEnvConfig* c,
                       const DDPolicyConsts* consts, int32_t mode, float temperature, uint32_t t0, int32_t T, uint8_t* actions_tn, float* logp_tn, float* reward_tn, uint8_t* done_tn,
                       float* obs_tn, float* probs_tn, float* shaped_tn, uint64_t* stats, int64_t n, void* stream)
 {
-    if (!s || !p || !c || !blob || !consts) return DD_E_NULL;
-    if (s->dtype != DD_F32) return DD_E_DTYPE;                 // the fused kernel is the fp32 throughput path
-    if (mode != DD_ACTION_THRESHOLD && mode != DD_ACTION_SAMPLE) return DD_E_RANGE;
-    if (consts->operands != DD_OPERANDS_BF16 && consts->operands != DD_OPERANDS_FP16) return DD_E_RANGE;       // not filled by dd_policy_pack
-    if (mode == DD_ACTION_SAMPLE && !(temperature > 0.0f)) return DD_E_RANGE;
-    if (T < 0) return DD_E_RANGE;
-    dd::PArgs pa{};
-    if (int rc = dd::fill_args(pa.a, s, p, c, n)) return rc;   // the env block of dd_rollout (K5 ignores obs_stride)
-    if (reinterpret_cast<uintptr_t>(blob) & 15u) return DD_E_ALIGN;
-    if (shaped_tn && !s->prev_dist && n > 0) return DD_E_NULL;
-    if (shaped_tn && c->shaping != DD_SHAPING_PPO && c->shaping != DD_SHAPING_PG) return DD_E_RANGE;
-    if (n == 0 || T == 0) return 0;
-    pa.pc = *consts;
-    pa.a.stats = (unsigned long long*)stats;
-    pa.pre_margin = dd::pre_sc_margin(*p);
-    pa.blob = (const uint8_t*)blob; pa.mode = mode; pa.t0 = t0; pa.T = T;
-    pa.inv_temperature = mode == DD_ACTION_SAMPLE ? 1.0f / temperature : 1.0f;
-    pa.actions_tn = actions_tn; pa.logp_tn = logp_tn; pa.reward_tn = reward_tn; pa.done_tn = done_tn;
-    pa.obs_tn = obs_tn; pa.probs_tn = probs_tn; pa.shaped_tn = shaped_tn; pa.obs_in = nullptr; pa.auto_reset = c->auto_reset;
-    return dd::policy_launch(pa, *p, n, false, (cudaStream_t)stream);
+    return dd::policy_rollout_impl(s, p, c, blob, consts, mode, temperature, t0, T, actions_tn, logp_tn, reward_tn, done_tn,
+                                   obs_tn, probs_tn, shaped_tn, stats, n, (cudaStream_t)stream);
+}
+
+int dd_policy_rollout_sets(const DDState* s, const DDParamSets* ps, const DDEnvConfig* c, const void* blob,
+                           const DDPolicyConsts* consts, int32_t mode, float temperature, uint32_t t0, int32_t T, uint8_t* actions_tn,
+                           float* logp_tn, float* reward_tn, uint8_t* done_tn, float* obs_tn, float* probs_tn, float* shaped_tn,
+                           uint64_t* stats, int64_t n, void* stream)
+{
+    return dd::policy_rollout_impl(s, ps, c, blob, consts, mode, temperature, t0, T, actions_tn, logp_tn, reward_tn, done_tn,
+                                   obs_tn, probs_tn, shaped_tn, stats, n, (cudaStream_t)stream);
 }
 
 }  // extern "C"

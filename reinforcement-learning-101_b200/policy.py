@@ -140,16 +140,20 @@ def policy_rollout(env: BatchedDroneEnv, blob: PolicyBlob, T: int, sample: bool 
     iterations explore with fresh noise.  ``obs[t]`` is the observation BEFORE step t (the network input).
     ``temperature``: the evaluation sampling of the notebooks' ``evaluate_policy_simple`` (c18) -- actions drawn from
     ``p**(1/t) / (p**(1/t) + (1-p)**(1/t))``; 0 means ``probs > 0.5`` (like ``sample=False``), 1 the policy itself.
+    With per-env parameter sets (``env.set_param_sets``) every env runs under its own set, resampled at its auto-resets
+    if the env asks for that (include/drone_b200.h, dd_policy_rollout_sets); in-place edits of ``env.param_index`` take
+    effect at the next call.
     Returns the dict of buffers (allocated unless passed in ``out``)."""
+    if not isinstance(blob, PolicyBlob) or blob.head != 3:
+        got = "a critic blob (head=1)" if isinstance(blob, PolicyBlob) else type(blob).__name__
+        sets = " for an env with per-env parameter sets" if env.param_sets is not None else ""
+        raise ValueError(f"policy_rollout needs a policy PolicyBlob (head=3){sets}, got {got}")
     if temperature < 0:
         raise ValueError("temperature must be >= 0")
     if temperature == 0:
         sample, temperature = False, 1.0
     if env.dtype != torch.float32:
         raise ValueError("policy_rollout needs a float32 env")
-    if env.param_sets is not None:
-        raise ValueError("policy_rollout does not take per-env parameter sets: the fused policy kernel runs one DDParams "
-                         "per launch (call env.set_param_sets(None) first)")
     if env._needs_reset:
         raise RuntimeError("call reset() before policy_rollout()")
     n, dev = env.num_envs, env.device
@@ -169,10 +173,12 @@ def policy_rollout(env: BatchedDroneEnv, blob: PolicyBlob, T: int, sample: bool 
     if "shaped" in bufs:
         env._fresh_prev_dist()
     t0 = env._take_t0(t0, T)
-    nv.check(nv.lib().dd_policy_rollout(
-        C.byref(env._state), C.byref(env._params), C.byref(env._cfg), blob.blob.data_ptr(), C.byref(blob.consts),
+    fn, pargs = ((nv.lib().dd_policy_rollout, C.byref(env._params)) if env._ps is None
+                 else (nv.lib().dd_policy_rollout_sets, C.byref(env._ps)))
+    nv.check(fn(
+        C.byref(env._state), pargs, C.byref(env._cfg), blob.blob.data_ptr(), C.byref(blob.consts),
         ACTION_SAMPLE if sample else ACTION_THRESHOLD, float(temperature), int(t0), int(T), ptr("actions"), ptr("logp"), ptr("reward"),
         ptr("done"), ptr("obs"), ptr("probs"), ptr("shaped"), env.stats_slots.data_ptr() if stats else None, n,
         env._stream()),
-        "dd_policy_rollout")
+        fn.__name__)
     return bufs

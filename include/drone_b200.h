@@ -174,10 +174,19 @@ const char *dd_error_string(int code);
  *     aligned: DD_E_ALIGN; and every check of the single-set entry point, with the same codes.
  *   Plans.  dd_step_plan_sets keeps the table and index POINTERS: in-place edits of index[] or of the table contents
  *     reach the next dd_step_planned and captured graphs.  A different count or flags value needs a new plan.
- * The fused policy rollout takes them through dd_policy_rollout_sets (K5 section below); dd_gather_env takes none. */
+ * The fused policy rollout takes them through dd_policy_rollout_sets (K5 section below); dd_gather_env takes none.
+ *   Statistics per set (flags & DD_PARAM_SETS_STATS_BY_SET).  The `stats` argument of dd_step_sets, dd_step_plan_sets
+ *     (-> dd_step_planned), dd_rollout_sets and dd_policy_rollout_sets then points to
+ *     uint64[count][DD_STATS_SLOTS][DD_STATS_WORDS]: block s is an ordinary statistics block (words 0-5 as in
+ *     dd_stats_collapse) of the episodes that ended under set s.  An episode counts under the set its ENDING step ran
+ *     under, min(index[i], count-1) before any resample -- the set of its terminal reward and final_obs row; under
+ *     resampling the old set, not the one drawn for the next episode.  The sum of the count blocks equals, bit for bit,
+ *     the totals block the same call writes without the flag; every other output is unchanged.  dd_reset_sets writes no
+ *     statistics.  dd_stats_collapse_sets collapses the blocks. */
 #define DD_MAX_PARAM_SETS      64
 #define DD_PARAM_TABLE_BYTES   32768     /* fixed size: room for 64 sets of the float64 derived constants */
 #define DD_PARAM_SETS_RESAMPLE 0x01
+#define DD_PARAM_SETS_STATS_BY_SET 0x04
 
 typedef struct DDParamSets {
     const void *table;       /* device, 16-byte aligned, DD_PARAM_TABLE_BYTES: the bytes dd_param_sets_build wrote */
@@ -272,6 +281,14 @@ int dd_pack_actions(const uint8_t *actions3, uint8_t *packed, int64_t n, void *s
  *   7 reserved.  (Actor_Critic_PPO.ipynb c21:L94-95,L158-159,L169) */
 int dd_stats_collapse(const uint64_t *stats, const int32_t *steps, const uint8_t *flags, int64_t n,
                       uint64_t *out, void *stream);
+
+/* dd_stats_collapse of a by-set block (DD_PARAM_SETS_STATS_BY_SET): stats uint64[count][DD_STATS_SLOTS][DD_STATS_WORDS]
+ * -> out[count][DD_STATS_WORDS] (device).  Word 6 of block s adds the steps so far of each running episode of an env
+ * whose clamped index min(index[i], count-1) is s: the set that episode runs under (under resampling, index[i] was
+ * written at the reset that started it).  Checked before any CUDA call: NULL stats / out, steps xor flags with n > 0,
+ * or NULL index with steps given and n > 0: DD_E_NULL; count outside [1, DD_MAX_PARAM_SETS] or n < 0: DD_E_RANGE. */
+int dd_stats_collapse_sets(const uint64_t *stats, int32_t count, const int32_t *steps, const uint8_t *flags,
+                           const uint8_t *index, int64_t n, uint64_t *out, void *stream);
 
 /* Everything the per-game surfaces (DroneGame.get_state / _get_info / .done .steps .episode, game_engine.py:140-177,
  * 281-298) read about env i, gathered into ONE record of DD_ENV_RECORD_DOUBLES doubles so that a per-game step of the

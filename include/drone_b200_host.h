@@ -12,7 +12,8 @@
  *
  * Same argument meaning as the device entry points of drone_b200.h, with these differences:
  *   - every pointer is HOST memory, there is no stream, the call is synchronous;
- *   - `stats` is ONE block uint64[DD_STATS_WORDS] (no contention slots), words 0-5 as on the device;
+ *   - `stats` is ONE block uint64[DD_STATS_WORDS] (no contention slots), words 0-5 as on the device; under
+ *     DD_PARAM_SETS_STATS_BY_SET (the _sets twins) uint64[count][DD_STATS_WORDS], attributed as on the device;
  *   - DD_F32: bit-identical to the device kernels except where sin / cos enter (the device uses sincospif,
  *     the host rounds a float64 libm result; <= 1 ulp apart) and expf of the `pg` shaping.
  *     DD_F64: every product and sum rounded separately like the device path; libm sin / cos.

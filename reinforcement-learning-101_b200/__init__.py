@@ -11,11 +11,11 @@ The directory name is not a Python identifier; import it with
 """
 from . import _native as native
 from ._native import build_native
-from .distributed import (allreduce_moments, allreduce_stats, bind_to_gpu_numa, init_from_env, mean_std_from_moments,
-                          shard_range, stats_dict)
+from .distributed import (allreduce_moments, allreduce_stats, allreduce_stats_by_set, bind_to_gpu_numa, init_from_env,
+                          mean_std_from_moments, shard_range, stats_dict)
 
 __all__ = ["native", "build_native", "BatchedDroneEnv", "ShardedDroneEnv", "StepInfo", "gae", "discounted_returns", "advantage_moments",
-           "normalize_advantages", "allreduce_stats", "allreduce_moments", "shard_range", "stats_dict",
+           "normalize_advantages", "allreduce_stats", "allreduce_stats_by_set", "allreduce_moments", "shard_range", "stats_dict",
            "mean_std_from_moments", "init_from_env", "bind_to_gpu_numa", "PolicyBlob", "ValueBlob", "policy_forward", "value_forward",
            "rollout_values", "policy_rollout",
            "step_schedule", "collect_episodes", "curriculum_sweep"]

@@ -42,6 +42,7 @@ LAUNCH_PDL, LAUNCH_BLOCK_128, LAUNCH_BLOCK_512 = 0x01, 0x10, 0x20
 OPERANDS_AUTO, OPERANDS_BF16, OPERANDS_FP16 = 0, 1, 2
 OBS_NATIVE, OBS_F16, OBS_BF16 = 0, 1, 2
 MAX_PARAM_SETS, PARAM_TABLE_BYTES, PARAM_SETS_RESAMPLE = 64, 32768, 0x01
+PARAM_SETS_STATS_BY_SET = 0x04
 
 _PARAM_FIELDS = (
     "width", "height", "gravity", "drag", "angular_drag", "drone_height", "main_thrust", "side_thrust",
@@ -193,6 +194,8 @@ def lib():
     L.dd_pack_actions.argtypes = [vp, vp, i64, vp]
     L.dd_stats_collapse.restype = C.c_int
     L.dd_stats_collapse.argtypes = [vp, vp, vp, i64, vp, vp]
+    L.dd_stats_collapse_sets.restype = C.c_int
+    L.dd_stats_collapse_sets.argtypes = [vp, i32, vp, vp, vp, i64, vp, vp]
     L.dd_moments.restype = C.c_int
     L.dd_moments.argtypes = [vp, i64, vp, vp]
     L.dd_normalize.restype = C.c_int
@@ -256,7 +259,7 @@ EXPORTS = (
     "dd_abi_version", "dd_default_params", "dd_error_string", "dd_reset", "dd_step", "dd_step_plan", "dd_step_planned",
     "dd_rollout", "dd_rollout_shaped",
     "dd_param_sets_build", "dd_reset_sets", "dd_step_sets", "dd_step_plan_sets", "dd_rollout_sets",
-    "dd_fill_random_actions", "dd_pack_actions", "dd_stats_collapse", "dd_moments", "dd_normalize", "dd_gae", "dd_gae_moments",
+    "dd_fill_random_actions", "dd_pack_actions", "dd_stats_collapse", "dd_stats_collapse_sets", "dd_moments", "dd_normalize", "dd_gae", "dd_gae_moments",
     "dd_policy_pack", "dd_policy_pack_ex", "dd_policy_forward", "dd_policy_rollout", "dd_policy_rollout_sets", "dd_policy_rollout_grid", "dd_value_pack", "dd_value_forward", "dd_gather_env", "dd_discounted_returns",
 )
 HOST_TWIN_EXPORTS = ("dd_host_abi_version", "dd_reset_host", "dd_step_host", "dd_rollout_host", "dd_obs16_convert_host",

@@ -154,6 +154,44 @@ __device__ __forceinline__ void stats_warp_commit(unsigned long long* stats, uin
     }
 }
 
+// ---- statistics per parameter set (DD_PARAM_SETS_STATS_BY_SET) ----------------------------------
+// `stats` is uint64[count][DD_STATS_SLOTS][DD_STATS_WORDS]; an episode counts in the block of the set its ending step ran
+// under.  Slot choice as above: only the sums are defined.
+__device__ __forceinline__ unsigned long long* stats_set_slot(unsigned long long* stats, uint32_t set, unsigned slot) {
+    return stats + ((size_t)set * DD_STATS_SLOTS + slot % DD_STATS_SLOTS) * DD_STATS_WORDS;
+}
+
+// stats_warp_commit with the ending lanes grouped by `set`: one pass of the same reductions per distinct set among them
+// (usually one).  Called by ALL 32 lanes; the common case is still the one ballot.
+template <typename R>
+__device__ __forceinline__ void stats_warp_commit_by_set(unsigned long long* stats, uint32_t f, R ret, int32_t steps,
+                                                         uint32_t set) {
+    unsigned todo = __ballot_sync(0xffffffffu, f != 0u);
+    if (todo == 0u) return;                                // warp-uniform
+    const long long rfx = f ? return_fx(ret) : 0ll;
+    const unsigned gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    do {
+        const uint32_t s = __shfl_sync(0xffffffffu, set, __ffs(todo) - 1);
+        const bool mine = f != 0u && set == s;
+        const unsigned done = __ballot_sync(0xffffffffu, mine);
+        todo &= ~done;
+        const unsigned landed = __ballot_sync(0xffffffffu, mine && (f & DD_LANDED) != 0u);
+        const unsigned crashed = __ballot_sync(0xffffffffu, mine && (f & DD_CRASHED) != 0u);
+        const unsigned trunc = __ballot_sync(0xffffffffu, mine && (f & DD_TRUNCATED) != 0u);
+        const long long rsum = warp_sum(mine ? rfx : 0ll);
+        const unsigned len = __reduce_add_sync(0xffffffffu, mine ? (unsigned)steps : 0u);
+        if ((threadIdx.x & 31) == 0) {
+            unsigned long long* b = stats_set_slot(stats, s, gw);
+            atomicAdd(b + 0, (unsigned long long)__popc(done));
+            if (landed) atomicAdd(b + 1, (unsigned long long)__popc(landed));
+            if (crashed) atomicAdd(b + 2, (unsigned long long)__popc(crashed));
+            if (trunc) atomicAdd(b + 3, (unsigned long long)__popc(trunc));
+            atomicAdd(b + 4, (unsigned long long)rsum);
+            atomicAdd(b + 5, (unsigned long long)len);
+        }
+    } while (todo);
+}
+
 // The same statistics accumulated PER THREAD over a multi-step kernel and committed once at its end: integer sums, so
 // the totals equal a stats_warp_commit per step.  (In the T-steps-per-launch kernels the per-step commit -- a ballot every
 // step; three more ballots, ten shuffles and six atomics whenever a lane's episode ended -- was 1-6 % of the issue slots.)
@@ -184,6 +222,45 @@ struct StatsAcc {
             atomicAdd(s + 4, (unsigned long long)rsum);
             atomicAdd(s + 5, (unsigned long long)lsum);
         }
+    }
+    // By-set mode.  commit with the lanes grouped by their (final) set, called by ALL 32 lanes.
+    __device__ __forceinline__ void commit_by_set(unsigned long long* stats, uint32_t set) const {
+        unsigned todo = __ballot_sync(0xffffffffu, done != 0u);
+        if (todo == 0u) return;                            // warp-uniform
+        const unsigned gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+        do {
+            const uint32_t s = __shfl_sync(0xffffffffu, set, __ffs(todo) - 1);
+            const bool mine = done != 0u && set == s;
+            todo &= ~__ballot_sync(0xffffffffu, mine);
+            const unsigned nd = __reduce_add_sync(0xffffffffu, mine ? done : 0u),
+                           nl = __reduce_add_sync(0xffffffffu, mine ? landed : 0u),
+                           nc = __reduce_add_sync(0xffffffffu, mine ? crashed : 0u),
+                           nt = __reduce_add_sync(0xffffffffu, mine ? trunc : 0u);
+            const long long lsum = warp_sum(mine ? (long long)len : 0ll), rsum = warp_sum(mine ? ret : 0ll);
+            if ((threadIdx.x & 31) == 0) {
+                unsigned long long* b = stats_set_slot(stats, s, gw);
+                atomicAdd(b + 0, (unsigned long long)nd);
+                if (nl) atomicAdd(b + 1, (unsigned long long)nl);
+                if (nc) atomicAdd(b + 2, (unsigned long long)nc);
+                if (nt) atomicAdd(b + 3, (unsigned long long)nt);
+                atomicAdd(b + 4, (unsigned long long)rsum);
+                atomicAdd(b + 5, (unsigned long long)lsum);
+            }
+        } while (todo);
+    }
+    // By-set mode, when a resampling reset moves the thread to another set: this thread's totals so far go to `set`'s
+    // block on their own (a few REDs in the episode-end branch; no warp collective there) and the accumulator restarts.
+    __device__ __forceinline__ void flush_thread(unsigned long long* stats, uint32_t set) {
+        if (done) {
+            unsigned long long* b = stats_set_slot(stats, set, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5));
+            atomicAdd(b + 0, (unsigned long long)done);
+            if (landed) atomicAdd(b + 1, (unsigned long long)landed);
+            if (crashed) atomicAdd(b + 2, (unsigned long long)crashed);
+            if (trunc) atomicAdd(b + 3, (unsigned long long)trunc);
+            atomicAdd(b + 4, (unsigned long long)ret);
+            atomicAdd(b + 5, (unsigned long long)len);
+        }
+        *this = StatsAcc();
     }
 };
 

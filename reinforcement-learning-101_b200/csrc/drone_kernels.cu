@@ -64,9 +64,11 @@ __device__ __forceinline__ obs_elem_t<R, OF>* obs_ptr(R* p) { return reinterpret
 // =================================================================================================
 // SETS: per-env parameter sets (KArgsPS): env i's constants are set min(index[i], count - 1) of the table, read through
 // L1 after the index byte arrives; under ps_resample each auto-reset draws a new set (param_set_draw) before it spawns.
-template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK, int OF, bool SETS>
+// BYSET (SETS only, DD_PARAM_SETS_STATS_BY_SET): the statistics go to the block of the set the ending step ran under.
+template <typename R, bool AUTO, bool OBS, bool DEF, int BLOCK, int OF, bool SETS, bool BYSET = false>
 __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KArgsOf<R, SETS> a)
 {
+    static_assert(SETS || !BYSET, "statistics per set: parameter-set kernels only");
     using O = obs_elem_t<R, OF>;
     __shared__ __align__(128) O s_obs[OBS ? BLOCK * kMaxObsStride : 1];
     Consts<R> k;
@@ -78,6 +80,7 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
 
     pdl_wait();                                            // state / actions may come from the previous launch
     uint32_t f_stat = 0; R ret_stat = 0; int32_t len_stat = 0;
+    uint32_t set_stat = 0;                                 // BYSET: the set of the ending step
     if (live) {
         // ---- every load of this thread, back to back ----
         Env<R> e;
@@ -100,6 +103,7 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
             oflags = f;
             if (f) {                                           // rare: ~1 % of env-steps
                 f_stat = f; ret_stat = e.ret; len_stat = e.steps;
+                if constexpr (BYSET) set_stat = param_set_clamp(set, a.ps_count);
                 if (a.final_obs) {                             // terminal observation (scattered rows)
                     O* fo = obs_ptr<OF>(a.final_obs) + (size_t)i * a.obs_stride;
                     if (!OBS) speed = Arith<R>::sqrt_(Arith<R>::fma_(e.vx, e.vx, Arith<R>::mul(e.vy, e.vy)));
@@ -146,7 +150,10 @@ __global__ void __launch_bounds__(BLOCK) step_kernel(const __grid_constant__ KAr
         pdl_launch_dependents();
     }
 
-    if (a.stats) stats_warp_commit(a.stats, f_stat, ret_stat, len_stat);
+    if (a.stats) {
+        if constexpr (BYSET) stats_warp_commit_by_set(a.stats, f_stat, ret_stat, len_stat, set_stat);
+        else stats_warp_commit(a.stats, f_stat, ret_stat, len_stat);
+    }
     if (OBS) {
         const uint32_t rem = a.n - tile0;
         const int rows = rem < (uint32_t)BLOCK ? (int)rem : BLOCK;
@@ -228,9 +235,12 @@ struct RArgs {
 // sweep and the throughput bench -- compiles their address arithmetic and predicated stores away.
 // SETS: as in step_kernel; the env's constants stay in registers over the T steps and are reloaded when a resampling
 // auto-reset draws a new set (index[i] is written back once, at the end).
-template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS, int OF, bool SETS>
+// BYSET (SETS only): statistics per set.  A thread's totals belong to its current set: they are committed, grouped by set,
+// at the end, and flushed by the thread itself when a resampling reset moves it to another set.
+template <typename R, bool OBS, bool DEF, int POLICY, bool OUTS, int OF, bool SETS, bool BYSET = false>
 __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__ RArgs<R, KArgsOf<R, SETS>> ra)
 {
+    static_assert(SETS || !BYSET, "statistics per set: parameter-set kernels only");
     using O = obs_elem_t<R, OF>;
     __shared__ __align__(128) O s_obs[OBS ? kBlock * kMaxObsStride : 1];
     const auto& a = ra.a;
@@ -308,7 +318,13 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
                     if (auto_reset) {
                         if constexpr (SETS) {
                             if (a.ps_resample) {
-                                set = param_set_draw(a.seed, gid, ep, a.ps_count);
+                                if constexpr (BYSET) {          // the totals so far belong to the old set
+                                    const uint32_t drawn = param_set_draw(a.seed, gid, ep, a.ps_count);
+                                    if (do_stats && drawn != set) st.flush_thread(a.stats, set);
+                                    set = drawn;
+                                } else {
+                                    set = param_set_draw(a.seed, gid, ep, a.ps_count);
+                                }
                                 set_dirty = true;
                                 k = param_set<R>(a.ps_table, set);
                             }
@@ -361,7 +377,10 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
         for (int32_t t = 0; t < ra.T; ++t) one_step(t);
     }
 
-    if (do_stats) st.commit(a.stats);
+    if (do_stats) {
+        if constexpr (BYSET) st.commit_by_set(a.stats, set);
+        else st.commit(a.stats);
+    }
     if (live) {
         store_env(a, i, e);
         a.flags[i] = (uint8_t)pflags;
@@ -438,6 +457,47 @@ __global__ void __launch_bounds__(kBlock) live_steps_kernel(const int32_t* steps
     if ((threadIdx.x & 31) == 0 && t) atomicAdd(out + 6, t);
 }
 
+// By-set blocks (DD_PARAM_SETS_STATS_BY_SET): thread j collapses word j % 8 of block j / 8, as stats_collapse_kernel does.
+__global__ void stats_collapse_sets_kernel(const unsigned long long* stats, int count, unsigned long long* out)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= count * DD_STATS_WORDS) return;
+    const int w = j % DD_STATS_WORDS;
+    const unsigned long long* b = stats + (size_t)(j / DD_STATS_WORDS) * DD_STATS_SLOTS * DD_STATS_WORDS;
+    unsigned long long t = 0;
+    const int col = (w == 6) ? 5 : w;
+    for (int s = 0; s < DD_STATS_SLOTS; ++s) t += b[s * DD_STATS_WORDS + col];
+    out[j] = (w == 7) ? 0ull : t;
+}
+
+// out[s][6] += sum of steps[i] over running episodes with min(index[i], count-1) == s: per warp, one pass per distinct set
+// among its running envs, into per-CTA totals, then one atomic per set and CTA.
+__global__ void __launch_bounds__(kBlock) live_steps_sets_kernel(const int32_t* steps, const uint8_t* flags,
+                                                                  const uint8_t* index, uint32_t count, int64_t n,
+                                                                  unsigned long long* out)
+{
+    __shared__ unsigned long long acc[DD_MAX_PARAM_SETS];
+    for (int j = threadIdx.x; j < DD_MAX_PARAM_SETS; j += kBlock) acc[j] = 0ull;
+    __syncthreads();
+    const int64_t stride = (int64_t)gridDim.x * kBlock;
+    for (int64_t base = (int64_t)blockIdx.x * kBlock + (threadIdx.x & ~31); base < n; base += stride) {
+        const int64_t i = base + (threadIdx.x & 31);     // the whole warp walks the loop together
+        const bool run = i < n && !(flags[i] & DD_DONE);
+        const uint32_t set = run ? param_set_clamp(index[i], count) : 0u;
+        unsigned todo = __ballot_sync(0xffffffffu, run);
+        while (todo) {
+            const uint32_t s = __shfl_sync(0xffffffffu, set, __ffs(todo) - 1);
+            const bool mine = run && set == s;
+            todo &= ~__ballot_sync(0xffffffffu, mine);
+            const long long t = warp_sum(mine ? (long long)steps[i] : 0ll);
+            if ((threadIdx.x & 31) == 0 && t) atomicAdd(acc + s, (unsigned long long)t);
+        }
+    }
+    __syncthreads();
+    for (uint32_t s = threadIdx.x; s < count; s += kBlock)
+        if (acc[s]) atomicAdd(out + (size_t)s * DD_STATS_WORDS + 6, acc[s]);
+}
+
 // =================================================================================================
 // host side of the ABI
 // =================================================================================================
@@ -511,7 +571,9 @@ static int step_resolve(StepPlanT<R, SETS>& pl, const DDState* s, const P* p, co
             with_bool(c->auto_reset != 0, [&](auto au) {
                 with_bool(obs != nullptr, [&](auto ob) {
                     with_block<R>(c->launch_flags, [&](auto block) {
-                        pl.kern = step_kernel<R, au, ob, def, block, of, SETS>;
+                        with_by_set<SETS>(*p, [&](auto bs) {
+                            pl.kern = step_kernel<R, au, ob, def, block, of, SETS, bs>;
+                        });
                         pl.block = block;
                     });
                 });
@@ -590,7 +652,11 @@ static int rollout_impl(const DDState* s, const P* p, const DDEnvConfig* c, int3
     const auto run = [&](auto obs, auto of) {
         return with_def<SETS>(*p, [&](auto def) {
             return with_bool(outs, [&](auto out) {
-                const auto go = [&](auto pol) { return launch(rollout_kernel<R, obs, def, pol, out, of, SETS>, g, kBlock, st, pdl, ra); };
+                const auto go = [&](auto pol) {
+                    return with_by_set<SETS>(*p, [&](auto bs) {
+                        return launch(rollout_kernel<R, obs, def, pol, out, of, SETS, bs>, g, kBlock, st, pdl, ra);
+                    });
+                };
                 return policy == DD_POLICY_TRACE    ? go(int_c<DD_POLICY_TRACE>())
                      : policy == DD_POLICY_RANDOM ? go(int_c<DD_POLICY_RANDOM>())
                                                   : go(int_c<DD_POLICY_BANGBANG>());
@@ -779,6 +845,26 @@ int dd_stats_collapse(const uint64_t* stats, const int32_t* steps, const uint8_t
         int g = dd::grid_for(n, dd::kBlock * 8);
         if (g > 148 * 8) g = 148 * 8;
         dd::live_steps_kernel<<<g, dd::kBlock, 0, (cudaStream_t)stream>>>(steps, flags, n, (unsigned long long*)out);
+    }
+    return (int)cudaGetLastError();
+}
+
+int dd_stats_collapse_sets(const uint64_t* stats, int32_t count, const int32_t* steps, const uint8_t* flags,
+                           const uint8_t* index, int64_t n, uint64_t* out, void* stream)
+{
+    if (!stats || !out) return DD_E_NULL;
+    if (count < 1 || count > DD_MAX_PARAM_SETS || n < 0) return DD_E_RANGE;
+    if (n > 0 && ((steps == nullptr) != (flags == nullptr))) return DD_E_NULL;
+    if (steps && n > 0 && !index) return DD_E_NULL;
+    dd::DeviceGuard g((cudaStream_t)stream, stats);
+    if (g.err != cudaSuccess) return (int)g.err;
+    dd::stats_collapse_sets_kernel<<<count, DD_STATS_WORDS, 0, (cudaStream_t)stream>>>(
+        (const unsigned long long*)stats, count, (unsigned long long*)out);
+    if (steps && n > 0) {
+        int gr = dd::grid_for(n, dd::kBlock * 8);
+        if (gr > 148 * 8) gr = 148 * 8;
+        dd::live_steps_sets_kernel<<<gr, dd::kBlock, 0, (cudaStream_t)stream>>>(steps, flags, index, (uint32_t)count, n,
+                                                                              (unsigned long long*)out);
     }
     return (int)cudaGetLastError();
 }

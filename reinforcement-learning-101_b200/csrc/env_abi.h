@@ -44,7 +44,8 @@ inline int fill_args(KArgsPS<R>& a, const DDState* s, const DDParamSets* ps, con
     if (!ps) return DD_E_NULL;
     if (int rc = fill_state(a, s, c, n)) return rc;
     if (n > 0 && (!ps->table || !ps->index)) return DD_E_NULL;
-    if (ps->count < 1 || ps->count > DD_MAX_PARAM_SETS || (ps->flags & ~DD_PARAM_SETS_RESAMPLE)) return DD_E_RANGE;
+    if (ps->count < 1 || ps->count > DD_MAX_PARAM_SETS || (ps->flags & ~(DD_PARAM_SETS_RESAMPLE | DD_PARAM_SETS_STATS_BY_SET)))
+        return DD_E_RANGE;
     if (ps->dtype != s->dtype) return DD_E_DTYPE;
     if (reinterpret_cast<uintptr_t>(ps->table) & 15u) return DD_E_ALIGN;
     a.ps_table = ps->table; a.ps_index = ps->index;
@@ -95,6 +96,14 @@ template <typename F>
 inline auto with_bool(bool b, F&& f) { return b ? f(std::true_type()) : f(std::false_type()); }
 
 template <int V> using int_c = std::integral_constant<int, V>;
+
+// f(std::bool_constant<BYSET>()): the statistics-per-set kernels exist for parameter-set calls only.
+template <bool SETS, typename P, typename F>
+inline auto with_by_set(const P& p, F&& f)
+{
+    if constexpr (SETS) return with_bool((p.flags & DD_PARAM_SETS_STATS_BY_SET) != 0, f);
+    else return f(std::false_type());
+}
 
 // f(int_c<OF>()) for a DDEnvConfig.obs_format that check_obs_format accepted: the 16-bit formats exist for float only.
 template <typename R, typename F>

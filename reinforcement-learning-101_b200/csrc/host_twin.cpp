@@ -75,11 +75,19 @@ struct ConstSource {
     {
         if (!sets) { if (!p) return DD_E_NULL; k0 = make_consts<R>(*p); return 0; }
         if (n > 0 && (!sets->table || !sets->index)) return DD_E_NULL;
-        if (sets->count < 1 || sets->count > DD_MAX_PARAM_SETS || (sets->flags & ~DD_PARAM_SETS_RESAMPLE)) return DD_E_RANGE;
+        if (sets->count < 1 || sets->count > DD_MAX_PARAM_SETS ||
+            (sets->flags & ~(DD_PARAM_SETS_RESAMPLE | DD_PARAM_SETS_STATS_BY_SET))) return DD_E_RANGE;
         if (sets->dtype != s->dtype) return DD_E_DTYPE;
         if (reinterpret_cast<uintptr_t>(sets->table) & 15u) return DD_E_ALIGN;
         ps = sets;
         return 0;
+    }
+    // the statistics block of env i's current set: `stats` is uint64[count][DD_STATS_WORDS] under
+    // DD_PARAM_SETS_STATS_BY_SET (read before a resampling reset rewrites index[i]: the ending step's set)
+    uint64_t* stats_of(uint64_t* stats, int64_t i) const
+    {
+        if (!stats || !ps || !(ps->flags & DD_PARAM_SETS_STATS_BY_SET)) return stats;
+        return stats + (size_t)param_set_clamp(ps->index[i], (uint32_t)ps->count) * DD_STATS_WORDS;
     }
     Consts<R> of(int64_t i) const
     {
@@ -183,7 +191,7 @@ int step_host(const DDState* s, const DDParams* p, const DDParamSets* ps, const 
             if (!f && c->max_steps > 0 && e.steps >= c->max_steps) f = DD_DONE | DD_TRUNCATED;
             oflags = f;
             if (f) {
-                stats_commit(stats, f, e.ret, e.steps);
+                stats_commit(src.stats_of(stats, i), f, e.ret, e.steps);
                 if (final_obs) obs_row(final_obs, i, stride, c->obs_format, e, f, speed, dist, k, false, (R)0);
                 if (AUTO) {
                     const uint32_t ep = h.episode[i];
@@ -261,7 +269,7 @@ int rollout_host(const DDState* s, const DDParams* p, const DDParamSets* ps, con
                     dcur = Arith<R>::div(dist, k.width, k.inv_width);
                 }
                 if (f) {
-                    stats_commit(stats, f, e.ret, e.steps);
+                    stats_commit(src.stats_of(stats, i), f, e.ret, e.steps);
                     if (auto_reset) {
                         k = src.at_reset(i, k, c->seed, gid, ep);
                         spawn(e, k, c->seed, gid, ep, c->randomize_drone != 0, c->randomize_platform != 0);

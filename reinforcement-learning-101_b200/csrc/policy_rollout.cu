@@ -409,10 +409,13 @@ __device__ __forceinline__ void store_a_chunk_relu_tmem(uint32_t ta, int c, cons
 // through L1 where they are used: the observation's at the top of the step, the env step's (and its landing margin,
 // pre_sc_margin_of) under the head MMA.  Under ps_resample the set of the NEXT episode is drawn with its spawn, ahead of
 // time; the reset switches to it (index[i] is written back once, at the end).
-template <bool DEF, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false, bool SETS = false>
+// BYSET (SETS only): statistics per set, as in rollout_kernel -- committed grouped by set at the end, and flushed by the
+// thread when a resampling reset moves it to another set.
+template <bool DEF, bool FWD, int HEAD = 3, bool FAST = false, bool F16 = false, bool SETS = false, bool BYSET = false>
 __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __grid_constant__ PArgsOf<SETS> pa)
 {
     static_assert(!SETS || (!DEF && !FWD && HEAD == 3), "parameter sets: rollout instantiations with generic constants only");
+    static_assert(SETS || !BYSET, "statistics per set: parameter-set kernels only");
     extern __shared__ __align__(1024) uint8_t smem[];
     const KArgs<float>& a = pa.a;
     const Consts<float> k = consts_of<float, DEF>(a);
@@ -790,6 +793,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
                         Consts<float> kn = ks;
                         kn.max_fuel = ks_next_fuel;            // (spawn_apply reads max_fuel only)
                         spawn_apply(e, kn, nsx, nsy, nspx, nspy);
+                        if constexpr (BYSET) { if (nset != set) st.flush_thread(a.stats, set); }
                         if (pa.ps_resample) set_dirty = true;
                         set = nset;
                     } else {
@@ -817,7 +821,10 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_rollout_kernel(const __
         pend.oflags = oflags;
     }
     if (!forward_only && T_mine > 0) flush_pending((size_t)(T_mine - 1) * a.n + i);
-    if (!forward_only && do_stats && T_mine > 0) st.commit(a.stats);            // one statistics commit per warp and rollout
+    if (!forward_only && do_stats && T_mine > 0) {                               // one statistics commit per warp and rollout
+        if constexpr (BYSET) st.commit_by_set(a.stats, set);
+        else st.commit(a.stats);
+    }
 
     if (live && !forward_only) {
         store4(a.pos_vel, i, e.x, e.y, e.vx, e.vy);
@@ -999,9 +1006,10 @@ static int policy_launch(PA& pa, cudaStream_t st, Pick&& pick)
     return (int)cudaGetLastError();
 }
 
-// The rollout launch (single set: p; per-env sets: SETS).  FAST is the PPO-collection configuration of the kernel's header.
-template <bool SETS>
-static int rollout_launch(PArgsOf<SETS>& pa, const DDParams* p, int64_t n, cudaStream_t st)
+// The rollout launch (single set: P = DDParams; per-env sets: P = DDParamSets, SETS).  FAST is the PPO-collection
+// configuration of the kernel's header.
+template <bool SETS, typename P>
+static int rollout_launch(PArgsOf<SETS>& pa, const P* p, int64_t n, cudaStream_t st)
 {
     const bool fast = pa.mode == DD_ACTION_SAMPLE && pa.inv_temperature == 1.0f && pa.auto_reset && pa.a.stats &&
                       pa.actions_tn && pa.logp_tn && pa.reward_tn && pa.done_tn && pa.obs_tn && !pa.shaped_tn && !pa.probs_tn;
@@ -1010,7 +1018,7 @@ static int rollout_launch(PArgsOf<SETS>& pa, const DDParams* p, int64_t n, cudaS
         grid = rollout_grid(n, sms);
         return with_bool(fast, [&](auto fa) {
             return with_bool(f16, [&](auto h) {
-                if constexpr (SETS) return policy_rollout_kernel<false, false, 3, fa, h, true>;
+                if constexpr (SETS) return with_by_set<true>(*p, [&](auto bs) { return policy_rollout_kernel<false, false, 3, fa, h, true, bs>; });
                 else return with_bool(params_are_default(*p), [&](auto def) { return policy_rollout_kernel<def, false, 3, fa, h>; });
             });
         });
@@ -1059,8 +1067,7 @@ static int policy_rollout_impl(const DDState* s, const P* p, const DDEnvConfig* 
     pa.inv_temperature = mode == DD_ACTION_SAMPLE ? 1.0f / temperature : 1.0f;
     pa.actions_tn = actions_tn; pa.logp_tn = logp_tn; pa.reward_tn = reward_tn; pa.done_tn = done_tn;
     pa.obs_tn = obs_tn; pa.probs_tn = probs_tn; pa.shaped_tn = shaped_tn; pa.obs_in = nullptr; pa.auto_reset = c->auto_reset;
-    if constexpr (SETS) return rollout_launch<true>(pa, nullptr, n, st);
-    else return rollout_launch<false>(pa, p, n, st);
+    return rollout_launch<SETS>(pa, p, n, st);
 }
 
 static int pack_common(const DDPolicy* p, int head, int operands, void* blob, DDPolicyConsts* consts, void* stream)

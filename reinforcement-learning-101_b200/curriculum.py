@@ -23,13 +23,23 @@ def step_schedule(num_iterations: int, start: int = 300, end: int = 500, steepne
     return np.round(start + (end - start) * x ** steepness).astype(np.int32)
 
 
+def _collect_keys(max_steps: int, s: Dict[str, float]) -> Dict[str, float]:
+    return {"max_steps": int(max_steps), "num_games": s["episodes"], "num_successes": s["landed"],
+            "success_rate": s["landing_rate"], "avg_reward": s["mean_return"], "avg_steps": s["mean_length"],
+            "crashed": s["crashed"], "timed_out": s["truncated"], "env_steps": s["sum_length"]}
+
+
 def collect_episodes(env: BatchedDroneEnv, max_steps: int, policy: str = "random", blob=None, sample: bool = True,
-                     reduce: bool = True, t0: Optional[int] = None) -> Dict[str, float]:
+                     reduce: bool = True, t0: Optional[int] = None, by_set: bool = False) -> Dict[str, float]:
     """One curriculum iteration: every env plays one episode of at most ``max_steps`` steps.
     ``policy``: 'random' / 'bangbang' (scripted, in-kernel) or 'network' with a ``PolicyBlob``.
     ``t0``: offset of the in-kernel noise streams; ``None`` continues the env's running counter, so every stage /
     iteration explores with fresh noise (include/drone_b200.h, t0 contract).
-    Returns the (all-reduced) statistics dict: success_rate, avg_reward (engine return), avg_steps, ..."""
+    Returns the (all-reduced) statistics dict: success_rate, avg_reward (engine return), avg_steps, ...
+    ``by_set=True`` (an env with ``set_param_sets(..., stats_by_set=True)``): the dict also holds ``"by_set"``, one dict
+    with the same keys per parameter set -- one policy evaluated on several worlds in one launch."""
+    if by_set and not env.stats_by_set:
+        raise ValueError("by_set=True needs an env with set_param_sets(..., stats_by_set=True)")
     if env.auto_reset:
         raise ValueError("collect_episodes needs an env built with auto_reset=False (one episode per env)")
     env.max_steps = int(max_steps)
@@ -42,16 +52,16 @@ def collect_episodes(env: BatchedDroneEnv, max_steps: int, policy: str = "random
         policy_rollout(env, blob, int(max_steps), sample=sample, t0=t0, want="")
     else:
         env.rollout(int(max_steps), policy, t0=t0)
-    s = env.stats(reduce=reduce)
-    return {"max_steps": int(max_steps), "num_games": s["episodes"], "num_successes": s["landed"],
-            "success_rate": s["landing_rate"], "avg_reward": s["mean_return"], "avg_steps": s["mean_length"],
-            "crashed": s["crashed"], "timed_out": s["truncated"], "env_steps": s["sum_length"]}
+    out = _collect_keys(max_steps, env.stats(reduce=reduce))
+    if by_set:
+        out["by_set"] = [_collect_keys(max_steps, s) for s in env.stats(reduce=reduce, by_set=True)]
+    return out
 
 
 def curriculum_sweep(env: BatchedDroneEnv, caps: Iterable[int], policy: str = "random", blob=None,
-                     sample: bool = True, reduce: bool = True) -> List[Dict[str, float]]:
+                     sample: bool = True, reduce: bool = True, by_set: bool = False) -> List[Dict[str, float]]:
     """``collect_episodes`` for each cap in ``caps`` (e.g. ``step_schedule(8, 75, 250)``)."""
     out = []
     for cap in caps:        # t0=None: each stage continues the env's noise counter (stage j starts at sum(caps[:j]))
-        out.append(collect_episodes(env, int(cap), policy=policy, blob=blob, sample=sample, reduce=reduce))
+        out.append(collect_episodes(env, int(cap), policy=policy, blob=blob, sample=sample, reduce=reduce, by_set=by_set))
     return out

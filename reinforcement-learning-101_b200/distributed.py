@@ -1,7 +1,8 @@
 """Multi-GPU plumbing: environments shard by contiguous global id, one process per GPU, and the
 only collectives are two tiny all-reduces (SURVEY.md 8e):
 
-  * episode statistics  -- 8 int64 words        (Actor_Critic_PPO.ipynb c21:L94-95,L158-159,L169)
+  * episode statistics  -- 8 int64 words        (Actor_Critic_PPO.ipynb c21:L94-95,L158-159,L169),
+                           or count x 8 with statistics per parameter set
   * advantage moments   -- n, sum x, sum x^2     (Actor_Critic_PPO.ipynb c21:L105)
 
 There is no per-step communication.  Integer sums make the statistics independent of the GPU
@@ -79,6 +80,16 @@ def allreduce_stats(words: torch.Tensor) -> torch.Tensor:
     """Sum the int64[8] statistics block over all ranks (in place; returns it)."""
     if words.dtype != torch.int64 or words.numel() != len(STAT_NAMES):
         raise ValueError("stats block must be int64[8]")
+    if world()[1] > 1:
+        dist.all_reduce(words, op=dist.ReduceOp.SUM)
+    return words
+
+
+def allreduce_stats_by_set(words: torch.Tensor) -> torch.Tensor:
+    """Sum an int64[count, 8] statistics block per parameter set over all ranks, in one collective (in place; returns
+    it).  Every rank must hold the same count."""
+    if words.dtype != torch.int64 or words.dim() != 2 or words.shape[1] != len(STAT_NAMES) or words.shape[0] < 1:
+        raise ValueError("per-set stats block must be int64[count, 8]")
     if world()[1] > 1:
         dist.all_reduce(words, op=dist.ReduceOp.SUM)
     return words

@@ -174,6 +174,7 @@ class BatchedDroneEnv:
         # ---- episode statistics (K3) ----
         self.stats_slots = torch.zeros(nv.STATS_SLOTS, nv.STATS_WORDS, dtype=torch.int64, device=dev)
         self._stats_out = torch.zeros(nv.STATS_WORDS, dtype=torch.int64, device=dev)
+        self._stats_plain = (self.stats_slots, self._stats_out)    # the totals buffers, kept for plain mode
 
         self._state = nv.DDState(self.pos_vel.data_ptr(), self.att_fuel.data_ptr(), self.platform.data_ptr(),
                                  self.steps.data_ptr(), self.episode.data_ptr(), self.flags.data_ptr(),
@@ -192,6 +193,7 @@ class BatchedDroneEnv:
         self._ps = None
         self._ps_table = None
         self.param_index: Optional[torch.Tensor] = None
+        self._stats_by_set = False
         if param_sets is not None:
             self.set_param_sets(param_sets, param_index, resample_param_sets)
         elif param_index is not None or resample_param_sets:
@@ -235,7 +237,8 @@ class BatchedDroneEnv:
         self._plans.clear()
 
     # ---- per-env parameter sets --------------------------------------------------------------------
-    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False) -> None:
+    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False,
+                       stats_by_set: bool = False) -> None:
         """Give env i the physics of ``sets[min(param_index[i], len(sets) - 1)]`` (include/drone_b200.h, DDParamSets).
 
         ``sets``: a sequence of 1-64 ``DDParams`` structs (copied), or None to return every env to ``params``.
@@ -243,12 +246,17 @@ class BatchedDroneEnv:
         ``param_index`` (uint8 ``[N]`` on the device): editing that tensor in place takes effect at the next call.
         ``resample``: every reset of an env -- ``reset`` and same-step auto-resets -- draws its next set from
         Philox(seed, env id, episode, stream 3), writes it to ``param_index`` and spawns under it; the step that ends an
-        episode keeps the old set.  Drops the resolved step launches, like the ``params`` setter."""
+        episode keeps the old set.  Drops the resolved step launches, like the ``params`` setter.
+        ``stats_by_set``: keep the episode statistics per set (``stats(by_set=True)``) instead of in one totals block.
+        An episode counts under the set its ending step ran under (under ``resample`` the old set).  The totals
+        (``stats()``) stay what plain mode reports.  Entering, leaving or changing the sets of this mode starts the
+        statistics afresh."""
         self._plans.clear()
         if sets is None:
-            if index is not None or resample:
-                raise ValueError("index / resample need sets")
+            if index is not None or resample or stats_by_set:
+                raise ValueError("index / resample / stats_by_set need sets")
             self._sets = self._ps = self._ps_table = self.param_index = None
+            self._select_stats(0)
             return
         sets = [nv.DDParams.from_buffer_copy(p) if isinstance(p, nv.DDParams) else p for p in sets]
         dt = nv.F32 if self.dtype == torch.float32 else nv.F64
@@ -269,7 +277,28 @@ class BatchedDroneEnv:
         self._sets = sets
         self.param_index = idx
         self._ps = nv.DDParamSets(self._ps_table.data_ptr(), idx.data_ptr(), len(sets), dt,
-                                  nv.PARAM_SETS_RESAMPLE if resample else 0, 0)
+                                  (nv.PARAM_SETS_RESAMPLE if resample else 0)
+                                  | (nv.PARAM_SETS_STATS_BY_SET if stats_by_set else 0), 0)
+        self._select_stats(len(sets) if stats_by_set else 0)
+
+    def _select_stats(self, by_set_count: int) -> None:
+        """The statistics buffers of the mode: the totals block (0), kept as it is when plain mode stays, or a fresh
+        ``[count, 64, 8]`` by-set block."""
+        if by_set_count == 0 and not self._stats_by_set:
+            return
+        if by_set_count:
+            self.stats_slots = torch.zeros(by_set_count, nv.STATS_SLOTS, nv.STATS_WORDS, dtype=torch.int64,
+                                           device=self.device)
+            self._stats_out = torch.zeros(by_set_count, nv.STATS_WORDS, dtype=torch.int64, device=self.device)
+        else:
+            self.stats_slots, self._stats_out = self._stats_plain
+            self.stats_slots.zero_()
+        self._stats_by_set = by_set_count > 0
+
+    @property
+    def stats_by_set(self) -> bool:
+        """Whether the episode statistics are kept per parameter set (``set_param_sets(..., stats_by_set=True)``)."""
+        return self._stats_by_set
 
     @property
     def param_sets(self):
@@ -473,23 +502,38 @@ class BatchedDroneEnv:
         return out
 
     # ---- episode statistics (K3) --------------------------------------------------------------------
-    def stats_tensor(self) -> torch.Tensor:
+    def stats_tensor(self, by_set: bool = False) -> torch.Tensor:
         """int64[8] on device: episodes, landed, crashed, truncated, sum_return (2^-20 units),
         sum_length, env_steps (= sum_length + steps so far of the running episodes), reserved --
-        accumulated since the last ``reset_stats()``."""
-        nv.check(self._lib.dd_stats_collapse(self.stats_slots.data_ptr(), self.steps.data_ptr(), self.flags.data_ptr(),
-                                             self.num_envs, self._stats_out.data_ptr(), self._stream()),
-                 "dd_stats_collapse")
-        return self._stats_out
+        accumulated since the last ``reset_stats()``.
+        ``by_set=True`` (statistics per set only): int64[count, 8], row s for the episodes of set s; the running
+        episodes' steps count under their env's ``param_index``.  In that mode ``by_set=False`` gives the totals, the
+        sum of the rows."""
+        if by_set and not self._stats_by_set:
+            raise ValueError("by_set=True needs set_param_sets(..., stats_by_set=True)")
+        if not self._stats_by_set:
+            nv.check(self._lib.dd_stats_collapse(self.stats_slots.data_ptr(), self.steps.data_ptr(),
+                                                 self.flags.data_ptr(), self.num_envs, self._stats_out.data_ptr(),
+                                                 self._stream()), "dd_stats_collapse")
+            return self._stats_out
+        nv.check(self._lib.dd_stats_collapse_sets(self.stats_slots.data_ptr(), self._ps.count, self.steps.data_ptr(),
+                                                  self.flags.data_ptr(), self.param_index.data_ptr(), self.num_envs,
+                                                  self._stats_out.data_ptr(), self._stream()), "dd_stats_collapse_sets")
+        return self._stats_out if by_set else self._stats_out.sum(0)
 
     def reset_stats(self) -> None:
         self.stats_slots.zero_()
 
-    def stats(self, reduce: bool = False) -> Dict[str, float]:
+    def stats(self, reduce: bool = False, by_set: bool = False):
         """Host dict of the episode statistics (Actor_Critic_PPO.ipynb c21:L94-95,L158-159,L169);
-        ``reduce=True`` all-reduces the 8 words over the default process group first."""
-        from .distributed import allreduce_stats, stats_dict
-        w = self.stats_tensor()
+        ``reduce=True`` all-reduces the 8 words over the default process group first.
+        ``by_set=True`` (statistics per set only): a list of one such dict per parameter set."""
+        from .distributed import allreduce_stats, allreduce_stats_by_set, stats_dict
+        w = self.stats_tensor(by_set)
+        if by_set:
+            if reduce:
+                w = allreduce_stats_by_set(w.clone())
+            return [stats_dict(r) for r in w]
         if reduce:
             w = allreduce_stats(w.clone())
         return stats_dict(w)

@@ -240,7 +240,8 @@ class ShardedDroneEnv:
             e.params = p
         self._drop_graphs()
 
-    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False) -> None:
+    def set_param_sets(self, sets, index: Optional[torch.Tensor] = None, resample: bool = False,
+                       stats_by_set: bool = False) -> None:
         """Per-env parameter sets for every shard (``BatchedDroneEnv.set_param_sets``); ``index``: ``[S, N]`` (None:
         env i of each shard runs under set ``i % len(sets)``).  The captured graphs are dropped.  Afterwards in-place
         edits of ``shards[s].param_index`` reach the graphs as they are (they hold its pointer; ``join()`` first)."""
@@ -248,15 +249,16 @@ class ShardedDroneEnv:
             raise ValueError(f"index must have shape {(self.S, self.N)}")
         self.join()
         for s, e in enumerate(self.shards):
-            e.set_param_sets(sets, None if index is None else index[s], resample)
+            e.set_param_sets(sets, None if index is None else index[s], resample, stats_by_set)
         self._drop_graphs()
 
     # ---- statistics / state -------------------------------------------------------------------------------------
-    def stats_tensor(self) -> torch.Tensor:
+    def stats_tensor(self, by_set: bool = False) -> torch.Tensor:
+        """The shards' ``stats_tensor(by_set)`` summed: int64[8], or int64[count, 8] per parameter set."""
         self.join()
-        out = self.shards[0].stats_tensor().clone()
+        out = self.shards[0].stats_tensor(by_set).clone()
         for e in self.shards[1:]:
-            out += e.stats_tensor()
+            out += e.stats_tensor(by_set)
         return out
 
     def reset_stats(self) -> None:
@@ -264,9 +266,13 @@ class ShardedDroneEnv:
         for e in self.shards:
             e.reset_stats()
 
-    def stats(self, reduce: bool = False) -> Dict[str, float]:
-        from .distributed import allreduce_stats, stats_dict
-        w = self.stats_tensor()
+    def stats(self, reduce: bool = False, by_set: bool = False):
+        from .distributed import allreduce_stats, allreduce_stats_by_set, stats_dict
+        w = self.stats_tensor(by_set)
+        if by_set:
+            if reduce:
+                w = allreduce_stats_by_set(w)
+            return [stats_dict(r) for r in w]
         if reduce:
             w = allreduce_stats(w)
         return stats_dict(w)
